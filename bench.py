@@ -3,6 +3,7 @@
 CMash-style sketch database, plus the probe kernel's fraction of the HBM roofline.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload weak|strong|stream|stress]
+                  [--dump-outputs DIR]
 
 A "step" is one whole pass of the hot path over one batch of synthetic reads: canonical 60-mer counting
 against the database (K1), intersection, multi-k prefix expansion (K2), per-genome tables (K3), and -- with
@@ -14,6 +15,9 @@ streaming its share from pinned host memory in 10M-read batches through one quer
 
 After the timed region rank 0 runs the CPU oracle over ALL reads of the job and compares its per-genome tables and
 intersection size with the GPU's (`parity_checked`; skipped above 100M reads / 2e5 genomes unless MLG_BENCH_PARITY=1).
+
+--dump-outputs DIR writes what the last timed step of the native arm handed its caller as DIR/<name>.npy (float64), so that
+two builds run with the same arguments (the inputs are seeded) can be compared output for output: see dump_outputs().
 
 Environment overrides (for quick runs): MLG_BENCH_G, MLG_BENCH_READS (per GPU), MLG_BENCH_TOTAL_READS,
 MLG_BENCH_BATCH_READS, MLG_BENCH_CPU_READS, MLG_BENCH_SKIP_CPU=1, MLG_BENCH_PARITY=0|1, MLG_EXCHANGE=sparse|dense|p2p.
@@ -132,6 +136,25 @@ def measured_request_ceiling():
         return best
     except Exception:
         return None
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy in float64 (counts and genome indices are exact there).  When the arrays exceed
+    DUMP_BYTES (the dense tables of a large database), those with one row per row of "ci" keep a seeded sample of their
+    rows, the same rows in every run, whose indices go to sampled_rows.npy."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        n = arrays["ci"].shape[0]
+        keep = np.sort(np.random.default_rng(SEED).choice(n, n * DUMP_BYTES // (2 * total), replace=False))
+        arrays = {k: (a[keep] if a.shape[0] == n else a) for k, a in arrays.items()}
+        arrays["sampled_rows"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def synth_params(G, paired):
@@ -368,6 +391,20 @@ def run_native(args):
         q.close()
         return ni, st
 
+    def step_outputs(ni):
+        """copies of what the last step handed its caller: the dense tables, or the rows of the genomes with a hit sorted
+        by genome (the library returns them in no particular order); and |I|"""
+        if os.environ.get("MLG_BENCH_READBACK_ALL") or os.environ.get("MLG_BENCH_DENSE_RESULT"):
+            out = {"ci": h_ci.numpy().reshape(G, nk)}
+            if os.environ.get("MLG_BENCH_READBACK_ALL"):
+                out.update(num=h_num.numpy().reshape(G, nk), den=h_den.numpy().reshape(G, nk))
+        else:
+            g = h_rows_g.numpy()[:rows[0]]
+            order = np.argsort(g, kind="stable")
+            out = {"genomes": g[order], "ci": h_rows_ci.numpy()[:rows[0] * nk].reshape(-1, nk)[order]}
+        out["n_intersect"] = np.array([ni])
+        return {k: np.array(v, dtype=np.float64) for k, v in out.items()}
+
     def barrier():
         if world > 1:
             tdist.barrier()
@@ -399,6 +436,7 @@ def run_native(args):
 
     sampler = ClockSampler(local) if rank == 0 else None
     ms_dev, wall_dev, st_dev, ni, clocks = timed(False, args.steps, args.warmup, sampler)
+    outputs = step_outputs(ni) if args.dump_outputs and rank == 0 else None
     ms_e2e, wall_e2e, st_e2e, ni2, _ = timed(True, args.steps, args.warmup)
     assert ni == ni2
     ni3, _ = step(False, readback_all=True)          # untimed: the integer tables for the oracle check below
@@ -516,6 +554,8 @@ def run_native(args):
         tdist.destroy_process_group()
     if rank != 0:
         return
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     # ---- CPU legs on rank 0, after every collective: cpu_baseline (N = 1) and the oracle check of the job's table
     line["cpu_baseline"] = None
     line["parity_checked"] = False
@@ -558,7 +598,13 @@ def main():
     ap.add_argument("--workload", default=os.environ.get("MLG_BENCH_WORKLOAD", "weak"), choices=sorted(WORKLOADS),
                     help="weak: 10M reads per GPU (configs[1] at one GPU); strong: configs[2], 100M reads sharded; "
                          "stream: configs[3], 500M reads streamed in batches; stress: configs[4], 10x database")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float64, at most 64 MB; native arm)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs needs --impl native")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -3,6 +3,7 @@
 //   ncu --metrics dram__bytes_read.sum,lts__t_sectors_srcunit_tex_op_read.sum,lts__t_requests_srcunit_tex_op_read.sum,gpu__time_duration.sum
 // to see how many DRAM bytes and L2 sectors ONE access costs for each flavour; without ncu it prints the rate.
 //   gather [log2 words = 28] [loads per thread = 64] [L2 fetch granularity limit = 0 (leave)] [policy window: 0 none, 1 streaming, 2 normal]
+// Build: nvcc -O3 -gencode arch=compute_100a,code=sm_100a -o scripts/ubench/gather scripts/ubench/gather.cu
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>

@@ -3,6 +3,7 @@ order, whatever the world size; the reference arm takes the native arm's first b
 import importlib.util
 import os
 
+import numpy as np
 import pytest
 
 from conftest import ROOT
@@ -38,3 +39,34 @@ def test_env_overrides(monkeypatch):
     G, paired, batches, total, desc = bench.workload_plan("stream", 3, 1)
     assert G == 1234 and total == 1_000_000
     assert batches[0][0] == 333_334 and sum(n for _, n in batches) == 333_333 and max(n for _, n in batches) == 300_000
+
+
+def test_dump_outputs_within_budget(tmp_path, monkeypatch):
+    """--dump-outputs: every array as float64; over the budget, tables keep a seeded sample of rows, the same in every run"""
+    G, nk = 10_000, 4
+    ci = np.random.default_rng(1).random((G, nk))
+    num = np.arange(G * nk, dtype=np.int64).reshape(G, nk)
+    arrays = {"ci": ci, "num": num, "n_intersect": np.array([123456789], dtype=np.uint64)}
+    bench.dump_outputs(str(tmp_path / "whole"), arrays)
+    assert np.array_equal(np.load(tmp_path / "whole" / "ci.npy"), ci)
+    assert not (tmp_path / "whole" / "sampled_rows.npy").exists()
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 16)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    got = {f: np.load(tmp_path / "a" / f) for f in sorted(os.listdir(tmp_path / "a"))}
+    assert sorted(got) == ["ci.npy", "n_intersect.npy", "num.npy", "sampled_rows.npy"]
+    assert all(a.dtype == np.float64 for a in got.values()) and sum(a.nbytes for a in got.values()) <= 1 << 16
+    rows = got["sampled_rows.npy"].astype(np.int64)
+    assert rows.size > 0 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(got["ci.npy"], ci[rows]) and np.array_equal(got["num.npy"], num[rows])
+    assert got["n_intersect.npy"].tolist() == [123456789.0]
+    for f, a in got.items():
+        assert np.array_equal(np.load(tmp_path / "b" / f), a)
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "d"]])
+def test_bad_arguments_are_refused(argv, monkeypatch):
+    monkeypatch.setattr(bench.sys, "argv", ["bench.py"] + argv)
+    with pytest.raises(SystemExit) as e:
+        bench.main()
+    assert e.value.code == 2

@@ -1,6 +1,7 @@
 """metalign_b200/h5min.py -- the minimal HDF5 reader that lets scripts/make_db_from_h5.py read CMash's training database
-(select_db.py:69) without h5py -- pinned on a REAL HDF5 file of the image (written by MATLAB's HDF5 library; scipy ships it
-as test data) and on files made by the independent writer tests/h5write.py in CMash's layout (SURVEY.md A.2)."""
+(select_db.py:69) without h5py -- pinned on a REAL HDF5 file (written by MATLAB's HDF5 library: tests/golden/testhdf5_7.4_GLNX86.mat,
+a copy of scipy's test file scipy/io/matlab/tests/data/testhdf5_7.4_GLNX86.mat, BSD-3-Clause) and on files made by the
+independent writer tests/h5write.py in CMash's layout (SURVEY.md A.2)."""
 import importlib.util
 import os
 import random
@@ -12,24 +13,13 @@ import h5write
 from metalign_b200 import codec, dbformat, h5min
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def _real_hdf5_file():
-    try:
-        import scipy.io
-    except ImportError:
-        return None
-    p = os.path.join(os.path.dirname(scipy.io.__file__), "matlab", "tests", "data", "testhdf5_7.4_GLNX86.mat")
-    return p if os.path.exists(p) else None
+REAL_HDF5 = os.path.join(ROOT, "tests", "golden", "testhdf5_7.4_GLNX86.mat")
 
 
 def test_reads_a_real_hdf5_file():
     """a MATLAB v7.3 file = HDF5 behind a 512-byte user block: superblock 0, old-style root group, one float64 dataset with
     an attribute.  scipy's own tests say what the variable holds in the sibling files of other formats: theta = 0, pi/4 .. 2 pi"""
-    p = _real_hdf5_file()
-    if p is None:
-        pytest.skip("scipy's MATLAB test data is not installed")
-    with h5min.H5File(p) as f:
+    with h5min.H5File(REAL_HDF5) as f:
         assert f.base == 512 and f.keys() == ["testdouble"]
         d = f["testdouble"]
         assert isinstance(d, h5min.Dataset) and d.shape == (9, 1) and d.dtype == np.dtype("<f8")
