@@ -202,6 +202,47 @@ int mlg_query_dump_intersection(mlg_query* q, const char* dump_path, const char*
 int mlg_query_stats(mlg_query* q, mlg_stats* out);
 int mlg_query_free(mlg_query* q);
 
+/* Read k-mer table (off unless enabled): every canonical K-mer of the pushed reads with a count saturating at 255, the
+ * counting part of `kmc -k<K> -ci<min_count> -cs<counter_max>` (select_db.py:50-52), so that the two KMC databases the
+ * reference leaves in its temp dir (reads_60mers, 60mers_intersection) can be written.  The table lives on this rank's GPU
+ * and grows with the reads; max_table_bytes caps it (0 = no cap).  A table that would pass the cap, or whose allocation
+ * fails, stops counting: the query itself is unaffected and the read k-mer calls return MLG_ERR_NOMEM.  After any counter
+ * exchange (mlg_query_counts_*, mlg_query_exchange_*) they return MLG_ERR_STATE: the table is not merged across ranks.
+ * Without the table they return MLG_ERR_STATE too. */
+typedef struct mlg_read_kmer_stats {
+    uint64_t windows;        /* N-free K-long windows counted */
+    uint64_t distinct;       /* distinct canonical k-mers in the table */
+    uint64_t slots;          /* 16-byte slots of the table */
+    uint64_t bytes;          /* device bytes of the table */
+    uint64_t bytes_needed;   /* overflowed: the bytes the table would have needed */
+    uint32_t grows;          /* rehashes into a larger table */
+    uint32_t overflowed;     /* 1: the table passed its budget or could not be allocated */
+    double ms_count;         /* CUDA-event time of the count kernel launches */
+    double ms_rehash;        /* CUDA-event time of the rehash launches */
+    /* the last mlg_query_read_kmers / mlg_query_write_reads_kmc call */
+    uint64_t out_records;    /* k-mers selected */
+    uint64_t out_bytes;      /* bytes written (both files) */
+    double ms_compact;       /* selection of the slots >= min_count */
+    double ms_sort;          /* sort by key */
+    double ms_encode;        /* prefix table and .kmc_suf records */
+    double s_write;          /* seconds of copying back and writing the files */
+} mlg_read_kmer_stats;
+/* before the first push: also count every canonical K-mer of the pushed reads (K <= 60); max_table_bytes 0 = no cap */
+int mlg_query_enable_read_kmers(mlg_query* q, uint64_t max_table_bytes);
+/* after sync or finish: the read k-mers seen >= min_count times, counts saturated at counter_max, keys ascending; writes
+ * at most cap (hi,lo) pairs and counts, *n = their number */
+int mlg_query_read_kmers(mlg_query* q, uint32_t min_count, uint32_t counter_max, uint64_t* keys_out /* (hi,lo) */,
+                         uint8_t* counts_out, uint64_t cap, uint64_t* n);
+/* `kmc -k<K> -ci<min_count> -cs<counter_max>` of the pushed reads as <prefix>.kmc_pre / <prefix>.kmc_suf */
+int mlg_query_write_reads_kmc(mlg_query* q, const char* prefix, uint32_t min_count, uint32_t counter_max);
+/* after finish: `kmc_tools simple <reads> <db> intersect <prefix>`: the k-mers of I, count = the count column of
+ * mlg_query_dump_intersection.  Needs no read k-mer table. */
+int mlg_query_write_intersection_kmc(mlg_query* q, const char* prefix, uint32_t counter_max);
+/* Both files are written in the version-0 layout (one sorted table, what kmc_tools writes; lut_prefix_length = the
+ * smallest p >= 4 with (K - p) % 4 == 0, counter_size 1); the reads file has min_count / max_count = min_count /
+ * counter_max, the intersection file 1 / counter_max.  The stats join the compute stream. */
+int mlg_query_read_kmer_stats(mlg_query* q, mlg_read_kmer_stats* out);
+
 /* Sketch builder (offline): bottom-n MinHash sketch of G genomes, CMash semantics (MinHash.CountEstimator with
  * rev_comp=False, as MakeStreamingDNADatabase.py builds Metalign's training database): every K-long window of
  * text[genome_off[g] .. genome_off[g+1]) that consists of ACGT/acgt only is upper-cased and hashed with

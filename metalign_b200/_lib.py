@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("MLG_LIB_PATH") or os.path.join(_HERE, "libmetalign_b2
 _LIB = None
 
 
+MLG_ERR_NOMEM = -5
 MLG_ERR_RETRY = -6
 
 
@@ -30,6 +31,16 @@ class Stats(C.Structure):
                 ("h2d_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64), ("ms_probe", C.c_double),
                 ("ms_query", C.c_double), ("probe_launches", C.c_uint32), ("filter_words", C.c_uint32),
                 ("n_bucket_fetches", C.c_uint64), ("layout", C.c_uint32), ("reserved", C.c_uint32)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+class ReadKmerStats(C.Structure):
+    _fields_ = [("windows", C.c_uint64), ("distinct", C.c_uint64), ("slots", C.c_uint64), ("bytes", C.c_uint64),
+                ("bytes_needed", C.c_uint64), ("grows", C.c_uint32), ("overflowed", C.c_uint32), ("ms_count", C.c_double),
+                ("ms_rehash", C.c_double), ("out_records", C.c_uint64), ("out_bytes", C.c_uint64), ("ms_compact", C.c_double),
+                ("ms_sort", C.c_double), ("ms_encode", C.c_double), ("s_write", C.c_double)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
@@ -94,6 +105,11 @@ SIGNATURES = {
     "mlg_query_intersection": (C.c_int, [_vp, _u64p, C.c_uint64, C.POINTER(C.c_uint64)]),
     "mlg_query_dump_intersection": (C.c_int, [_vp, C.c_char_p, C.c_char_p, C.c_uint32]),
     "mlg_query_stats": (C.c_int, [_vp, C.POINTER(Stats)]),
+    "mlg_query_enable_read_kmers": (C.c_int, [_vp, C.c_uint64]),
+    "mlg_query_read_kmers": (C.c_int, [_vp, C.c_uint32, C.c_uint32, _u64p, _u8p, C.c_uint64, C.POINTER(C.c_uint64)]),
+    "mlg_query_write_reads_kmc": (C.c_int, [_vp, C.c_char_p, C.c_uint32, C.c_uint32]),
+    "mlg_query_write_intersection_kmc": (C.c_int, [_vp, C.c_char_p, C.c_uint32]),
+    "mlg_query_read_kmer_stats": (C.c_int, [_vp, C.POINTER(ReadKmerStats)]),
     "mlg_query_free": (C.c_int, [_vp]),
     "mlg_sketch_genomes": (C.c_int, [_vp, _vp, _u64p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint64, _u64p, _u32p, _vp, _vp]),
 }

@@ -155,8 +155,18 @@ class Database:
         check(_lib.lib().mlg_db_denominators(self._h, int(count_empty_in_den), den.ctypes.data))
         return den
 
-    def query(self, ci_min: int = 2, gate: str = "exact", count_empty_in_den: bool = True) -> "Query":
-        return Query(self, ci_min, gate, count_empty_in_den)
+    def query(self, ci_min: int = 2, gate: str = "exact", count_empty_in_den: bool = True, read_kmers: bool = False,
+              read_kmer_budget: int = 0) -> "Query":
+        """read_kmers: also count every canonical K-mer of the pushed reads (K <= 60; Query.read_kmers /
+        write_reads_kmc); read_kmer_budget caps that table's device bytes (0 = no cap)"""
+        q = Query(self, ci_min, gate, count_empty_in_den)
+        if read_kmers:
+            try:
+                check(_lib.lib().mlg_query_enable_read_kmers(q._h, int(read_kmer_budget)))
+            except BaseException:
+                q.close()
+                raise
+        return q
 
     def close(self):
         if self._h:
@@ -348,6 +358,30 @@ class Query:
         counter_max = the -cs3 of both KMC runs of the reference"""
         check(_lib.lib().mlg_query_dump_intersection(self._h, dump_path.encode(), fasta_path.encode() if fasta_path else None,
                                                      int(counter_max)))
+
+    def read_kmers(self, min_count: int = 1, counter_max: int = 255):
+        """(keys uint64[n, 2] as (hi, lo), ascending; counts uint8[n] saturated at counter_max) of the read k-mers seen
+        >= min_count times (needs Database.query(read_kmers=True))"""
+        cap = self.read_kmer_stats()["distinct"]
+        keys = np.empty((cap, 2), dtype=np.uint64)
+        counts = np.empty(cap, dtype=np.uint8)
+        n = C.c_uint64()
+        check(_lib.lib().mlg_query_read_kmers(self._h, int(min_count), int(counter_max), keys.ctypes.data, counts.ctypes.data,
+                                              cap, C.byref(n)))
+        return keys[:n.value], counts[:n.value]
+
+    def write_reads_kmc(self, prefix: str, min_count: int = 2, counter_max: int = 3) -> None:
+        """<prefix>.kmc_pre / .kmc_suf: `kmc -k<K> -ci<min_count> -cs<counter_max>` of the pushed reads (select_db.py:50)"""
+        check(_lib.lib().mlg_query_write_reads_kmc(self._h, prefix.encode(), int(min_count), int(counter_max)))
+
+    def write_intersection_kmc(self, prefix: str, counter_max: int = 3) -> None:
+        """after finish: <prefix>.kmc_pre / .kmc_suf of `kmc_tools simple ... intersect` (select_db.py:54-56)"""
+        check(_lib.lib().mlg_query_write_intersection_kmc(self._h, prefix.encode(), int(counter_max)))
+
+    def read_kmer_stats(self) -> dict:
+        s = _lib.ReadKmerStats()
+        check(_lib.lib().mlg_query_read_kmer_stats(self._h, C.byref(s)))
+        return s.as_dict()
 
     def stats(self) -> dict:
         s = Stats()

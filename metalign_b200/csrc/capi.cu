@@ -150,6 +150,10 @@ struct mlg_query {
     // so that the 0.1 GB memset runs beside the probe kernel instead of behind it
     DevBuf<uint32_t> hitbits;
     DevBuf<unsigned long long> d_num;
+    // read k-mer table (mlg_query_enable_read_kmers; null = off) and what its last output stage measured
+    ReadKmerTable* rk = nullptr;
+    KmcOutStats rk_out;
+    bool exchanged = false;                        // counters went through an exchange: the per-rank table no longer matches
 };
 
 namespace {
@@ -196,8 +200,14 @@ int run_probe(mlg_query* q, Staging& s, const unsigned char* d_bases, const unsi
         CUDA_TRY(cudaEventRecord(e1, ctx->s_comp));
         q->probe_events.emplace_back(e0, e1);
         q->st.gpu_launches += 1; q->st.probe_launches += 1;
+        if (q->rk) MLG_TRY(rk_count_range(q->rk, a, nbases, &q->st.gpu_launches));
         return MLG_OK;
     };
+    if (q->rk) {
+        const uint32_t K = q->db->v.K;
+        const unsigned long long windows = read_len ? n_reads * (read_len >= K ? read_len - K + 1ull : 0ull) : nbases;   // upper bound
+        MLG_TRY(rk_before_batch(q->rk, windows, &q->st.gpu_launches));
+    }
     if (ranges) {
         unsigned long long r0 = 0;
         for (auto& rr : *ranges) {
@@ -212,6 +222,7 @@ int run_probe(mlg_query* q, Staging& s, const unsigned char* d_bases, const unsi
     } else {
         MLG_TRY(launch_range(0, n_reads));
     }
+    if (q->rk) MLG_TRY(rk_after_batch(q->rk, q->cur));
     if (!s.done) CUDA_TRY(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
     CUDA_TRY(cudaEventRecord(s.done, ctx->s_comp));
     s.used = true;
@@ -571,6 +582,7 @@ MLG_API int mlg_query_counts_export(mlg_query* q, uint8_t** d_counts, uint64_t* 
     if (!q || !d_counts || !n_counts) { mlg_set_error("null argument"); return MLG_ERR_ARG; }
     if (q->finished) { mlg_set_error("query already finished"); return MLG_ERR_STATE; }
     MLG_TRY(ensure_device(q->ctx));
+    q->exchanged = true;
     if (q->touched.p) {     // nothing pushed: every counter is still zero
         MLG_TRY(launch_clamp_counts(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ci_min, q->ctx->s_comp));
         q->st.gpu_launches += 1;
@@ -584,6 +596,7 @@ MLG_API int mlg_query_counts_export_sparse(mlg_query* q, uint64_t** d_entries, u
     if (q->finished) { mlg_set_error("query already finished"); return MLG_ERR_STATE; }
     if (q->merged || q->reduced) { mlg_set_error("counters were already combined across ranks"); return MLG_ERR_STATE; }
     MLG_TRY(ensure_device(q->ctx));
+    q->exchanged = true;
     *d_entries = nullptr; *n_entries = 0;
     if (!q->touched.p) return MLG_OK;                      // nothing pushed: no non-zero counter
     cudaStream_t st = q->ctx->s_comp;
@@ -603,7 +616,7 @@ MLG_API int mlg_query_counts_merge_sparse(mlg_query* q, const uint64_t* d_entrie
     if (q->finished) { mlg_set_error("query already finished"); return MLG_ERR_STATE; }
     if (q->reduced) { mlg_set_error("counters were already reduced densely"); return MLG_ERR_STATE; }
     MLG_TRY(ensure_device(q->ctx));
-    q->merged = true;
+    q->merged = true; q->exchanged = true;
     if (!n_entries) return MLG_OK;
     if (!d_entries) { mlg_set_error("null entries"); return MLG_ERR_ARG; }
     if (!q->present.p) { MLG_TRY(q->present.alloc((size_t)q->db->v.nd + 1)); MLG_TRY(q->touched.alloc((size_t)q->db->v.nd + 1)); }
@@ -614,7 +627,7 @@ MLG_API int mlg_query_counts_merge_sparse(mlg_query* q, const uint64_t* d_entrie
 }
 MLG_API int mlg_query_counts_import(mlg_query* q) {
     if (!q) { mlg_set_error("null query"); return MLG_ERR_ARG; }
-    q->reduced = true;
+    q->reduced = true; q->exchanged = true;
     return MLG_OK;
 }
 
@@ -689,6 +702,7 @@ static int check_exchange(mlg_query* q, mlg_exchange* ex) {
     if ((unsigned long long)q->ci_min * ex->world > 255ull) { mlg_set_error("ci_min * world must fit the 8-bit counters"); return MLG_ERR_ARG; }
     MLG_TRY(ensure_device(q->ctx));
     if (!q->present.p) { MLG_TRY(q->present.alloc((size_t)q->db->v.nd + 1)); MLG_TRY(q->touched.alloc((size_t)q->db->v.nd + 1)); }
+    q->exchanged = true;
     return MLG_OK;
 }
 // the probe kernels run on the compute stream, the copies feeding them on the copy stream, and every copy chunk is
@@ -743,7 +757,7 @@ MLG_API int mlg_query_exchange_dense(mlg_query* q, uint8_t** d_counts, uint64_t*
         q->st.gpu_launches += 1;
     }
     *d_counts = q->cnt8.p; *n_counts = q->db->v.nd;
-    q->reduced = true;
+    q->reduced = true; q->exchanged = true;
     return MLG_OK;
 }
 
@@ -961,6 +975,78 @@ MLG_API int mlg_query_dump_intersection(mlg_query* q, const char* dump_path, con
     return MLG_OK;
 }
 
+// ------------------------------------------------------------------ read k-mer table (csrc/readkmers.cu)
+MLG_API int mlg_query_enable_read_kmers(mlg_query* q, uint64_t max_table_bytes) {
+    if (!q) { mlg_set_error("null query"); return MLG_ERR_ARG; }
+    if (q->rk) return MLG_OK;
+    if (q->finished || q->exchanged || q->stg[0].used || q->stg[1].used) {
+        mlg_set_error("the read k-mer table must be enabled before the first push"); return MLG_ERR_STATE;
+    }
+    MLG_TRY(ensure_device(q->ctx));
+    return rk_create(q->ctx, q->db->v.K, max_table_bytes, &q->rk);
+}
+static int check_read_kmers(mlg_query* q, uint32_t min_count, uint32_t counter_max) {
+    if (!q) { mlg_set_error("null query"); return MLG_ERR_ARG; }
+    if (!q->rk) { mlg_set_error("the read k-mer table is off (mlg_query_enable_read_kmers)"); return MLG_ERR_STATE; }
+    if (q->exchanged) { mlg_set_error("the read k-mer table is per rank and the counters went through an exchange"); return MLG_ERR_STATE; }
+    if (min_count < 1 || min_count > 255 || counter_max < 1 || counter_max > 255) { mlg_set_error("min_count and counter_max must be 1..255"); return MLG_ERR_ARG; }
+    MLG_TRY(ensure_device(q->ctx));
+    return rk_check(q->rk);
+}
+MLG_API int mlg_query_read_kmers(mlg_query* q, uint32_t min_count, uint32_t counter_max, uint64_t* keys_out, uint8_t* counts_out,
+                                 uint64_t cap, uint64_t* n) {
+    if (!n) { mlg_set_error("null n"); return MLG_ERR_ARG; }
+    MLG_TRY(check_read_kmers(q, min_count, counter_max));
+    DevBuf<key128> keys; DevBuf<uint32_t> cnt;
+    uint32_t m = 0;
+    q->rk_out = KmcOutStats{};
+    MLG_TRY(rk_collect(q->rk, min_count, keys, cnt, &m, &q->rk_out));
+    q->rk_out.records = m;
+    *n = m;
+    const uint64_t c = std::min<uint64_t>(cap, m);
+    if (!c) return MLG_OK;
+    std::vector<uint32_t> hc(c);
+    if (keys_out) CUDA_TRY(cudaMemcpyAsync(keys_out, keys.p, c * sizeof(key128), cudaMemcpyDeviceToHost, q->ctx->s_comp));
+    CUDA_TRY(cudaMemcpyAsync(hc.data(), cnt.p, c * 4, cudaMemcpyDeviceToHost, q->ctx->s_comp));
+    CUDA_TRY(cudaStreamSynchronize(q->ctx->s_comp));
+    if (counts_out) for (uint64_t i = 0; i < c; ++i) counts_out[i] = (uint8_t)std::min(hc[i], counter_max);
+    return MLG_OK;
+}
+MLG_API int mlg_query_write_reads_kmc(mlg_query* q, const char* prefix, uint32_t min_count, uint32_t counter_max) {
+    if (!prefix) { mlg_set_error("null prefix"); return MLG_ERR_ARG; }
+    MLG_TRY(check_read_kmers(q, min_count, counter_max));
+    DevBuf<key128> keys; DevBuf<uint32_t> cnt;
+    uint32_t m = 0;
+    q->rk_out = KmcOutStats{};
+    MLG_TRY(rk_collect(q->rk, min_count, keys, cnt, &m, &q->rk_out));
+    return kmc_write(q->ctx, prefix, keys.p, cnt.p, m, q->db->v.K, min_count, counter_max, &q->rk_out);
+}
+MLG_API int mlg_query_write_intersection_kmc(mlg_query* q, const char* prefix, uint32_t counter_max) {
+    if (!q || !prefix) { mlg_set_error("null argument"); return MLG_ERR_ARG; }
+    if (!q->finished) { mlg_set_error("call mlg_query_finish first"); return MLG_ERR_STATE; }
+    if (counter_max == 0 || counter_max > 255) { mlg_set_error("counter_max must be 1..255"); return MLG_ERR_ARG; }
+    MLG_TRY(ensure_device(q->ctx));
+    const uint32_t n = q->n_present;
+    DevBuf<key128> d, keys; DevBuf<unsigned char> dc; DevBuf<uint32_t> cnt;
+    if (n) {
+        MLG_TRY(d.alloc(n)); MLG_TRY(dc.alloc(n));
+        MLG_TRY(launch_gather_keys(q->db->D_key.p, q->present.p, n, d.p, q->ctx->s_comp));
+        MLG_TRY(launch_gather_counts(q->cnt8.p, q->db->D_mult.p, q->present.p, n, counter_max, dc.p, q->ctx->s_comp));
+        MLG_TRY(rk_sort_pairs(q->ctx, d.p, dc.p, n, q->db->v.K, keys, cnt));
+    }
+    return kmc_write(q->ctx, prefix, keys.p, cnt.p, n, q->db->v.K, 1, counter_max, nullptr);
+}
+MLG_API int mlg_query_read_kmer_stats(mlg_query* q, mlg_read_kmer_stats* out) {
+    if (!q || !out) { mlg_set_error("null argument"); return MLG_ERR_ARG; }
+    if (!q->rk) { mlg_set_error("the read k-mer table is off (mlg_query_enable_read_kmers)"); return MLG_ERR_STATE; }
+    MLG_TRY(ensure_device(q->ctx));
+    MLG_TRY(rk_stats(q->rk, out));
+    out->out_records = q->rk_out.records; out->out_bytes = q->rk_out.bytes;
+    out->ms_compact = q->rk_out.ms_compact; out->ms_sort = q->rk_out.ms_sort; out->ms_encode = q->rk_out.ms_encode;
+    out->s_write = q->rk_out.s_write;
+    return MLG_OK;
+}
+
 MLG_API int mlg_query_stats(mlg_query* q, mlg_stats* out) {
     if (!q || !out) { mlg_set_error("null argument"); return MLG_ERR_ARG; }
     *out = q->st;
@@ -982,6 +1068,7 @@ MLG_API int mlg_query_free(mlg_query* q) {
         }
         if (ok) { std::swap(q->cnt8.p, q->db->clean_cnt8.p); std::swap(q->cnt8.n, q->db->clean_cnt8.n); }
     }
+    rk_destroy(q->rk);
     for (auto& pe : q->probe_events) { cudaEventDestroy(pe.first); cudaEventDestroy(pe.second); }
     for (auto& e : q->chunk_events) cudaEventDestroy(e);
     for (auto& s : q->stg) if (s.done) cudaEventDestroy(s.done);

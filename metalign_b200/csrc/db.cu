@@ -206,6 +206,8 @@ int sort_pairs_u32(const uint32_t* keys_in, uint32_t* keys_out, const uint32_t* 
     return MLG_OK;
 }
 
+}  // namespace
+
 // Sort n 2K-bit keys given as split (hi, lo) arrays; on return out[i] is the i-th smallest key and, if
 // vals is non-null, vals_out[i] the value that travelled with it.  LSD: by lo, then stably by hi.
 int sort_keys128(unsigned long long* hi, unsigned long long* lo, const uint32_t* vals, uint32_t n, uint32_t K,
@@ -243,6 +245,8 @@ int sort_keys128(unsigned long long* hi, unsigned long long* lo, const uint32_t*
     CUDA_TRY(cudaGetLastError());
     return MLG_OK;
 }
+
+namespace {
 
 // level-1 table geometry from the number of distinct keys: slots per bucket and number of buckets (a power of two)
 void choose_buckets(DbView& v, uint32_t nd) {

@@ -198,3 +198,23 @@ int launch_gather_hit_flags(const uint32_t* hitbits, unsigned long long words_pe
                             uint32_t nk, unsigned char* out, cudaStream_t st);
 int launch_gather_counts(const unsigned char* cnt8, const unsigned char* D_mult, const uint32_t* present, uint32_t n_present, uint32_t cap,
                          unsigned char* out, cudaStream_t st);
+
+// sort of split 2K-bit keys (db.cu), shared by the database build and the KMC writers
+int sort_keys128(unsigned long long* hi, unsigned long long* lo, const uint32_t* vals, uint32_t n, uint32_t K,
+                 key128* out, uint32_t* vals_out, cudaStream_t st);
+
+// ---- read k-mer table and KMC database writers (readkmers.cu) ----
+struct ReadKmerTable;
+struct KmcOutStats { double ms_compact = 0, ms_sort = 0, ms_encode = 0, s_write = 0; unsigned long long records = 0, bytes = 0; };
+int rk_create(mlg_ctx* ctx, uint32_t K, unsigned long long max_table_bytes, ReadKmerTable** out);
+void rk_destroy(ReadKmerTable* t);
+int rk_before_batch(ReadKmerTable* t, unsigned long long batch_windows, uint32_t* launches);   // growth (may launch a rehash)
+int rk_count_range(ReadKmerTable* t, const ProbeArgs& a, unsigned long long batch_bases, uint32_t* launches);   // a.r_begin..a.r_end
+int rk_after_batch(ReadKmerTable* t, int staging_set);
+int rk_check(ReadKmerTable* t);                // joins the streams; MLG_ERR_NOMEM once the table overflowed
+int rk_stats(ReadKmerTable* t, mlg_read_kmer_stats* out);
+int rk_collect(ReadKmerTable* t, uint32_t min_count, DevBuf<key128>& keys, DevBuf<uint32_t>& counts, uint32_t* n, KmcOutStats* ws);
+int rk_sort_pairs(mlg_ctx* ctx, const key128* keys, const unsigned char* counts, uint32_t n, uint32_t K, DevBuf<key128>& keys_out,
+                  DevBuf<uint32_t>& counts_out);
+int kmc_write(mlg_ctx* ctx, const char* prefix, const key128* keys, const uint32_t* counts, uint32_t n, uint32_t K, uint32_t min_count,
+              uint32_t counter_max, KmcOutStats* ws);

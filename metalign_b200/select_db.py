@@ -8,7 +8,7 @@ FASTA `cmashed_db.fna`, `subset_db_info.txt`).  What changes is behind `run_kmc_
 The database is the native file `data/cmash_db_n1000_k60.mlgdb` (metalign_b200.dbformat) in place of
 cmash_db_n1000_k60.h5 / _30-60-10.bf / _dump.kmc_* (select_db.py:44,69,70).
 
-Extra, optional flags (not in the reference): --db_file, --gate, --device, --k_range.
+Extra, optional flags (not in the reference): --db_file, --gate, --device, --k_range, --read_kmer_budget.
 """
 from __future__ import annotations
 
@@ -50,7 +50,9 @@ def select_parseargs(argv=None):
     p.add_argument("--dbinfo_in", default="AUTO", help="db_info file of the full database (default data/db_info.txt)")
     p.add_argument("--dbinfo_out", default="AUTO", help="where to write the subset db_info (default temp_dir/subset_db_info.txt)")
     p.add_argument("--input_type", default="AUTO", choices=["fastq", "fasta", "AUTO"], help="reads format (default: by extension)")
-    p.add_argument("--keep_temp_files", action="store_true", help="keep the intersection dump")
+    p.add_argument("--keep_temp_files", action="store_true",
+                   help="keep the intermediate files the reference keeps: the KMC databases of the reads (reads_60mers, "
+                        "-ci2 -cs3) and of the intersection (60mers_intersection), and the intersection dump")
     p.add_argument("--strain_level", action="store_true", help="keep every strain above the cutoff (default: one per species)")
     p.add_argument("--temp_dir", default="AUTO/", help="directory for intermediate files")
     p.add_argument("--threads", type=int, default=4, help="accepted for compatibility (KMC threads in the reference)")
@@ -58,6 +60,9 @@ def select_parseargs(argv=None):
     p.add_argument("--db_file", default="AUTO", help="native database file (default data/%s)" % DB_BASENAME)
     p.add_argument("--gate", default="exact", choices=["exact", "none"], help="smallest-k prefilter model (see DESIGN.md)")
     p.add_argument("--device", type=int, default=0, help="CUDA device")
+    p.add_argument("--read_kmer_budget", type=int, default=0,
+                   help="with --keep_temp_files: cap in bytes on the GPU table of read k-mers behind reads_60mers (0 = none); "
+                        "past it that database is skipped and everything else is still written")
     return p.parse_args(argv)
 
 
@@ -120,7 +125,9 @@ def run_kmc_steps(args):
         if "error" in box:
             raise box["error"]
         _tick("database loaded, reader started")
-        query = db.query(ci_min=2, gate=args.gate, count_empty_in_den=True)     # -ci2 (select_db.py:50)
+        # -ci2 (select_db.py:50); the read k-mer table only for the reads_60mers database --keep_temp_files leaves behind
+        query = db.query(ci_min=2, gate=args.gate, count_empty_in_den=True, read_kmers=bool(args.keep_temp_files),
+                         read_kmer_budget=args.read_kmer_budget)
         for bases, nruns, off, n_reads in reader:
             query.push_packed_nruns(bases, nruns if len(nruns) else None, off, n_reads)
         query.sync()
@@ -145,6 +152,7 @@ def run_cmash_and_cutoff(args, taxid2info):
     rule exactly as select_db.py:80-96 does, reading the CSV back in file order."""
     if args.cmash_results == "NONE":
         from . import cmash_tail, codec
+        from ._lib import MLG_ERR_NOMEM, MlgError
         ctx, db, query = args._mlg
         cmash_out = args.temp_dir + "cmash_query_results.csv"
         res = query.finish_sparse()                       # rows for the genomes with a hit: all the CSV can hold
@@ -155,6 +163,14 @@ def run_cmash_and_cutoff(args, taxid2info):
             # what kmc_dump and the FASTA rewrite leave in the temp dir (select_db.py:58-65): "<k-mer>\t<count>" lines
             # and the ">seq" records CMash is given
             query.dump_intersection(args.temp_dir + "60mers_intersection_dump", args.temp_dir + "60mers_intersection_dump.fa")
+            # the two KMC databases of select_db.py:50-56
+            query.write_intersection_kmc(args.temp_dir + "60mers_intersection", counter_max=3)
+            try:
+                query.write_reads_kmc(args.temp_dir + "reads_60mers", min_count=2, counter_max=3)
+            except MlgError as e:
+                if e.code != MLG_ERR_NOMEM:
+                    raise
+                sys.stderr.write("select_db: reads_60mers.kmc_* not written: %s\n" % e)
         if not getattr(args, "_mlg_leave_open", False):     # the command-line script exits right after: no point in freeing GBs first
             query.close(); db.close(); ctx.close()
         del args._mlg
@@ -212,7 +228,7 @@ def make_db_and_dbinfo(args, organisms_to_include, taxid2info):
 
 def _normalise(args):
     """AUTO / NONE resolution, same outcomes as select_db.py:126-153"""
-    for name, default in (("db_file", "AUTO"), ("gate", "exact"), ("device", 0)):
+    for name, default in (("db_file", "AUTO"), ("gate", "exact"), ("device", 0), ("read_kmer_budget", 0)):
         if not hasattr(args, name):
             setattr(args, name, default)       # Namespace handed over by the reference's metalign.py
     if not args.data.endswith("/"):
