@@ -235,6 +235,32 @@ int mlg_query_read_kmers(mlg_query* q, uint32_t min_count, uint32_t counter_max,
                          uint8_t* counts_out, uint64_t cap, uint64_t* n);
 /* `kmc -k<K> -ci<min_count> -cs<counter_max>` of the pushed reads as <prefix>.kmc_pre / <prefix>.kmc_suf */
 int mlg_query_write_reads_kmc(mlg_query* q, const char* prefix, uint32_t min_count, uint32_t counter_max);
+/* Key-range passes: a second mode of the same calls for read sets whose table would not fit.  Enabled before the first
+ * push instead of mlg_query_enable_read_kmers (either after the other, or after a push: MLG_ERR_STATE).  The pushes only
+ * copy the reads into a device archive (0.375 bytes per base; no kernel launch).  Every mlg_query_read_kmers /
+ * mlg_query_write_reads_kmc call then plans contiguous intervals of the canonical key order from a histogram of the
+ * archive and counts each interval in a table of its own, one after the other; the results are those of the single
+ * table.  max_bytes caps the archive plus one pass (0 = the free device memory at the output call, less 1 GiB).  An
+ * archive that would pass it, or whose allocation fails, stops archiving: the query is unaffected and the output calls
+ * return MLG_ERR_NOMEM, as they do when the cap leaves no room for the smallest pass.  Passes lift the 2^32 limit on the
+ * records of one call (each pass sorts < 2^32 keys).  In this mode mlg_read_kmer_stats describes the last output call:
+ * windows (from the histogram), distinct (summed over the passes), slots / bytes (of the largest pass), ms_count (summed),
+ * out_* as in the other mode; grows and ms_rehash are 0; bytes_needed, once the archive overflowed, what the archive of
+ * every batch pushed would need.  A failed mlg_query_write_reads_kmc leaves neither file behind. */
+int mlg_query_enable_read_kmer_passes(mlg_query* q, uint64_t max_bytes);
+typedef struct mlg_read_kmer_plan {
+    uint32_t passes;         /* key-range passes of the last output call */
+    uint32_t refined_bins;   /* histogram bins that alone passed the cap and were split by their next bases */
+    uint64_t archive_bytes;  /* device copy of the reads */
+    uint64_t pass_cap_bytes; /* device bytes one pass may use: table + output stage */
+    uint64_t max_pass_bound; /* largest bound on the distinct keys of one pass */
+    uint64_t distinct;       /* distinct canonical k-mers, summed over the passes */
+    double ms_histogram;     /* CUDA-event time of the histogram launches */
+    double ms_count;         /* CUDA-event time of the ranged count launches */
+    double ms_output;        /* CUDA-event time of selection, sort and encoding */
+} mlg_read_kmer_plan;
+/* the plan of the last output call in passes mode (MLG_ERR_STATE in any other mode) */
+int mlg_query_read_kmer_plan(mlg_query* q, mlg_read_kmer_plan* out);
 /* after finish: `kmc_tools simple <reads> <db> intersect <prefix>`: the k-mers of I, count = the count column of
  * mlg_query_dump_intersection.  Needs no read k-mer table. */
 int mlg_query_write_intersection_kmc(mlg_query* q, const char* prefix, uint32_t counter_max);

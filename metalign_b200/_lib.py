@@ -46,6 +46,15 @@ class ReadKmerStats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class ReadKmerPlan(C.Structure):
+    _fields_ = [("passes", C.c_uint32), ("refined_bins", C.c_uint32), ("archive_bytes", C.c_uint64), ("pass_cap_bytes", C.c_uint64),
+                ("max_pass_bound", C.c_uint64), ("distinct", C.c_uint64), ("ms_histogram", C.c_double), ("ms_count", C.c_double),
+                ("ms_output", C.c_double)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
 def build(force: bool = False) -> str:
     """Compile the CUDA sources for sm_100a (nvcc cross-compiles without a GPU)."""
     src_dir = os.path.join(_HERE, "csrc")
@@ -110,6 +119,8 @@ SIGNATURES = {
     "mlg_query_write_reads_kmc": (C.c_int, [_vp, C.c_char_p, C.c_uint32, C.c_uint32]),
     "mlg_query_write_intersection_kmc": (C.c_int, [_vp, C.c_char_p, C.c_uint32]),
     "mlg_query_read_kmer_stats": (C.c_int, [_vp, C.POINTER(ReadKmerStats)]),
+    "mlg_query_enable_read_kmer_passes": (C.c_int, [_vp, C.c_uint64]),
+    "mlg_query_read_kmer_plan": (C.c_int, [_vp, C.POINTER(ReadKmerPlan)]),
     "mlg_query_free": (C.c_int, [_vp]),
     "mlg_sketch_genomes": (C.c_int, [_vp, _vp, _u64p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint64, _u64p, _u32p, _vp, _vp]),
 }

@@ -156,13 +156,17 @@ class Database:
         return den
 
     def query(self, ci_min: int = 2, gate: str = "exact", count_empty_in_den: bool = True, read_kmers: bool = False,
-              read_kmer_budget: int = 0) -> "Query":
+              read_kmer_budget: int = 0, read_kmer_passes: bool = False) -> "Query":
         """read_kmers: also count every canonical K-mer of the pushed reads (K <= 60; Query.read_kmers /
-        write_reads_kmc); read_kmer_budget caps that table's device bytes (0 = no cap)"""
+        write_reads_kmc); read_kmer_budget caps that table's device bytes (0 = no cap).  read_kmer_passes: count them
+        instead in key-range passes over a device copy of the reads at each output call, for read sets whose table would
+        not fit; read_kmer_budget then caps the copy plus one pass (0 = the free device memory)"""
         q = Query(self, ci_min, gate, count_empty_in_den)
         if read_kmers:
             try:
-                check(_lib.lib().mlg_query_enable_read_kmers(q._h, int(read_kmer_budget)))
+                enable = _lib.lib().mlg_query_enable_read_kmer_passes if read_kmer_passes else _lib.lib().mlg_query_enable_read_kmers
+                check(enable(q._h, int(read_kmer_budget)))
+                q._rk_passes = bool(read_kmer_passes)
             except BaseException:
                 q.close()
                 raise
@@ -185,6 +189,7 @@ class Query:
         check(_lib.lib().mlg_query_begin(db.ctx._h, db._h, int(ci_min), GATE[gate], int(count_empty_in_den),
                                          C.byref(self._h)))
         self._keep = []   # host buffers that must outlive the asynchronous copies
+        self._rk_passes = False
 
     def push_packed(self, bases: np.ndarray, nmask: Optional[np.ndarray], off: Optional[np.ndarray],
                     n_reads: int, read_len: int = 0):
@@ -362,10 +367,14 @@ class Query:
     def read_kmers(self, min_count: int = 1, counter_max: int = 255):
         """(keys uint64[n, 2] as (hi, lo), ascending; counts uint8[n] saturated at counter_max) of the read k-mers seen
         >= min_count times (needs Database.query(read_kmers=True))"""
-        cap = self.read_kmer_stats()["distinct"]
+        n = C.c_uint64()
+        if self._rk_passes:       # the number of records is only known after the passes have run: count them first
+            check(_lib.lib().mlg_query_read_kmers(self._h, int(min_count), int(counter_max), None, None, 0, C.byref(n)))
+            cap = n.value
+        else:
+            cap = self.read_kmer_stats()["distinct"]
         keys = np.empty((cap, 2), dtype=np.uint64)
         counts = np.empty(cap, dtype=np.uint8)
-        n = C.c_uint64()
         check(_lib.lib().mlg_query_read_kmers(self._h, int(min_count), int(counter_max), keys.ctypes.data, counts.ctypes.data,
                                               cap, C.byref(n)))
         return keys[:n.value], counts[:n.value]
@@ -381,6 +390,13 @@ class Query:
     def read_kmer_stats(self) -> dict:
         s = _lib.ReadKmerStats()
         check(_lib.lib().mlg_query_read_kmer_stats(self._h, C.byref(s)))
+        return s.as_dict()
+
+    def read_kmer_plan(self) -> dict:
+        """mlg_query_read_kmer_plan: passes, refined bins, archive bytes, per-pass cap, largest pass bound, distinct keys and
+        event times of the last read_kmers / write_reads_kmc call (needs Database.query(read_kmer_passes=True))"""
+        s = _lib.ReadKmerPlan()
+        check(_lib.lib().mlg_query_read_kmer_plan(self._h, C.byref(s)))
         return s.as_dict()
 
     def stats(self) -> dict:

@@ -152,6 +152,7 @@ struct mlg_query {
     DevBuf<unsigned long long> d_num;
     // read k-mer table (mlg_query_enable_read_kmers; null = off) and what its last output stage measured
     ReadKmerTable* rk = nullptr;
+    ReadKmerPasses* rkp = nullptr;                 // the key-range mode instead (mlg_query_enable_read_kmer_passes; null = off)
     KmcOutStats rk_out;
     bool exchanged = false;                        // counters went through an exchange: the per-rank table no longer matches
 };
@@ -223,6 +224,7 @@ int run_probe(mlg_query* q, Staging& s, const unsigned char* d_bases, const unsi
         MLG_TRY(launch_range(0, n_reads));
     }
     if (q->rk) MLG_TRY(rk_after_batch(q->rk, q->cur));
+    if (q->rkp) MLG_TRY(rkp_archive(q->rkp, a, n_reads, nbases));
     if (!s.done) CUDA_TRY(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
     CUDA_TRY(cudaEventRecord(s.done, ctx->s_comp));
     s.used = true;
@@ -979,27 +981,39 @@ MLG_API int mlg_query_dump_intersection(mlg_query* q, const char* dump_path, con
 MLG_API int mlg_query_enable_read_kmers(mlg_query* q, uint64_t max_table_bytes) {
     if (!q) { mlg_set_error("null query"); return MLG_ERR_ARG; }
     if (q->rk) return MLG_OK;
+    if (q->rkp) { mlg_set_error("read k-mer passes are already enabled on this query"); return MLG_ERR_STATE; }
     if (q->finished || q->exchanged || q->stg[0].used || q->stg[1].used) {
         mlg_set_error("the read k-mer table must be enabled before the first push"); return MLG_ERR_STATE;
     }
     MLG_TRY(ensure_device(q->ctx));
     return rk_create(q->ctx, q->db->v.K, max_table_bytes, &q->rk);
 }
+MLG_API int mlg_query_enable_read_kmer_passes(mlg_query* q, uint64_t max_bytes) {
+    if (!q) { mlg_set_error("null query"); return MLG_ERR_ARG; }
+    if (q->rkp) return MLG_OK;
+    if (q->rk) { mlg_set_error("the read k-mer table is already enabled on this query"); return MLG_ERR_STATE; }
+    if (q->finished || q->exchanged || q->stg[0].used || q->stg[1].used) {
+        mlg_set_error("read k-mer passes must be enabled before the first push"); return MLG_ERR_STATE;
+    }
+    MLG_TRY(ensure_device(q->ctx));
+    return rkp_create(q->ctx, q->db->v.K, max_bytes, &q->rkp);
+}
 static int check_read_kmers(mlg_query* q, uint32_t min_count, uint32_t counter_max) {
     if (!q) { mlg_set_error("null query"); return MLG_ERR_ARG; }
-    if (!q->rk) { mlg_set_error("the read k-mer table is off (mlg_query_enable_read_kmers)"); return MLG_ERR_STATE; }
+    if (!q->rk && !q->rkp) { mlg_set_error("the read k-mer table is off (mlg_query_enable_read_kmers)"); return MLG_ERR_STATE; }
     if (q->exchanged) { mlg_set_error("the read k-mer table is per rank and the counters went through an exchange"); return MLG_ERR_STATE; }
     if (min_count < 1 || min_count > 255 || counter_max < 1 || counter_max > 255) { mlg_set_error("min_count and counter_max must be 1..255"); return MLG_ERR_ARG; }
     MLG_TRY(ensure_device(q->ctx));
-    return rk_check(q->rk);
+    return q->rk ? rk_check(q->rk) : rkp_check(q->rkp);
 }
 MLG_API int mlg_query_read_kmers(mlg_query* q, uint32_t min_count, uint32_t counter_max, uint64_t* keys_out, uint8_t* counts_out,
                                  uint64_t cap, uint64_t* n) {
     if (!n) { mlg_set_error("null n"); return MLG_ERR_ARG; }
     MLG_TRY(check_read_kmers(q, min_count, counter_max));
+    q->rk_out = KmcOutStats{};
+    if (q->rkp) return rkp_read_kmers(q->rkp, min_count, counter_max, keys_out, counts_out, cap, n, &q->rk_out);
     DevBuf<key128> keys; DevBuf<uint32_t> cnt;
     uint32_t m = 0;
-    q->rk_out = KmcOutStats{};
     MLG_TRY(rk_collect(q->rk, min_count, keys, cnt, &m, &q->rk_out));
     q->rk_out.records = m;
     *n = m;
@@ -1015,9 +1029,10 @@ MLG_API int mlg_query_read_kmers(mlg_query* q, uint32_t min_count, uint32_t coun
 MLG_API int mlg_query_write_reads_kmc(mlg_query* q, const char* prefix, uint32_t min_count, uint32_t counter_max) {
     if (!prefix) { mlg_set_error("null prefix"); return MLG_ERR_ARG; }
     MLG_TRY(check_read_kmers(q, min_count, counter_max));
+    q->rk_out = KmcOutStats{};
+    if (q->rkp) return rkp_write_kmc(q->rkp, prefix, min_count, counter_max, &q->rk_out);
     DevBuf<key128> keys; DevBuf<uint32_t> cnt;
     uint32_t m = 0;
-    q->rk_out = KmcOutStats{};
     MLG_TRY(rk_collect(q->rk, min_count, keys, cnt, &m, &q->rk_out));
     return kmc_write(q->ctx, prefix, keys.p, cnt.p, m, q->db->v.K, min_count, counter_max, &q->rk_out);
 }
@@ -1038,13 +1053,18 @@ MLG_API int mlg_query_write_intersection_kmc(mlg_query* q, const char* prefix, u
 }
 MLG_API int mlg_query_read_kmer_stats(mlg_query* q, mlg_read_kmer_stats* out) {
     if (!q || !out) { mlg_set_error("null argument"); return MLG_ERR_ARG; }
-    if (!q->rk) { mlg_set_error("the read k-mer table is off (mlg_query_enable_read_kmers)"); return MLG_ERR_STATE; }
+    if (!q->rk && !q->rkp) { mlg_set_error("the read k-mer table is off (mlg_query_enable_read_kmers)"); return MLG_ERR_STATE; }
     MLG_TRY(ensure_device(q->ctx));
-    MLG_TRY(rk_stats(q->rk, out));
+    MLG_TRY(q->rk ? rk_stats(q->rk, out) : rkp_stats(q->rkp, out));
     out->out_records = q->rk_out.records; out->out_bytes = q->rk_out.bytes;
     out->ms_compact = q->rk_out.ms_compact; out->ms_sort = q->rk_out.ms_sort; out->ms_encode = q->rk_out.ms_encode;
     out->s_write = q->rk_out.s_write;
     return MLG_OK;
+}
+MLG_API int mlg_query_read_kmer_plan(mlg_query* q, mlg_read_kmer_plan* out) {
+    if (!q || !out) { mlg_set_error("null argument"); return MLG_ERR_ARG; }
+    if (!q->rkp) { mlg_set_error("read k-mer passes are off (mlg_query_enable_read_kmer_passes)"); return MLG_ERR_STATE; }
+    return rkp_plan(q->rkp, out);
 }
 
 MLG_API int mlg_query_stats(mlg_query* q, mlg_stats* out) {
@@ -1069,6 +1089,7 @@ MLG_API int mlg_query_free(mlg_query* q) {
         if (ok) { std::swap(q->cnt8.p, q->db->clean_cnt8.p); std::swap(q->cnt8.n, q->db->clean_cnt8.n); }
     }
     rk_destroy(q->rk);
+    rkp_destroy(q->rkp);
     for (auto& pe : q->probe_events) { cudaEventDestroy(pe.first); cudaEventDestroy(pe.second); }
     for (auto& e : q->chunk_events) cudaEventDestroy(e);
     for (auto& s : q->stg) if (s.done) cudaEventDestroy(s.done);

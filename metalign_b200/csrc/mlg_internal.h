@@ -218,3 +218,15 @@ int rk_sort_pairs(mlg_ctx* ctx, const key128* keys, const unsigned char* counts,
                   DevBuf<uint32_t>& counts_out);
 int kmc_write(mlg_ctx* ctx, const char* prefix, const key128* keys, const uint32_t* counts, uint32_t n, uint32_t K, uint32_t min_count,
               uint32_t counter_max, KmcOutStats* ws);
+// key-range passes (mlg_query_enable_read_kmer_passes): the pushes archive the reads on the device, every output call
+// counts them in passes over contiguous intervals of the key order
+struct ReadKmerPasses;
+int rkp_create(mlg_ctx* ctx, uint32_t K, unsigned long long max_bytes, ReadKmerPasses** out);
+void rkp_destroy(ReadKmerPasses* t);
+int rkp_archive(ReadKmerPasses* t, const ProbeArgs& a, unsigned long long n_reads, unsigned long long nbases);   // no kernel
+int rkp_check(ReadKmerPasses* t);              // joins the streams; MLG_ERR_NOMEM once the archive overflowed
+int rkp_read_kmers(ReadKmerPasses* t, uint32_t min_count, uint32_t counter_max, uint64_t* keys_out, uint8_t* counts_out, uint64_t cap,
+                   uint64_t* n_total, KmcOutStats* ws);
+int rkp_write_kmc(ReadKmerPasses* t, const char* prefix, uint32_t min_count, uint32_t counter_max, KmcOutStats* ws);
+int rkp_stats(ReadKmerPasses* t, mlg_read_kmer_stats* out);
+int rkp_plan(ReadKmerPasses* t, mlg_read_kmer_plan* out);

@@ -8,7 +8,8 @@ FASTA `cmashed_db.fna`, `subset_db_info.txt`).  What changes is behind `run_kmc_
 The database is the native file `data/cmash_db_n1000_k60.mlgdb` (metalign_b200.dbformat) in place of
 cmash_db_n1000_k60.h5 / _30-60-10.bf / _dump.kmc_* (select_db.py:44,69,70).
 
-Extra, optional flags (not in the reference): --db_file, --gate, --device, --k_range, --read_kmer_budget.
+Extra, optional flags (not in the reference): --db_file, --gate, --device, --k_range, --read_kmer_budget,
+--read_kmer_passes.
 """
 from __future__ import annotations
 
@@ -63,6 +64,10 @@ def select_parseargs(argv=None):
     p.add_argument("--read_kmer_budget", type=int, default=0,
                    help="with --keep_temp_files: cap in bytes on the GPU table of read k-mers behind reads_60mers (0 = none); "
                         "past it that database is skipped and everything else is still written")
+    p.add_argument("--read_kmer_passes", action="store_true",
+                   help="with --keep_temp_files: count the k-mers behind reads_60mers in key-range passes over a GPU copy of "
+                        "the reads, for read sets whose table would not fit in one GPU; --read_kmer_budget then caps that "
+                        "copy plus one pass, and only reads that do not fit themselves skip the database")
     return p.parse_args(argv)
 
 
@@ -127,7 +132,7 @@ def run_kmc_steps(args):
         _tick("database loaded, reader started")
         # -ci2 (select_db.py:50); the read k-mer table only for the reads_60mers database --keep_temp_files leaves behind
         query = db.query(ci_min=2, gate=args.gate, count_empty_in_den=True, read_kmers=bool(args.keep_temp_files),
-                         read_kmer_budget=args.read_kmer_budget)
+                         read_kmer_budget=args.read_kmer_budget, read_kmer_passes=args.read_kmer_passes)
         for bases, nruns, off, n_reads in reader:
             query.push_packed_nruns(bases, nruns if len(nruns) else None, off, n_reads)
         query.sync()
@@ -228,7 +233,8 @@ def make_db_and_dbinfo(args, organisms_to_include, taxid2info):
 
 def _normalise(args):
     """AUTO / NONE resolution, same outcomes as select_db.py:126-153"""
-    for name, default in (("db_file", "AUTO"), ("gate", "exact"), ("device", 0), ("read_kmer_budget", 0)):
+    for name, default in (("db_file", "AUTO"), ("gate", "exact"), ("device", 0), ("read_kmer_budget", 0),
+                          ("read_kmer_passes", False)):
         if not hasattr(args, name):
             setattr(args, name, default)       # Namespace handed over by the reference's metalign.py
     if not args.data.endswith("/"):
