@@ -165,7 +165,10 @@ int mlg_query_counts_merge_sparse(mlg_query* q, const uint64_t* d_entries, uint6
  *                     every rank must call it once per query, in the same order.
  *   dense form:       mlg_query_exchange_dense() = mlg_query_counts_export() + _import() without the host join.
  * If some rank had more than cap_entries non-zero counters, nothing is merged on any rank and mlg_query_finish()
- * returns MLG_ERR_RETRY: repeat the exchange with a larger mlg_exchange and call finish again. */
+ * returns MLG_ERR_RETRY: repeat the exchange with a larger mlg_exchange and call finish again.  Every rank judges all
+ * world counts, its own included, so every rank gets the same answer, and the error message names the largest count.
+ * Every form leaves the same counters on every rank: the sum over ranks of min(count, ci_min).  The pack calls
+ * (mlg_query_counts_export*, mlg_query_exchange_pack / _p2p / _dense) clamp the rank's own counters to ci_min in place. */
 int mlg_exchange_create(mlg_ctx* ctx, uint32_t world, uint32_t rank, uint64_t cap_entries, mlg_exchange** out);
 int mlg_exchange_destroy(mlg_exchange* ex);
 int mlg_exchange_buffers(mlg_exchange* ex, uint64_t** d_send, uint64_t** d_recv, uint64_t* block_words);
@@ -196,8 +199,8 @@ int mlg_query_intersection(mlg_query* q, uint64_t* keys_out, uint64_t cap, uint6
  * for, the ">seq" / k-mer records of 60mers_intersection_dump.fa.  count = what `kmc_tools simple ... intersect` keeps: the
  * smaller of the k-mer's occurrences in the reads and the number of sketch slots that hold it, both saturated at
  * counter_max (the reference builds both KMC databases with -cs3: select_db.py:50, retrain_and_test_metalign.sh:66).
- * Exact for a query whose reads were all pushed here; after a multi-GPU exchange the read counters are sums of per-rank
- * counters clamped to ci_min. */
+ * Exact for a query whose reads were all pushed here; after a multi-GPU exchange, in every form and on every rank, the
+ * read counter is the sum over ranks of the per-rank counters clamped to ci_min. */
 int mlg_query_dump_intersection(mlg_query* q, const char* dump_path, const char* fasta_path_or_null, uint32_t counter_max);
 int mlg_query_stats(mlg_query* q, mlg_stats* out);
 int mlg_query_free(mlg_query* q);

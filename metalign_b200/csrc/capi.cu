@@ -117,7 +117,8 @@ struct mlg_exchange {
     mlg_ctx* ctx = nullptr;
     uint32_t world = 1, rank = 0;
     unsigned long long cap = 0, block_words = 0;
-    DevBuf<unsigned long long> send, recv, status;     // status: [0] largest count of an overflowing exchange, [1] peer timeout, [2] CTA counter
+    DevBuf<unsigned long long> send, recv, status;     // status: [0] largest count of an overflowing exchange, [1] peer timeout,
+                                                       // [2] CTA counter, [3] this rank's count at the last pack
     unsigned long long* mailbox = nullptr;             // [world senders][2 parities][block_words], cudaMalloc'ed (IPC-exportable)
     unsigned long long* peer_mailbox[MLG_MAX_RANKS] = {};   // peers' mailboxes as mapped into this process (own slot unused)
     bool connected = false;
@@ -714,7 +715,8 @@ MLG_API int mlg_query_exchange_pack(mlg_query* q, mlg_exchange* ex) {
     MLG_TRY(check_exchange(q, ex));
     cudaStream_t st = q->ctx->s_comp;
     CUDA_TRY(cudaMemsetAsync(ex->status.p, 0, 16, st));
-    MLG_TRY(launch_pack_exchange(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ci_min, ex->send.p, ex->cap, st));
+    MLG_TRY(launch_pack_exchange(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ci_min, ex->send.p, ex->cap, ex->status.p + 3,
+                                 st));
     q->st.gpu_launches += 1;
     return MLG_OK;
 }
@@ -739,7 +741,7 @@ MLG_API int mlg_query_exchange_p2p(mlg_query* q, mlg_exchange* ex) {
         if (w != ex->rank) boxes[np++] = ex->peer_mailbox[w] + ((unsigned long long)ex->rank * 2ull + parity) * ex->block_words;
     CUDA_TRY(cudaMemsetAsync(ex->status.p, 0, 16, st));
     MLG_TRY(launch_push_peers(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ci_min, boxes, np, ex->cap, epoch,
-                              reinterpret_cast<unsigned int*>(ex->status.p + 2), st));
+                              reinterpret_cast<unsigned int*>(ex->status.p + 2), ex->status.p + 3, st));
     MLG_TRY(launch_merge_exchange(q->cnt8.p, ex->mailbox + parity * ex->block_words, 2ull * ex->block_words, ex->world, ex->rank, ex->cap,
                                   q->db->v.nd, (uint32_t)q->ci_min, q->present.p, q->touched.p, q->d_scalar.p, ex->status.p, epoch,
                                   ex->timeout_ns, st));

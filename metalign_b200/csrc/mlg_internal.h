@@ -155,15 +155,15 @@ int launch_pack_ascii(const unsigned char* text, unsigned long long nbases, unsi
 int launch_ascii_to_keys(const unsigned char* text, unsigned long long nslots, uint32_t K, key128* keys, cudaStream_t st);
 
 int launch_clamp_counts(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min, cudaStream_t st);
-int launch_pack_touched(const unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
+int launch_pack_touched(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
                         unsigned long long* out, cudaStream_t st);
 int launch_merge_sparse(unsigned char* cnt8, const unsigned long long* entries, unsigned long long n, uint32_t nd, uint32_t ci_min,
                         uint32_t* present, uint32_t* touched, unsigned long long* d_cursors, cudaStream_t st);
-int launch_pack_exchange(const unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
-                         unsigned long long* out, unsigned long long cap, cudaStream_t st);
-int launch_push_peers(const unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
+int launch_pack_exchange(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
+                         unsigned long long* out, unsigned long long cap, unsigned long long* own_count, cudaStream_t st);
+int launch_push_peers(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
                       unsigned long long* const* boxes, uint32_t n_peers, unsigned long long cap, unsigned long long epoch,
-                      unsigned int* done_ctas, cudaStream_t st);
+                      unsigned int* done_ctas, unsigned long long* own_count, cudaStream_t st);
 int launch_merge_exchange(unsigned char* cnt8, const unsigned long long* recv, unsigned long long stride_words, uint32_t world, uint32_t rank,
                           unsigned long long cap, uint32_t nd, uint32_t ci_min, uint32_t* present, uint32_t* touched,
                           unsigned long long* d_cursors, unsigned long long* d_status, unsigned long long epoch,

@@ -353,14 +353,21 @@ __global__ void k_clamp_counts(unsigned char* cnt8, const uint32_t* __restrict__
         if (cnt8[e] > ci_min) cnt8[e] = (unsigned char)ci_min;
     }
 }
+// a rank's own counter clamped to ci_min in place, as its contribution to the cross-rank sum: after a merge the table
+// holds sum over ranks of min(count, ci_min) on every rank, the same as the dense form (k_clamp_counts) leaves it
+__device__ __forceinline__ uint32_t clamp_own(unsigned char* cnt8, uint32_t e, uint32_t ci_min) {
+    const uint32_t c = cnt8[e];
+    if (c <= ci_min) return c;
+    cnt8[e] = (unsigned char)ci_min;
+    return ci_min;
+}
 // sparse form of a rank's contribution: one 64-bit entry per non-zero counter = index | min(count, ci_min) << 32
-__global__ void k_pack_touched(const unsigned char* __restrict__ cnt8, const uint32_t* __restrict__ touched,
+__global__ void k_pack_touched(unsigned char* cnt8, const uint32_t* __restrict__ touched,
                                const unsigned long long* __restrict__ d_n, uint32_t ci_min, unsigned long long* out) {
     const unsigned long long n = *d_n;
     for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
         const uint32_t e = touched[i];
-        const uint32_t c = cnt8[e];
-        out[i] = (unsigned long long)e | ((unsigned long long)(c > ci_min ? ci_min : c) << 32);
+        out[i] = (unsigned long long)e | ((unsigned long long)clamp_own(cnt8, e, ci_min) << 32);
     }
 }
 // add another rank's sparse entries into this rank's counters (saturating); a counter that crosses ci_min joins present[]
@@ -390,30 +397,32 @@ __global__ void k_merge_sparse(unsigned char* cnt8, const unsigned long long* __
 // ---- the multi-GPU exchange without a host round trip (mlg_exchange, capi.cu) --------------------------------------
 // A rank's contribution travels as one BLOCK of block_words 64-bit words: word 0 = number of non-zero counters n
 // (| epoch << 40 on the direct path), word 1 unused, then min(n, cap) entries index | min(count, ci_min) << 32.
+// Both pack kernels clamp ALL n own counters (not only the first cap) and leave n in *own_count, the count the merge
+// judges this rank's block by: the merge itself appends to touched[] and so cannot read n there.
 constexpr unsigned long long XCNT_MASK = (1ull << 40) - 1ull;
 // fill this rank's block in local memory (the caller all-gathers the blocks, e.g. with NCCL)
-__global__ void k_pack_exchange(const unsigned char* __restrict__ cnt8, const uint32_t* __restrict__ touched,
-                                const unsigned long long* __restrict__ d_n, uint32_t ci_min, unsigned long long* out,
-                                unsigned long long cap) {
-    const unsigned long long n = *d_n, m = n < cap ? n : cap;
-    if (blockIdx.x == 0 && threadIdx.x == 0) { out[0] = n; out[1] = 0; }
-    for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < m; i += (unsigned long long)gridDim.x * blockDim.x) {
+__global__ void k_pack_exchange(unsigned char* cnt8, const uint32_t* __restrict__ touched, const unsigned long long* __restrict__ d_n,
+                                uint32_t ci_min, unsigned long long* out, unsigned long long cap, unsigned long long* own_count) {
+    const unsigned long long n = *d_n;
+    if (blockIdx.x == 0 && threadIdx.x == 0) { out[0] = n; out[1] = 0; *own_count = n; }
+    for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
         const uint32_t e = touched[i];
-        const uint32_t c = cnt8[e];
-        out[2 + i] = (unsigned long long)e | ((unsigned long long)(c > ci_min ? ci_min : c) << 32);
+        const uint32_t c = clamp_own(cnt8, e, ci_min);
+        if (i < cap) out[2 + i] = (unsigned long long)e | ((unsigned long long)c << 32);
     }
 }
 // direct path: store the block straight into every peer's mailbox over NVLink (peer-mapped pointers), then -- once every
 // CTA's stores are fenced -- publish count | epoch << 40 in word 0 of each copy with a system-scope release
 struct PeerBoxes { unsigned long long* box[MLG_MAX_RANKS]; uint32_t n; };
-__global__ void k_push_peers(const unsigned char* __restrict__ cnt8, const uint32_t* __restrict__ touched,
-                             const unsigned long long* __restrict__ d_n, uint32_t ci_min, PeerBoxes pb, unsigned long long cap,
-                             unsigned long long epoch, unsigned int* done_ctas) {
-    const unsigned long long n = *d_n, m = n < cap ? n : cap;
-    for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < m; i += (unsigned long long)gridDim.x * blockDim.x) {
+__global__ void k_push_peers(unsigned char* cnt8, const uint32_t* __restrict__ touched, const unsigned long long* __restrict__ d_n,
+                             uint32_t ci_min, PeerBoxes pb, unsigned long long cap, unsigned long long epoch, unsigned int* done_ctas,
+                             unsigned long long* own_count) {
+    const unsigned long long n = *d_n;
+    for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
         const uint32_t e = touched[i];
-        const uint32_t c = cnt8[e];
-        const unsigned long long en = (unsigned long long)e | ((unsigned long long)(c > ci_min ? ci_min : c) << 32);
+        const uint32_t c = clamp_own(cnt8, e, ci_min);
+        if (i >= cap) continue;
+        const unsigned long long en = (unsigned long long)e | ((unsigned long long)c << 32);
         for (uint32_t p = 0; p < pb.n; ++p) pb.box[p][2 + i] = en;
     }
     __threadfence_system();
@@ -422,6 +431,7 @@ __global__ void k_push_peers(const unsigned char* __restrict__ cnt8, const uint3
         const unsigned int t = atomicAdd(done_ctas, 1u);
         if (t == gridDim.x - 1u) {                       // the last CTA: every other CTA's stores are fenced before its increment
             *done_ctas = 0u;
+            *own_count = n;
             __threadfence_system();
             const unsigned long long flag = (n & XCNT_MASK) | (epoch << 40);
             for (uint32_t p = 0; p < pb.n; ++p)
@@ -433,6 +443,8 @@ __global__ void k_push_peers(const unsigned char* __restrict__ cnt8, const uint3
 // recv + w * stride_words = block of rank w.  epoch != 0: the blocks were stored by the peers themselves -- wait for word 0
 // of each to carry this epoch (bounded by timeout_ns).  If any rank had more entries than a block holds, NOTHING is merged
 // and status[0] = the largest count (the caller repeats the exchange with larger blocks); status[1] = 1 on a timeout.
+// The verdict covers all world counts, this rank's own (status[3], left by the pack kernel) included, so that every rank
+// reaches the same one: a rank that alone overflowed must repeat the exchange together with its peers.
 __global__ void k_merge_exchange(unsigned char* cnt8, const unsigned long long* recv, unsigned long long stride_words, uint32_t world,
                                  uint32_t rank, unsigned long long cap, uint32_t nd, uint32_t ci_min, uint32_t* present, uint32_t* touched,
                                  unsigned long long* cursors, unsigned long long* status, unsigned long long epoch,
@@ -444,7 +456,10 @@ __global__ void k_merge_exchange(unsigned char* cnt8, const unsigned long long* 
     if (threadIdx.x < world) {
         const uint32_t w = threadIdx.x;
         unsigned long long v = 0;
-        if (w != rank) {
+        if (w == rank) {
+            v = __ldcg(status + 3);
+            if (v > cap) atomicMax(&s_bad, 1);
+        } else {
             const unsigned long long* fp = recv + (unsigned long long)w * stride_words;
             if (epoch) {
                 unsigned long long t0, t1;
@@ -477,7 +492,7 @@ __global__ void k_merge_exchange(unsigned char* cnt8, const unsigned long long* 
     for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < total; i += (unsigned long long)gridDim.x * blockDim.x) {
         const uint32_t w = (uint32_t)(i / cap);
         const unsigned long long k = i - (unsigned long long)w * cap;
-        if (k >= s_cnt[w]) continue;                      // s_cnt[rank] == 0: the own block is skipped
+        if (w == rank || k >= s_cnt[w]) continue;         // the own counters are in the table already
         const unsigned long long en = __ldcg(recv + (unsigned long long)w * stride_words + 2ull + k);
         const uint32_t e = (uint32_t)en, c = (uint32_t)(en >> 32);
         if (c == 0u || e >= nd) continue;
@@ -571,7 +586,7 @@ int launch_clamp_counts(unsigned char* cnt8, const uint32_t* touched, const unsi
     CUDA_TRY(cudaGetLastError());
     return MLG_OK;
 }
-int launch_pack_touched(const unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
+int launch_pack_touched(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
                         unsigned long long* out, cudaStream_t st) {
     k_pack_touched<<<148u * 4u, 256, 0, st>>>(cnt8, touched, d_n_touched, ci_min, out);
     CUDA_TRY(cudaGetLastError());
@@ -585,19 +600,19 @@ int launch_merge_sparse(unsigned char* cnt8, const unsigned long long* entries, 
     CUDA_TRY(cudaGetLastError());
     return MLG_OK;
 }
-int launch_pack_exchange(const unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
-                         unsigned long long* out, unsigned long long cap, cudaStream_t st) {
-    k_pack_exchange<<<148u * 2u, 256, 0, st>>>(cnt8, touched, d_n_touched, ci_min, out, cap);
+int launch_pack_exchange(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
+                         unsigned long long* out, unsigned long long cap, unsigned long long* own_count, cudaStream_t st) {
+    k_pack_exchange<<<148u * 2u, 256, 0, st>>>(cnt8, touched, d_n_touched, ci_min, out, cap, own_count);
     CUDA_TRY(cudaGetLastError());
     return MLG_OK;
 }
-int launch_push_peers(const unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
+int launch_push_peers(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
                       unsigned long long* const* boxes, uint32_t n_peers, unsigned long long cap, unsigned long long epoch,
-                      unsigned int* done_ctas, cudaStream_t st) {
+                      unsigned int* done_ctas, unsigned long long* own_count, cudaStream_t st) {
     PeerBoxes pb{};
     pb.n = n_peers;
     for (uint32_t p = 0; p < n_peers && p < MLG_MAX_RANKS; ++p) pb.box[p] = boxes[p];
-    k_push_peers<<<148u, 256, 0, st>>>(cnt8, touched, d_n_touched, ci_min, pb, cap, epoch, done_ctas);
+    k_push_peers<<<148u, 256, 0, st>>>(cnt8, touched, d_n_touched, ci_min, pb, cap, epoch, done_ctas, own_count);
     CUDA_TRY(cudaGetLastError());
     return MLG_OK;
 }
