@@ -211,7 +211,8 @@ int mlg_query_free(mlg_query* q);
  * and grows with the reads; max_table_bytes caps it (0 = no cap).  A table that would pass the cap, or whose allocation
  * fails, stops counting: the query itself is unaffected and the read k-mer calls return MLG_ERR_NOMEM.  After any counter
  * exchange (mlg_query_counts_*, mlg_query_exchange_*) they return MLG_ERR_STATE: the table is not merged across ranks.
- * Without the table they return MLG_ERR_STATE too. */
+ * (The key-range passes below count across ranks instead: mlg_query_read_kmer_archive.)  Without the table they return
+ * MLG_ERR_STATE too. */
 typedef struct mlg_read_kmer_stats {
     uint64_t windows;        /* N-free K-long windows counted */
     uint64_t distinct;       /* distinct canonical k-mers in the table */
@@ -261,9 +262,44 @@ typedef struct mlg_read_kmer_plan {
     double ms_histogram;     /* CUDA-event time of the histogram launches */
     double ms_count;         /* CUDA-event time of the ranged count launches */
     double ms_output;        /* CUDA-event time of selection, sort and encoding */
+    /* the count across ranks (mlg_query_read_kmer_archive); a query that never called it is rank 0 of 1 */
+    uint32_t rank;           /* this rank: its output holds share `rank` of the key order */
+    uint32_t world;          /* ranks */
+    uint32_t peers_added;    /* peer archives added */
+    uint32_t reserved;
+    uint64_t share_first_bin; /* the share: top-level bins [first, end) of the min(K, 10) leading bases of the canonical key */
+    uint64_t share_end_bin;
+    uint64_t share_windows;  /* windows of the share's bins (mlg_read_kmer_stats.windows stays the total over every archive) */
 } mlg_read_kmer_plan;
 /* the plan of the last output call in passes mode (MLG_ERR_STATE in any other mode) */
 int mlg_query_read_kmer_plan(mlg_query* q, mlg_read_kmer_plan* out);
+/* The read k-mers of reads sharded over W ranks, in passes mode only: every rank receives every other rank's archive, and
+ * rank r counts share r of the canonical key order over all the reads, so its counts are global and exact.  Share r is
+ * a contiguous run of the top-level histogram bins (DESIGN.md section 10); the shares of ranks 0..W-1, in rank order,
+ * are the whole key order, and so are the KMC databases the ranks write (mlg_kmc_concat joins them into the file one
+ * query over all the reads writes).
+ *   mlg_query_read_kmer_archive   after the last push: this rank's archive packed into one device blob the query owns
+ *                                 (copies on the compute stream, no host join; valid until the first output call or
+ *                                 mlg_query_free, so a peer's copy of it must be ordered on this context's compute stream
+ *                                 before that call).  From then on the query is rank `rank` of `world` (1..16) and
+ *                                 refuses pushes.  An archive that outgrew its budget sends a header flagged overflowed.
+ *                                 MLG_ERR_STATE without passes or on a second call; MLG_ERR_ARG for rank >= world or world > 16.
+ *   mlg_query_read_kmer_add_archive  a peer's blob (device memory of this GPU, 8-byte aligned), copied into the archive: it counts
+ *                                 against the budget.  The blob is checked first -- header (magic, library version, K,
+ *                                 world, sizes that add up to `bytes`), its rank (not this one, not one already added,
+ *                                 < world) and, by a kernel, every batch's read offsets -- and a blob that fails returns
+ *                                 MLG_ERR_ARG and changes nothing.  A flagged blob, or one past the budget, makes the
+ *                                 output calls return MLG_ERR_NOMEM on this rank too, so every rank reaches the same verdict.
+ * mlg_query_read_kmers / mlg_query_write_reads_kmc return MLG_ERR_STATE until every one of the world - 1 peers has been
+ * added, and then return / write the share's keys only; a counter exchange no longer makes them refuse. */
+int mlg_query_read_kmer_archive(mlg_query* q, uint32_t rank, uint32_t world, const void** d_blob, uint64_t* bytes);
+int mlg_query_read_kmer_add_archive(mlg_query* q, const void* d_blob, uint64_t bytes);
+/* Host only (no context): the version-0 KMC databases part_prefixes[0..n_parts) -- the same k, mode, counter size,
+ * lut_prefix_length, min / max count, each one's keys above the last one's -- joined into <prefix>.kmc_pre / .kmc_suf:
+ * the suffix bodies one after the other, the prefix tables and totals summed.  The parts are read in pieces and left as
+ * they are; a call that fails leaves no output file behind (MLG_ERR_ARG for parts that do not fit together, MLG_ERR_IO
+ * for files that cannot be read or written). */
+int mlg_kmc_concat(const char* prefix, const char* const* part_prefixes, uint32_t n_parts);
 /* after finish: `kmc_tools simple <reads> <db> intersect <prefix>`: the k-mers of I, count = the count column of
  * mlg_query_dump_intersection.  Needs no read k-mer table. */
 int mlg_query_write_intersection_kmc(mlg_query* q, const char* prefix, uint32_t counter_max);

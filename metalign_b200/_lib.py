@@ -49,7 +49,8 @@ class ReadKmerStats(C.Structure):
 class ReadKmerPlan(C.Structure):
     _fields_ = [("passes", C.c_uint32), ("refined_bins", C.c_uint32), ("archive_bytes", C.c_uint64), ("pass_cap_bytes", C.c_uint64),
                 ("max_pass_bound", C.c_uint64), ("distinct", C.c_uint64), ("ms_histogram", C.c_double), ("ms_count", C.c_double),
-                ("ms_output", C.c_double)]
+                ("ms_output", C.c_double), ("rank", C.c_uint32), ("world", C.c_uint32), ("peers_added", C.c_uint32),
+                ("reserved", C.c_uint32), ("share_first_bin", C.c_uint64), ("share_end_bin", C.c_uint64), ("share_windows", C.c_uint64)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
@@ -121,6 +122,9 @@ SIGNATURES = {
     "mlg_query_read_kmer_stats": (C.c_int, [_vp, C.POINTER(ReadKmerStats)]),
     "mlg_query_enable_read_kmer_passes": (C.c_int, [_vp, C.c_uint64]),
     "mlg_query_read_kmer_plan": (C.c_int, [_vp, C.POINTER(ReadKmerPlan)]),
+    "mlg_query_read_kmer_archive": (C.c_int, [_vp, C.c_uint32, C.c_uint32, _pp, C.POINTER(C.c_uint64)]),
+    "mlg_query_read_kmer_add_archive": (C.c_int, [_vp, _vp, C.c_uint64]),
+    "mlg_kmc_concat": (C.c_int, [C.c_char_p, C.POINTER(C.c_char_p), C.c_uint32]),
     "mlg_query_free": (C.c_int, [_vp]),
     "mlg_sketch_genomes": (C.c_int, [_vp, _vp, _u64p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint64, _u64p, _u32p, _vp, _vp]),
 }

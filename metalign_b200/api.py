@@ -399,6 +399,17 @@ class Query:
         check(_lib.lib().mlg_query_read_kmer_plan(self._h, C.byref(s)))
         return s.as_dict()
 
+    def read_kmer_archive(self, rank: int, world: int):
+        """mlg_query_read_kmer_archive: (device pointer, bytes) of this rank's read archive as one blob; from now on the
+        query is rank `rank` of a `world`-rank read k-mer count (see metalign_b200.dist.share_read_kmers)"""
+        p, n = C.c_void_p(), C.c_uint64()
+        check(_lib.lib().mlg_query_read_kmer_archive(self._h, int(rank), int(world), C.byref(p), C.byref(n)))
+        return p.value or 0, n.value
+
+    def add_read_kmer_archive(self, d_blob_ptr: int, nbytes: int) -> None:
+        """mlg_query_read_kmer_add_archive: a peer's blob (device memory), checked and copied into this query's archive"""
+        check(_lib.lib().mlg_query_read_kmer_add_archive(self._h, d_blob_ptr, int(nbytes)))
+
     def stats(self) -> dict:
         s = Stats()
         check(_lib.lib().mlg_query_stats(self._h, C.byref(s)))
@@ -415,6 +426,13 @@ class Query:
 
     def __exit__(self, *exc):
         self.close()
+
+
+def kmc_concat(prefix: str, parts: Sequence[str]) -> None:
+    """mlg_kmc_concat: the KMC databases `parts` (version 0, ascending keys from one part to the next) joined into
+    <prefix>.kmc_pre / .kmc_suf; the parts are left as they are, and a failure leaves no output behind"""
+    arr = (C.c_char_p * max(len(parts), 1))(*[p.encode() for p in parts])
+    check(_lib.lib().mlg_kmc_concat(prefix.encode(), arr, len(parts)))
 
 
 class Exchange:

@@ -156,6 +156,7 @@ struct mlg_query {
     ReadKmerPasses* rkp = nullptr;                 // the key-range mode instead (mlg_query_enable_read_kmer_passes; null = off)
     KmcOutStats rk_out;
     bool exchanged = false;                        // counters went through an exchange: the per-rank table no longer matches
+    bool rk_shared = false;                        // rank of a read k-mer count across ranks (mlg_query_read_kmer_archive)
 };
 
 namespace {
@@ -237,6 +238,7 @@ int check_push(mlg_query* q) {
     if (!q) { mlg_set_error("null query"); return MLG_ERR_ARG; }
     if (q->finished) { mlg_set_error("query already finished"); return MLG_ERR_STATE; }
     if (q->reduced || q->merged) { mlg_set_error("counters were already combined across ranks; no more reads can be pushed"); return MLG_ERR_STATE; }
+    if (q->rk_shared) { mlg_set_error("the read archive was handed to the other ranks; no more reads can be pushed"); return MLG_ERR_STATE; }
     return ensure_device(q->ctx);
 }
 
@@ -1003,7 +1005,10 @@ MLG_API int mlg_query_enable_read_kmer_passes(mlg_query* q, uint64_t max_bytes) 
 static int check_read_kmers(mlg_query* q, uint32_t min_count, uint32_t counter_max) {
     if (!q) { mlg_set_error("null query"); return MLG_ERR_ARG; }
     if (!q->rk && !q->rkp) { mlg_set_error("the read k-mer table is off (mlg_query_enable_read_kmers)"); return MLG_ERR_STATE; }
-    if (q->exchanged) { mlg_set_error("the read k-mer table is per rank and the counters went through an exchange"); return MLG_ERR_STATE; }
+    if (q->exchanged && !q->rk_shared) { mlg_set_error("the read k-mer table is per rank and the counters went through an exchange"); return MLG_ERR_STATE; }
+    if (q->rk_shared && rkp_peers_missing(q->rkp)) {
+        mlg_set_error("%u peer read archives are still to be added (mlg_query_read_kmer_add_archive)", rkp_peers_missing(q->rkp)); return MLG_ERR_STATE;
+    }
     if (min_count < 1 || min_count > 255 || counter_max < 1 || counter_max > 255) { mlg_set_error("min_count and counter_max must be 1..255"); return MLG_ERR_ARG; }
     MLG_TRY(ensure_device(q->ctx));
     return q->rk ? rk_check(q->rk) : rkp_check(q->rkp);
@@ -1067,6 +1072,29 @@ MLG_API int mlg_query_read_kmer_plan(mlg_query* q, mlg_read_kmer_plan* out) {
     if (!q || !out) { mlg_set_error("null argument"); return MLG_ERR_ARG; }
     if (!q->rkp) { mlg_set_error("read k-mer passes are off (mlg_query_enable_read_kmer_passes)"); return MLG_ERR_STATE; }
     return rkp_plan(q->rkp, out);
+}
+
+MLG_API int mlg_query_read_kmer_archive(mlg_query* q, uint32_t rank, uint32_t world, const void** d_blob, uint64_t* bytes) {
+    if (!q || !d_blob || !bytes) { mlg_set_error("null argument"); return MLG_ERR_ARG; }
+    if (!q->rkp) { mlg_set_error("read k-mer passes are off (mlg_query_enable_read_kmer_passes)"); return MLG_ERR_STATE; }
+    if (q->rk_shared) { mlg_set_error("this query's read archive was already packed"); return MLG_ERR_STATE; }
+    if (world < 1 || world > MLG_MAX_RANKS || rank >= world) { mlg_set_error("rank %u of %u ranks: need rank < world <= %d", rank, world, MLG_MAX_RANKS); return MLG_ERR_ARG; }
+    MLG_TRY(ensure_device(q->ctx));
+    MLG_TRY(rkp_pack_archive(q->rkp, rank, world, d_blob, bytes));
+    q->rk_shared = true;
+    return MLG_OK;
+}
+MLG_API int mlg_query_read_kmer_add_archive(mlg_query* q, const void* d_blob, uint64_t bytes) {
+    if (!q) { mlg_set_error("null query"); return MLG_ERR_ARG; }
+    if (!q->rk_shared) { mlg_set_error("call mlg_query_read_kmer_archive first"); return MLG_ERR_STATE; }
+    if (!d_blob) { mlg_set_error("null blob"); return MLG_ERR_ARG; }
+    MLG_TRY(ensure_device(q->ctx));
+    return rkp_add_archive(q->rkp, d_blob, bytes, &q->st.gpu_launches);
+}
+MLG_API int mlg_kmc_concat(const char* prefix, const char* const* part_prefixes, uint32_t n_parts) {
+    if (!prefix || !part_prefixes || !n_parts) { mlg_set_error("null argument or no part"); return MLG_ERR_ARG; }
+    for (uint32_t i = 0; i < n_parts; ++i) if (!part_prefixes[i]) { mlg_set_error("null part prefix"); return MLG_ERR_ARG; }
+    return kmc_concat(prefix, part_prefixes, n_parts);
 }
 
 MLG_API int mlg_query_stats(mlg_query* q, mlg_stats* out) {

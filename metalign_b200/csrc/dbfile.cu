@@ -23,7 +23,7 @@
 
 namespace {
 
-constexpr uint32_t BUILD_TAG = 0x20261017u;      // minimizer identity = min/max multiply-add + xor-shift; hit records v2
+constexpr uint32_t BUILD_TAG = MLG_BUILD_TAG;
 enum : uint32_t { S_DKEY = 1, S_BSTART, S_F, S_ALIAS_Z, S_ALIAS_I, S_ALIAS_BLOOM, S_HOFF, S_HBASE, S_HITS, S_DEN, S_HASEMPTY, S_T1, S_DMULT };
 struct Section { uint32_t tag, elem; uint64_t count, offset; };
 constexpr size_t CHUNK = (size_t)8 << 20;        // staging granularity.  Page-locking costs ~0.7 ms per MiB on the GPU boxes: 12 x 32 MiB

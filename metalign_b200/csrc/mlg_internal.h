@@ -11,6 +11,9 @@
 #define MLG_MAX_KS 8
 #define MLG_MAX_RANKS 16        // ranks of one exchange (one NVSwitch domain)
 #define MLG_TILE_WORDS 256u     // 64-base words per K1 tile == threads per CTA
+// version of the device structures in built .mlgdb files and of the read archives ranks exchange: minimizer identity =
+// min/max multiply-add + xor-shift; hit records v2
+#define MLG_BUILD_TAG 0x20261017u
 
 void mlg_set_error(const char* fmt, ...);
 
@@ -230,3 +233,9 @@ int rkp_read_kmers(ReadKmerPasses* t, uint32_t min_count, uint32_t counter_max, 
 int rkp_write_kmc(ReadKmerPasses* t, const char* prefix, uint32_t min_count, uint32_t counter_max, KmcOutStats* ws);
 int rkp_stats(ReadKmerPasses* t, mlg_read_kmer_stats* out);
 int rkp_plan(ReadKmerPasses* t, mlg_read_kmer_plan* out);
+// the read k-mer count across ranks (mlg_query_read_kmer_archive / _add_archive): this rank's archive as one device blob,
+// a peer's blob appended to the archive, and the peers still missing before the output calls may run
+int rkp_pack_archive(ReadKmerPasses* t, uint32_t rank, uint32_t world, const void** d_blob, uint64_t* bytes);
+int rkp_add_archive(ReadKmerPasses* t, const void* d_blob, uint64_t bytes, uint32_t* launches);
+uint32_t rkp_peers_missing(const ReadKmerPasses* t);
+int kmc_concat(const char* prefix, const char* const* parts, uint32_t n_parts);

@@ -5,8 +5,12 @@
 // end of this file) counts a device copy of the reads at output time instead, one interval of the key order per pass.
 // DESIGN.md section 10.
 #include <cub/cub.cuh>
+#include <errno.h>
+#include <fcntl.h>
 #include <stdio.h>
 #include <string.h>
+#include <sys/stat.h>
+#include <unistd.h>
 #include <algorithm>
 #include <chrono>
 #include <deque>
@@ -563,37 +567,51 @@ static int kmc_append(KmcWriter& w, const key128* keys, const uint32_t* cnt, uin
     return rc;
 }
 
+// .kmc_pre: "KMCP" | LUT (+ guard) | header | header bytes | "KMCP"   (csrc/kmcdb.h), version 0.  The one writer of this
+// file: kmc_end and kmc_concat both go through it.
+struct KmcHeader {
+    uint32_t K = 0, mode = 0, counter_size = 1, p = 0, min_count = 0;
+    unsigned long long max_count = 0, total = 0;
+    unsigned char strands = 0;               // 0: both strands (canonical k-mers)
+};
+static int kmc_write_pre(const std::string& path, const std::vector<unsigned long long>& lut, const KmcHeader& h, unsigned long long* bytes) {
+    std::vector<unsigned char> pre;
+    auto put = [&](const void* v, size_t b) { const unsigned char* c = (const unsigned char*)v; pre.insert(pre.end(), c, c + b); };
+    auto u32 = [&](uint32_t v) { put(&v, 4); };
+    put("KMCP", 4);
+    put(lut.data(), lut.size() * 8);
+    const size_t h0 = pre.size();
+    u32(h.K); u32(h.mode); u32(h.counter_size); u32(h.p);           // k, mode (counters), counter_size, lut_prefix_length
+    u32(h.min_count); u32((uint32_t)h.max_count);
+    put(&h.total, 8);
+    const unsigned char hdr_tail[4] = {h.strands, 0, 0, 0}; put(hdr_tail, 4);   // strands + 3 pad bytes
+    u32((uint32_t)(h.max_count >> 32));                              // max_count, high word
+    const unsigned char reserved[20] = {}; put(reserved, 20);
+    u32(0);                                                          // kmc_version 0
+    u32((uint32_t)(pre.size() - h0));
+    put("KMCP", 4);
+    FILE* fp = fopen(path.c_str(), "wb");
+    if (!fp) { mlg_set_error("cannot create %s", path.c_str()); return MLG_ERR_IO; }
+    bool ok = fwrite(pre.data(), 1, pre.size(), fp) == pre.size();
+    ok = (fclose(fp) == 0) && ok;
+    if (!ok) { mlg_set_error("%s: short write", path.c_str()); return MLG_ERR_IO; }
+    *bytes = pre.size();
+    return MLG_OK;
+}
+
 static int kmc_end(KmcWriter& w) {
     const auto t0 = std::chrono::steady_clock::now();
     bool ok = w.ok && fwrite("KMCS", 1, 4, w.fs) == 4;
     ok = (fclose(w.fs) == 0) && ok;
     w.fs = nullptr;
     if (!ok) { mlg_set_error("%s: short write", w.suf_path.c_str()); return MLG_ERR_IO; }
-
-    // .kmc_pre: "KMCP" | LUT (+ guard) | header | header bytes | "KMCP"   (csrc/kmcdb.h)
-    std::vector<unsigned char> pre;
-    auto put = [&](const void* v, size_t b) { const unsigned char* c = (const unsigned char*)v; pre.insert(pre.end(), c, c + b); };
-    auto u32 = [&](uint32_t v) { put(&v, 4); };
-    put("KMCP", 4);
-    put(w.lut.data(), w.lut.size() * 8);
-    const size_t h0 = pre.size();
-    u32(w.K); u32(0); u32(1); u32(w.p);                             // k, mode (counters), counter_size, lut_prefix_length
-    u32(w.min_count); u32(w.counter_max);
-    const unsigned long long total = w.records; put(&total, 8);
-    const unsigned char hdr_tail[4] = {0, 0, 0, 0}; put(hdr_tail, 4);  // both strands (canonical) + 3 pad bytes
-    u32(0);                                                          // max_count, high word
-    const unsigned char reserved[20] = {}; put(reserved, 20);
-    u32(0);                                                          // kmc_version 0
-    u32((uint32_t)(pre.size() - h0));
-    put("KMCP", 4);
-    FILE* fp = fopen(w.pre_path.c_str(), "wb");
-    if (!fp) { mlg_set_error("cannot create %s", w.pre_path.c_str()); return MLG_ERR_IO; }
-    ok = fwrite(pre.data(), 1, pre.size(), fp) == pre.size();
-    ok = (fclose(fp) == 0) && ok;
-    if (!ok) { mlg_set_error("%s: short write", w.pre_path.c_str()); return MLG_ERR_IO; }
+    KmcHeader h;
+    h.K = w.K; h.p = w.p; h.min_count = w.min_count; h.max_count = w.counter_max; h.total = w.records;
+    unsigned long long pre_bytes = 0;
+    MLG_TRY(kmc_write_pre(w.pre_path, w.lut, h, &pre_bytes));
     w.finished = true;
     if (w.ws) {
-        w.ws->records = w.records; w.ws->bytes = pre.size() + w.sbytes + 8;
+        w.ws->records = w.records; w.ws->bytes = pre_bytes + w.sbytes + 8;
         w.ws->s_write += seconds_since(t0);
     }
     return MLG_OK;
@@ -644,6 +662,13 @@ struct ReadKmerPasses {
     std::deque<ArchivedBatch> batches;
     unsigned long long archive_bytes = 0, bytes_needed = 0;
     bool overflowed = false;
+    int overflowed_rank = -1;                // a peer's blob came flagged: that rank's archive overflowed
+    // rank `rank` of a `world`-rank count (mlg_query_read_kmer_archive): the output calls count share `rank` of the key
+    // order over this rank's batches and every peer's
+    uint32_t rank = 0, world = 1, peers = 0;
+    std::vector<char> added;                 // per rank: its batches are in the archive
+    DevBuf<unsigned char> blob;              // this rank's blob, until the first output call
+    std::vector<unsigned long long> blob_head;
     mlg_read_kmer_plan plan{};               // of the last output call
     mlg_read_kmer_stats st{};                // windows, distinct, slots, bytes, ms_count of the last output call
 };
@@ -659,17 +684,20 @@ void rkp_destroy(ReadKmerPasses* t) { delete t; }
 
 // Enqueued on the compute stream after the batch's last probe range, before the staging set's `done` event: copies of
 // what the probe read (whole 16-byte units of bases, the N mask as it saw it, the offsets).  No kernel.
+// the archive stops: batches freed, the output calls return MLG_ERR_NOMEM; bytes_needed = what it would have needed
+static int rkp_overflow(ReadKmerPasses* t, unsigned long long add) {
+    cudaGetLastError();                                   // a failed allocation is recorded here, not an error of the query
+    CUDA_TRY(cudaStreamSynchronize(t->ctx->s_comp));      // copies into the archive may still be in flight
+    t->batches.clear();
+    t->overflowed = true; t->bytes_needed = t->archive_bytes + add; t->archive_bytes = 0;
+    return MLG_OK;
+}
+
 int rkp_archive(ReadKmerPasses* t, const ProbeArgs& a, unsigned long long n_reads, unsigned long long nbases) {
     const unsigned long long add = a.base_words * 8 + (a.nmask ? a.nmask_words * 8 : 0) + (a.off ? (n_reads + 1) * 8 : 0);
     if (t->overflowed) { t->bytes_needed += add; return MLG_OK; }     // what the whole archive would have needed
     cudaStream_t st = t->ctx->s_comp;
-    auto overflow = [&]() -> int {
-        cudaGetLastError();                               // a failed allocation is recorded here, not an error of the query
-        CUDA_TRY(cudaStreamSynchronize(st));              // copies into the archive may still be in flight
-        t->batches.clear();
-        t->overflowed = true; t->bytes_needed = t->archive_bytes + add; t->archive_bytes = 0;
-        return MLG_OK;
-    };
+    auto overflow = [&]() -> int { return rkp_overflow(t, add); };
     if (t->budget && t->archive_bytes + add > t->budget) return overflow();
     t->batches.emplace_back();
     ArchivedBatch& b = t->batches.back();
@@ -684,6 +712,10 @@ int rkp_archive(ReadKmerPasses* t, const ProbeArgs& a, unsigned long long n_read
 }
 
 int rkp_check(ReadKmerPasses* t) {
+    if (t->overflowed && t->overflowed_rank >= 0) {
+        mlg_set_error("rank %d's device copy of the reads outgrew its read k-mer budget", t->overflowed_rank);
+        return MLG_ERR_NOMEM;
+    }
     if (t->overflowed) {
         mlg_set_error("the device copy of the reads outgrew the read k-mer budget: %llu bytes needed, %llu allowed", t->bytes_needed, t->budget);
         return MLG_ERR_NOMEM;
@@ -705,6 +737,22 @@ namespace {
 // The plan: bins of the leading bases of the canonical key (RK_BIN_BASES per level), each bounded by min(windows, keys
 // it can hold), grouped in key order into passes that fit the cap; a bin that alone does not fit is split by a histogram
 // over its next bases.  A bin that covers the whole k-mer holds one key, so the recursion ends.
+// Share r of a W-rank count: the top-level bins [s_r, s_{r+1}) with s_r = the first bin i such that W * (windows of the
+// bins before i) >= r * T, T = every window, and s_W = the number of bins.  Every rank holds the same reads, so every
+// rank finds the same boundaries.  A share holds fewer than T / W + (the largest bin) windows.
+void share_bins(const std::vector<unsigned long long>& h, uint32_t world, uint32_t rank, unsigned long long* b0, unsigned long long* b1) {
+    unsigned long long T = 0;
+    for (unsigned long long x : h) T += x;
+    auto bound = [&](uint32_t r) -> unsigned long long {
+        if (r >= world) return h.size();
+        unsigned long long before = 0;
+        for (unsigned long long i = 0; i < h.size(); before += h[i], ++i)
+            if ((u128)world * before >= (u128)r * T) return i;
+        return h.size();
+    };
+    *b0 = bound(rank); *b1 = bound(rank + 1);
+}
+
 struct Planner {
     ReadKmerPasses* t;
     unsigned long long cap;
@@ -747,8 +795,15 @@ struct Planner {
         MLG_TRY(histogram(depth, prefix, b));
         const std::vector<unsigned long long> h = bins;       // the recursion reuses `bins`
         const unsigned long long keys_per_bin = 2 * rest >= 64 ? ~0ull : 1ull << (2 * rest);
+        unsigned long long i0 = 0, i1 = h.size();               // this rank's share of the top-level bins
+        if (depth == 0) {
+            share_bins(h, t->world, t->rank, &i0, &i1);
+            t->plan.share_first_bin = i0; t->plan.share_end_bin = i1;
+        }
         for (unsigned long long i = 0; i < h.size(); ++i) {
             if (windows) *windows += h[i];
+            if (i < i0 || i >= i1) continue;
+            if (depth == 0) t->plan.share_windows += h[i];
             const u128 sub = (prefix << (2 * b)) | i;
             const unsigned long long bound = std::min(h[i], keys_per_bin);
             if (fits(bound)) { add(sub << (2 * rest), (sub + 1) << (2 * rest), bound); continue; }
@@ -767,7 +822,9 @@ static int rkp_plan_passes(ReadKmerPasses* t, std::vector<KeyRange>& passes) {
     mlg_read_kmer_plan& pl = t->plan;
     pl = mlg_read_kmer_plan{};
     t->st = mlg_read_kmer_stats{};
+    t->blob.release();                                     // the peers have their copies: rkp_check joined the stream
     pl.archive_bytes = t->archive_bytes;
+    pl.rank = t->rank; pl.world = t->world; pl.peers_added = t->peers;
     Planner P{t, 0};
     MLG_TRY(P.d_bins.alloc(1ull << (2 * RK_BIN_BASES)));
     if (t->budget) {
@@ -888,3 +945,323 @@ int rkp_stats(ReadKmerPasses* t, mlg_read_kmer_stats* o) {
     return MLG_OK;
 }
 int rkp_plan(ReadKmerPasses* t, mlg_read_kmer_plan* o) { *o = t->plan; return MLG_OK; }
+
+// ---------------------------------------------------------------- the read k-mer count across ranks
+// Each rank packs its archive into one device blob; every rank appends every peer's blob to its archive and then counts
+// its own share of the key order over all the reads.  Blob layout (8-byte words, all little endian):
+//   header   magic, BUILD_TAG | K << 32, rank | world << 32, overflowed, batches, bytes     (RKA_HEAD_WORDS)
+//   per batch n_reads, nbases, read_len, base_words, nmask_words, flags (1: N mask, 2: offsets)   (RKA_DESC_WORDS)
+//   data     per batch: bases (base_words words), N mask (nmask_words words), offsets (n_reads + 1 words)
+// DESIGN.md section 10.
+namespace {
+
+constexpr unsigned long long RKA_MAGIC = 0x3130414B52474C4Dull;      // "MLGRKA01"
+constexpr unsigned long long RKA_HEAD_WORDS = 6, RKA_DESC_WORDS = 6;
+constexpr unsigned long long RKA_MASK = 1, RKA_OFF = 2;
+constexpr unsigned long long RKA_FIRST_READ = 64 << 10;               // bytes of the first header copy
+
+inline unsigned long long rka_data_words(unsigned long long n_reads, unsigned long long base_words, unsigned long long nmask_words,
+                                         unsigned long long flags) {
+    return base_words + ((flags & RKA_MASK) ? nmask_words : 0) + ((flags & RKA_OFF) ? n_reads + 1 : 0);
+}
+
+// a peer's offsets before they are trusted: off[0] = 0, non-decreasing, off[n_reads] = nbases (bad[0] = 1 otherwise)
+__global__ void k_check_offsets(const unsigned long long* off, unsigned long long n_reads, unsigned long long nbases, unsigned long long* bad) {
+    for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i <= n_reads; i += (unsigned long long)gridDim.x * blockDim.x) {
+        const unsigned long long v = off[i];
+        if ((i == 0 && v != 0) || (i == n_reads && v != nbases) || (i < n_reads && off[i + 1] < v)) atomicOr(bad, 1ull);
+    }
+}
+
+}  // namespace
+
+int rkp_pack_archive(ReadKmerPasses* t, uint32_t rank, uint32_t world, const void** d_blob, uint64_t* bytes) {
+    cudaStream_t st = t->ctx->s_comp;
+    const unsigned long long nb = t->overflowed ? 0 : t->batches.size();     // an overflowed archive sends its flag only
+    std::vector<unsigned long long>& h = t->blob_head;                       // kept: the copy below is asynchronous
+    h.assign(RKA_HEAD_WORDS + nb * RKA_DESC_WORDS, 0);
+    unsigned long long words = h.size();
+    for (unsigned long long i = 0; i < nb; ++i) {
+        const ArchivedBatch& b = t->batches[i];
+        unsigned long long* d = h.data() + RKA_HEAD_WORDS + i * RKA_DESC_WORDS;
+        d[0] = b.n_reads; d[1] = b.nbases; d[2] = b.read_len; d[3] = b.base_words; d[4] = b.nmask_words;
+        d[5] = (b.nmask.p ? RKA_MASK : 0) | (b.off.p ? RKA_OFF : 0);
+        words += rka_data_words(d[0], d[3], d[4], d[5]);
+    }
+    h[0] = RKA_MAGIC; h[1] = MLG_BUILD_TAG | (unsigned long long)t->K << 32; h[2] = rank | (unsigned long long)world << 32;
+    h[3] = t->overflowed ? 1 : 0; h[4] = nb; h[5] = words * 8;
+    DevBuf<unsigned char> blob;
+    if (blob.alloc(words * 8) != MLG_OK) {
+        cudaGetLastError();
+        mlg_set_error("no device memory for the %llu-byte blob of the read archive", words * 8);
+        return MLG_ERR_NOMEM;
+    }
+    unsigned char* p = blob.p;
+    CUDA_TRY(cudaMemcpyAsync(p, h.data(), h.size() * 8, cudaMemcpyHostToDevice, st));
+    p += h.size() * 8;
+    for (unsigned long long i = 0; i < nb; ++i) {
+        const ArchivedBatch& b = t->batches[i];
+        CUDA_TRY(cudaMemcpyAsync(p, b.bases.p, b.base_words * 8, cudaMemcpyDeviceToDevice, st)); p += b.base_words * 8;
+        if (b.nmask.p) { CUDA_TRY(cudaMemcpyAsync(p, b.nmask.p, b.nmask_words * 8, cudaMemcpyDeviceToDevice, st)); p += b.nmask_words * 8; }
+        if (b.off.p) { CUDA_TRY(cudaMemcpyAsync(p, b.off.p, (b.n_reads + 1) * 8, cudaMemcpyDeviceToDevice, st)); p += (b.n_reads + 1) * 8; }
+    }
+    std::swap(t->blob.p, blob.p); std::swap(t->blob.n, blob.n);
+    t->rank = rank; t->world = world; t->peers = 0;
+    t->added.assign(world, 0); t->added[rank] = 1;
+    *d_blob = t->blob.p; *bytes = words * 8;
+    return MLG_OK;
+}
+
+// A peer's blob comes from outside the query: everything the count kernels rely on is checked before anything changes.
+int rkp_add_archive(ReadKmerPasses* t, const void* d_blob, uint64_t bytes, uint32_t* launches) {
+    cudaStream_t st = t->ctx->s_comp;
+    const unsigned char* blob = (const unsigned char*)d_blob;
+    if ((uintptr_t)d_blob % 8) { mlg_set_error("a read archive blob must start on an 8-byte boundary"); return MLG_ERR_ARG; }
+    if (bytes < RKA_HEAD_WORDS * 8 || bytes % 8) { mlg_set_error("a read archive blob has %llu bytes: not a blob", (unsigned long long)bytes); return MLG_ERR_ARG; }
+    std::vector<unsigned long long> h(std::min<unsigned long long>(bytes, RKA_FIRST_READ) / 8);
+    CUDA_TRY(cudaMemcpyAsync(h.data(), blob, h.size() * 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    const uint32_t tag = (uint32_t)h[1], K = (uint32_t)(h[1] >> 32), rank = (uint32_t)h[2], world = (uint32_t)(h[2] >> 32);
+    const unsigned long long nb = h[4];
+    if (h[0] != RKA_MAGIC || tag != MLG_BUILD_TAG) { mlg_set_error("not a read archive blob of this library version"); return MLG_ERR_ARG; }
+    if (K != t->K || world != t->world) { mlg_set_error("read archive blob of K = %u, %u ranks; this query has K = %u, %u ranks", K, world, t->K, t->world); return MLG_ERR_ARG; }
+    if (rank >= world || rank == t->rank || t->added[rank]) { mlg_set_error("read archive blob of rank %u: out of range, this rank's own, or already added", rank); return MLG_ERR_ARG; }
+    if (h[5] != bytes || h[3] > 1 || (h[3] && nb) || nb > (bytes / 8 - RKA_HEAD_WORDS) / RKA_DESC_WORDS) {
+        mlg_set_error("read archive blob of rank %u: its header does not match its %llu bytes", rank, (unsigned long long)bytes); return MLG_ERR_ARG;
+    }
+    const unsigned long long head = RKA_HEAD_WORDS + nb * RKA_DESC_WORDS;
+    if (head > h.size()) {
+        h.resize(head);
+        CUDA_TRY(cudaMemcpyAsync(h.data(), blob, head * 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+    }
+    u128 words = head;
+    for (unsigned long long i = 0; i < nb; ++i) {
+        const unsigned long long* d = h.data() + RKA_HEAD_WORDS + i * RKA_DESC_WORDS;
+        const unsigned long long n_reads = d[0], nbases = d[1], read_len = d[2], bw = d[3], mw = d[4], fl = d[5];
+        bool ok = fl <= (RKA_MASK | RKA_OFF) && read_len < (1ull << 32) && bw <= bytes / 8 && mw <= bytes / 8 && n_reads < bytes / 8 &&
+                  (u128)bw * 32 >= nbases && (!(fl & RKA_MASK) || (u128)mw * 64 >= nbases);
+        if (ok && !(fl & RKA_OFF)) ok = (u128)n_reads * read_len == nbases && (read_len || !n_reads);
+        if (!ok) { mlg_set_error("read archive blob of rank %u: batch %llu has an inconsistent descriptor", rank, i); return MLG_ERR_ARG; }
+        words += rka_data_words(n_reads, bw, mw, fl);
+    }
+    if (words * 8 != bytes) { mlg_set_error("read archive blob of rank %u: its batches do not add up to its %llu bytes", rank, (unsigned long long)bytes); return MLG_ERR_ARG; }
+    // the offsets, on the device: a bad one would send the count kernels' read search out of the batch
+    std::vector<const unsigned long long*> data(nb);
+    {
+        const unsigned char* p = blob + head * 8;
+        for (unsigned long long i = 0; i < nb; ++i) {
+            const unsigned long long* d = h.data() + RKA_HEAD_WORDS + i * RKA_DESC_WORDS;
+            data[i] = (const unsigned long long*)p;
+            p += rka_data_words(d[0], d[3], d[4], d[5]) * 8;
+        }
+    }
+    DevBuf<unsigned long long> bad; MLG_TRY(bad.alloc(1));
+    CUDA_TRY(cudaMemsetAsync(bad.p, 0, 8, st));
+    for (unsigned long long i = 0; i < nb; ++i) {
+        const unsigned long long* d = h.data() + RKA_HEAD_WORDS + i * RKA_DESC_WORDS;
+        if (!(d[5] & RKA_OFF)) continue;
+        const unsigned long long* off = data[i] + d[3] + ((d[5] & RKA_MASK) ? d[4] : 0);
+        k_check_offsets<<<grid_for(d[0] + 1, t->ctx->sm_count * 4), RK_TPB, 0, st>>>(off, d[0], d[1], bad.p);
+        CUDA_TRY(cudaGetLastError());
+        *launches += 1;
+    }
+    unsigned long long flag = 0;
+    CUDA_TRY(cudaMemcpyAsync(&flag, bad.p, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    if (flag) { mlg_set_error("read archive blob of rank %u: read offsets that do not start at 0, ascend and end at the batch's bases", rank); return MLG_ERR_ARG; }
+
+    t->added[rank] = 1; t->peers += 1;
+    const unsigned long long add = bytes - head * 8;
+    if (h[3]) {                                           // that rank's archive overflowed: so does the count on every rank
+        if (!t->overflowed) MLG_TRY(rkp_overflow(t, 0));
+        t->overflowed_rank = (int)rank;
+        return MLG_OK;
+    }
+    if (t->overflowed) { t->bytes_needed += add; return MLG_OK; }
+    if (t->budget && t->archive_bytes + add > t->budget) return rkp_overflow(t, add);
+    for (unsigned long long i = 0; i < nb; ++i) {
+        const unsigned long long* d = h.data() + RKA_HEAD_WORDS + i * RKA_DESC_WORDS;
+        t->batches.emplace_back();
+        ArchivedBatch& b = t->batches.back();
+        const bool m = d[5] & RKA_MASK, o = d[5] & RKA_OFF;
+        if (b.bases.alloc(d[3]) != MLG_OK || (m && b.nmask.alloc(d[4]) != MLG_OK) || (o && b.off.alloc(d[0] + 1) != MLG_OK)) return rkp_overflow(t, add);
+        const unsigned long long* p = data[i];
+        CUDA_TRY(cudaMemcpyAsync(b.bases.p, p, d[3] * 8, cudaMemcpyDeviceToDevice, st)); p += d[3];
+        if (m) { CUDA_TRY(cudaMemcpyAsync(b.nmask.p, p, d[4] * 8, cudaMemcpyDeviceToDevice, st)); p += d[4]; }
+        if (o) CUDA_TRY(cudaMemcpyAsync(b.off.p, p, (d[0] + 1) * 8, cudaMemcpyDeviceToDevice, st));
+        b.n_reads = d[0]; b.nbases = d[1]; b.read_len = (uint32_t)d[2]; b.base_words = d[3]; b.nmask_words = d[4];
+    }
+    t->archive_bytes += add;
+    return MLG_OK;
+}
+
+uint32_t rkp_peers_missing(const ReadKmerPasses* t) { return t->world - 1 - t->peers; }
+
+// ---------------------------------------------------------------- mlg_kmc_concat
+// Version-0 KMC databases whose keys ascend from one to the next, joined into one: the suffix bodies streamed one after
+// the other (copy_file_range, or reads and writes of 64 MiB), the prefix tables summed, the header of the parts with the
+// summed total.  Only the prefix files, the first and last record of each part and the file sizes are read to check them.
+namespace {
+
+constexpr unsigned long long KMC_HEADER_BYTES = 64;      // version 0: k .. kmc_version
+
+struct KmcPart {
+    std::string pre, suf;
+    KmcHeader h;
+    std::vector<unsigned long long> lut;
+    unsigned long long rec = 0;
+    u128 first = 0, last = 0;
+    struct stat st_pre{}, st_suf{};
+};
+
+bool slurp(const std::string& path, std::vector<unsigned char>& out) {
+    FILE* f = fopen(path.c_str(), "rb");
+    if (!f) return false;
+    bool ok = fseek(f, 0, SEEK_END) == 0;
+    const long n = ok ? ftell(f) : -1;
+    ok = ok && n >= 0 && fseek(f, 0, SEEK_SET) == 0;
+    if (ok) { out.resize((size_t)n); ok = fread(out.data(), 1, out.size(), f) == out.size(); }
+    fclose(f);
+    return ok;
+}
+
+bool pread_all(int fd, void* buf, size_t n, off_t at) {
+    unsigned char* b = (unsigned char*)buf;
+    while (n) {
+        const ssize_t r = pread(fd, b, n, at);
+        if (r <= 0) return false;
+        b += r; n -= (size_t)r; at += r;
+    }
+    return true;
+}
+
+// the key of record r of a part: its prefix from the prefix table, its suffix bytes from the suffix file
+bool record_key(const KmcPart& P, int fd, unsigned long long r, u128* key) {
+    const unsigned long long np = P.lut.size() - 1;
+    unsigned long long lo = 0, hi = np;              // the prefix i with lut[i] <= r < lut[i + 1]
+    while (hi - lo > 1) { const unsigned long long m = (lo + hi) / 2; if (P.lut[m] <= r) lo = m; else hi = m; }
+    const uint32_t sb = (P.h.K - P.h.p) / 4;
+    unsigned char b[16];
+    if (!pread_all(fd, b, sb, 4 + (off_t)(r * P.rec))) return false;
+    u128 k = lo;
+    for (uint32_t j = 0; j < sb; ++j) k = (k << 8) | b[j];
+    *key = k;
+    return true;
+}
+
+int read_part(const char* prefix, KmcPart& P) {
+    P.pre = std::string(prefix) + ".kmc_pre"; P.suf = std::string(prefix) + ".kmc_suf";
+    std::vector<unsigned char> pre;
+    if (!slurp(P.pre, pre) || stat(P.pre.c_str(), &P.st_pre) != 0) { mlg_set_error("cannot read %s", P.pre.c_str()); return MLG_ERR_IO; }
+    auto u32 = [&](size_t at) { uint32_t v; memcpy(&v, pre.data() + at, 4); return v; };
+    const size_t n = pre.size();
+    if (n < 8 + 8 + KMC_HEADER_BYTES + 8 || memcmp(pre.data(), "KMCP", 4) || memcmp(pre.data() + n - 4, "KMCP", 4) ||
+        u32(n - 8) != KMC_HEADER_BYTES || u32(n - 12) != 0) {
+        mlg_set_error("%s is not the prefix file of a version-0 KMC database", P.pre.c_str()); return MLG_ERR_ARG;
+    }
+    const size_t h0 = n - 8 - KMC_HEADER_BYTES;
+    KmcHeader& h = P.h;
+    h.K = u32(h0); h.mode = u32(h0 + 4); h.counter_size = u32(h0 + 8); h.p = u32(h0 + 12); h.min_count = u32(h0 + 16);
+    memcpy(&h.total, pre.data() + h0 + 24, 8);
+    h.strands = pre[h0 + 32];
+    h.max_count = u32(h0 + 20) | (unsigned long long)u32(h0 + 36) << 32;
+    const bool shape = h.p >= 1 && h.p <= 15 && h.K > h.p && h.K <= 64 && (h.K - h.p) % 4 == 0 && h.counter_size >= 1 && h.counter_size <= 4 &&
+                       h0 == 4 + ((1ull << (2 * h.p)) + 1) * 8;
+    if (!shape) { mlg_set_error("%s: k = %u, lut_prefix_length = %u, counter_size = %u and its prefix table do not fit together", P.pre.c_str(), h.K, h.p, h.counter_size); return MLG_ERR_ARG; }
+    P.lut.resize((1ull << (2 * h.p)) + 1);
+    memcpy(P.lut.data(), pre.data() + 4, P.lut.size() * 8);
+    bool mono = P.lut[0] == 0 && P.lut.back() == h.total;
+    for (size_t i = 1; mono && i < P.lut.size(); ++i) mono = P.lut[i - 1] <= P.lut[i];
+    if (!mono) { mlg_set_error("%s: the prefix table does not ascend to the total of %llu k-mers", P.pre.c_str(), h.total); return MLG_ERR_ARG; }
+    P.rec = (h.K - h.p) / 4 + h.counter_size;
+    const int fd = open(P.suf.c_str(), O_RDONLY);
+    if (fd < 0) { mlg_set_error("cannot read %s", P.suf.c_str()); return MLG_ERR_IO; }
+    struct Fd { int f; ~Fd() { close(f); } } guard{fd};
+    char m0[4], m1[4];
+    if (fstat(fd, &P.st_suf) != 0 || (u128)P.st_suf.st_size != 8 + (u128)h.total * P.rec || !pread_all(fd, m0, 4, 0) ||
+        !pread_all(fd, m1, 4, P.st_suf.st_size - 4) || memcmp(m0, "KMCS", 4) || memcmp(m1, "KMCS", 4)) {
+        mlg_set_error("%s does not hold the %llu records of %s", P.suf.c_str(), h.total, P.pre.c_str()); return MLG_ERR_ARG;
+    }
+    if (h.total && (!record_key(P, fd, 0, &P.first) || !record_key(P, fd, h.total - 1, &P.last))) { mlg_set_error("cannot read %s", P.suf.c_str()); return MLG_ERR_IO; }
+    return MLG_OK;
+}
+
+// bytes [at, at + n) of `in` appended to `out`
+bool copy_range(int in, off_t at, unsigned long long n, int out, std::vector<unsigned char>& buf) {
+    bool plain = false;
+    while (n) {
+        const size_t c = (size_t)std::min<unsigned long long>(n, 1ull << 30);
+        ssize_t r = -1;
+        if (!plain) {
+            loff_t a = at;
+            r = copy_file_range(in, &a, out, nullptr, c, 0);
+            if (r < 0 && (errno == EXDEV || errno == ENOSYS || errno == EINVAL || errno == EOPNOTSUPP || errno == EBADF)) { plain = true; continue; }
+        } else {
+            if (buf.empty()) buf.resize(64ull << 20);
+            const size_t m = std::min(c, buf.size());
+            if (!pread_all(in, buf.data(), m, at)) return false;
+            for (size_t w = 0; w < m;) { const ssize_t k = write(out, buf.data() + w, m - w); if (k <= 0) return false; w += (size_t)k; }
+            r = (ssize_t)m;
+        }
+        if (r <= 0) return false;
+        at += r; n -= (unsigned long long)r;
+    }
+    return true;
+}
+
+}  // namespace
+
+int kmc_concat(const char* prefix, const char* const* parts, uint32_t n_parts) {
+    std::vector<KmcPart> P(n_parts);
+    for (uint32_t i = 0; i < n_parts; ++i) {
+        MLG_TRY(read_part(parts[i], P[i]));
+        const KmcHeader &a = P[0].h, &b = P[i].h;
+        if (a.K != b.K || a.mode != b.mode || a.counter_size != b.counter_size || a.p != b.p || a.min_count != b.min_count ||
+            a.max_count != b.max_count || a.strands != b.strands) {
+            mlg_set_error("%s: its header (k, mode, counter size, lut_prefix_length, min / max count or strands) differs from %s's", parts[i], parts[0]);
+            return MLG_ERR_ARG;
+        }
+    }
+    const KmcPart* prev = nullptr;
+    for (const KmcPart& x : P) {
+        if (!x.h.total) continue;
+        if (prev && !(prev->last < x.first)) { mlg_set_error("%s does not start after the last k-mer of %s", x.pre.c_str(), prev->pre.c_str()); return MLG_ERR_ARG; }
+        prev = &x;
+    }
+    const std::string pre_path = std::string(prefix) + ".kmc_pre", suf_path = std::string(prefix) + ".kmc_suf";
+    for (const std::string& o : {pre_path, suf_path}) {
+        struct stat so;
+        if (stat(o.c_str(), &so) != 0) continue;
+        for (const KmcPart& x : P)
+            for (const struct stat* sp : {&x.st_pre, &x.st_suf})
+                if (sp->st_dev == so.st_dev && sp->st_ino == so.st_ino) { mlg_set_error("%s is one of the parts", o.c_str()); return MLG_ERR_ARG; }
+    }
+    KmcHeader h = P[0].h;
+    h.total = 0;
+    std::vector<unsigned long long> lut(P[0].lut.size(), 0);
+    for (const KmcPart& x : P) {
+        h.total += x.h.total;
+        for (size_t i = 0; i < lut.size(); ++i) lut[i] += x.lut[i];
+    }
+    struct Out { std::string pre, suf; int fd = -1; bool done = false;
+                 ~Out() { if (fd >= 0) close(fd); if (!done) { remove(suf.c_str()); remove(pre.c_str()); } } } out{pre_path, suf_path};
+    out.fd = open(suf_path.c_str(), O_WRONLY | O_CREAT | O_TRUNC, 0644);
+    if (out.fd < 0) { mlg_set_error("cannot create %s", suf_path.c_str()); return MLG_ERR_IO; }
+    std::vector<unsigned char> buf;
+    bool ok = write(out.fd, "KMCS", 4) == 4;
+    for (const KmcPart& x : P) {
+        if (!ok || !x.h.total) continue;
+        const int in = open(x.suf.c_str(), O_RDONLY);
+        ok = in >= 0 && copy_range(in, 4, x.h.total * x.rec, out.fd, buf);
+        if (in >= 0) close(in);
+    }
+    ok = ok && write(out.fd, "KMCS", 4) == 4;
+    ok = (close(out.fd) == 0) && ok;
+    out.fd = -1;
+    if (!ok) { mlg_set_error("%s: short write (%s)", suf_path.c_str(), strerror(errno)); return MLG_ERR_IO; }
+    unsigned long long pre_bytes = 0;
+    MLG_TRY(kmc_write_pre(pre_path, lut, h, &pre_bytes));
+    out.done = true;
+    return MLG_OK;
+}

@@ -11,6 +11,10 @@ The sum comes in two equivalent forms (NCCL over NVLink on GPUs, gloo on CPU):
   "dense"             one uint8 sum all-reduce of the whole table (|D| bytes, 0.16 GB for the default-scale
                       database) -- MLG_EXCHANGE=dense.
 
+The read k-mers of sharded reads (reads_60mers) take another route: share_read_kmers hands every rank's device copy
+of its reads to every other rank, each rank counts one share of the k-mer key order over all the reads, and
+write_reads_kmc joins the ranks' KMC databases into one file.
+
 The reference has nothing to compare with (it is a single process around subprocesses,
 scripts/select_db.py:50-76); this module is the new host-side plumbing, on torch.distributed.
 """
@@ -207,6 +211,120 @@ def reduce_query(query, device: int = 0, group=None, mode: str = None) -> None:
 
     query._exchange_retry = lambda need: run(1 << (2 * int(need) - 1).bit_length())
     run()
+
+
+def _world_rank(group):
+    import torch.distributed as dist
+    if dist.is_initialized():
+        return dist.get_world_size(group), dist.get_rank(group)
+    return 1, 0
+
+
+def _flag_min(ok: bool, device: int, group) -> bool:
+    """every rank's ok, and-ed over the ranks"""
+    import torch
+    import torch.distributed as dist
+    if _world_rank(group)[0] == 1:
+        return ok
+    on_gpu = dist.get_backend(group) == "nccl"
+    t = torch.tensor([1 if ok else 0], dtype=torch.int32, device="cuda:%d" % device if on_gpu else "cpu")
+    dist.all_reduce(t, op=dist.ReduceOp.MIN, group=group)
+    return bool(t.item())
+
+
+def share_read_kmers(query, device: int = 0, group=None) -> None:
+    """Collective: make this passes-mode query (Database.query(read_kmers=True, read_kmer_passes=True), every read pushed)
+    rank r of a W-rank read k-mer count.  Every rank's device copy of its reads goes to every other rank -- an all-gather
+    of the blob sizes, then one broadcast per source rank on the library's compute stream, each followed by the import on
+    the receivers -- so that read_kmers / write_reads_kmc of rank r give share r of the key order, counted over all the
+    reads.  Peak memory beside the archive: this rank's blob plus one receive buffer as large as the largest peer's blob,
+    returned to the device when the exchange ends.  Reads move, not k-mers: the reads are 0.375 bytes per base, their
+    distinct k-mers many times that.  A rank that fails (its blob, the receive buffer or an import) still takes part in
+    every broadcast, and then every rank raises."""
+    import torch
+    import torch.distributed as dist
+    world, rank = _world_rank(group)
+    if world == 1:
+        query.read_kmer_archive(0, 1)
+        return
+    err, ptr, nbytes = None, 0, 0
+    try:
+        ptr, nbytes = query.read_kmer_archive(rank, world)
+    except Exception as e:  # noqa: BLE001  (every rank has to take part in the collectives below)
+        err = e
+    dev = "cuda:%d" % device
+    n = torch.tensor([nbytes if err is None else -1], dtype=torch.int64, device=dev)
+    sizes = torch.empty(world, dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(sizes, n, group=group)
+    sizes = sizes.tolist()
+    if min(sizes) < 0:
+        raise err or RuntimeError("read k-mer exchange: a rank could not pack its read archive")
+    comp = _comp_stream(query.db.ctx, device)
+    recv = None
+    try:
+        with torch.cuda.stream(comp):
+            recv = torch.empty(max(sizes[r] for r in range(world) if r != rank), dtype=torch.uint8, device=dev)
+    except Exception as e:  # noqa: BLE001
+        err = e
+    if not _flag_min(err is None, device, group):
+        raise err or RuntimeError("read k-mer exchange: a rank could not allocate its receive buffer")
+    try:
+        with torch.cuda.stream(comp):
+            for src in range(world):
+                buf = device_view_u8(ptr, nbytes, device) if src == rank else recv[:sizes[src]]
+                dist.broadcast(buf, src=src if group is None else dist.get_global_rank(group, src), group=group)
+                if src != rank and err is None:
+                    try:
+                        query.add_read_kmer_archive(buf.data_ptr(), sizes[src])
+                    except Exception as e:  # noqa: BLE001
+                        err = e
+        ok = _flag_min(err is None, device, group)
+    finally:
+        comp.synchronize()
+        del recv
+        torch.cuda.empty_cache()                 # budget 0 plans the passes from the free device memory
+    if not ok:
+        raise err or RuntimeError("read k-mer exchange: another rank could not add a peer's archive")
+
+
+def write_reads_kmc(query, prefix: str, min_count: int = 2, counter_max: int = 3, device: int = 0, group=None) -> dict:
+    """Collective, after share_read_kmers: <prefix>.kmc_pre / .kmc_suf of all the ranks' reads, the file a single query
+    over all of them writes.  Every rank writes its share as <prefix>.part<r>, rank 0 joins the parts (api.kmc_concat),
+    and the parts are removed whatever happens; if any rank fails, every rank raises and no database is left.  Rank 0
+    reads every rank's part, so across nodes the prefix must be on storage every rank shares.  Returns the seconds this
+    rank spent writing its part and (rank 0) joining the parts."""
+    import time
+    from .api import kmc_concat
+    world, rank = _world_rank(group)
+    parts = ["%s.part%d" % (prefix, r) for r in range(world)]
+    err = None
+    t0 = time.perf_counter()
+    try:
+        query.write_reads_kmc(parts[rank], min_count, counter_max)
+    except Exception as e:  # noqa: BLE001  (every rank has to take part in the all-reduces below)
+        err = e
+    times = dict(part_s=time.perf_counter() - t0, concat_s=0.0)
+    try:
+        written = _flag_min(err is None, device, group)
+        if rank == 0 and written:
+            t0 = time.perf_counter()
+            try:
+                kmc_concat(prefix, parts)
+            except Exception as e:  # noqa: BLE001
+                err = e
+            times["concat_s"] = time.perf_counter() - t0
+        joined = _flag_min(err is None, device, group) and written
+    finally:
+        for ext in (".kmc_pre", ".kmc_suf"):
+            try:
+                os.remove(parts[rank] + ext)
+            except FileNotFoundError:
+                pass
+    if err is not None:
+        raise err
+    if not joined:
+        raise RuntimeError("the reads KMC database %s was not written: another rank failed" % prefix)
+    return times
 
 
 def close_exchanges():
