@@ -313,9 +313,16 @@ int mlg_query_read_kmer_stats(mlg_query* q, mlg_read_kmer_stats* out);
  * text[genome_off[g] .. genome_off[g+1]) that consists of ACGT/acgt only is upper-cased and hashed with
  * MurmurHash3_x64_128 (seed 0, first 64-bit word) modulo `prime` (0 = CMash's 9999999999971); a genome's sketch is its n
  * smallest distinct hash values in ascending order.  Records (contigs) of one genome are separated by any non-ACGT byte.
- * Outputs (host, G*n slots): mins (prime where the slot is unused), counts (occurrences of the hash in the genome),
- * kmers (K bytes per slot: the first k-mer with that hash, upper case; NUL-filled where unused -- the layout
- * mlg_db_from_ascii takes).  G < 2^20 genomes per call. */
+ * Outputs (host, G*n slots): mins (prime where the slot is unused), counts, kmers (K bytes per slot: the first k-mer
+ * with that hash, upper case; NUL-filled where unused -- the layout mlg_db_from_ascii takes).  counts are CountEstimator's:
+ * the occurrences of the hash in the genome, except in the last slot of a full sketch, whose repeats stop counting once
+ * the n-1 smaller hashes have all appeared (`h >= mins[-1]` returns early): there it is the number of occurrences before
+ * that moment, and at least 1 (so always 1 when n = 1); 0 where the slot is unused.
+ * Refused with MLG_ERR_ARG before anything is written: null pointers, K outside 1..64, n = 0, G = 0 or G >= 2^20,
+ * prime = 1 or prime >= 2^44, a genome_off that decreases anywhere, a single genome of about 4 GB or more.
+ * The text goes to the device in passes of about 1 GB (whole genomes; a genome larger than that has a pass of its own);
+ * the environment variable MLG_SKETCH_PASS_BYTES, read on every call, sets the bytes per pass instead (any value >= 1;
+ * an experiment and test knob, the results do not depend on it). */
 typedef struct mlg_sketch_stats {
     uint64_t n_windows;      /* N-free K-long windows hashed */
     uint64_t n_candidates;   /* windows below their genome's threshold (sorted and ranked) */

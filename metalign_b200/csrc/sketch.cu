@@ -18,6 +18,7 @@
 // Instruction-bound (two 64-bit multiplies per 8 bytes), not HBM-bound: every base is read once from DRAM.
 #include <cub/cub.cuh>
 #include <algorithm>
+#include <stdlib.h>
 #include <string.h>
 #include "mlg_internal.h"
 
@@ -30,6 +31,8 @@ namespace {
 constexpr int TPB = 256;
 constexpr uint32_t TILE = 4096;           // windows per CTA pass
 constexpr unsigned HBITS = 44;            // hash values are < prime < 2^44
+// device text of one pass, separators and 64 bytes of padding included, stays below this: positions are 32-bit
+constexpr unsigned long long PASS_LIMIT = 0xFFFFFFF0ull;
 
 __device__ __forceinline__ unsigned long long rotl64(unsigned long long x, int r) { return (x << r) | (x >> (64 - r)); }
 __device__ __forceinline__ unsigned long long fmix64(unsigned long long k) {
@@ -211,7 +214,7 @@ static int sketch_pass(mlg_ctx* ctx, const char* text, const uint64_t* off, cons
         total += len + 1;
     }
     d_off[ng] = total;
-    if (total + 64 >= 0xFFFFFFF0ull) { mlg_set_error("sketch batch of %llu bytes is too large (< 4 GB per pass)", total); return MLG_ERR_ARG; }
+    if (total + 64 >= PASS_LIMIT) { mlg_set_error("sketch batch of %llu bytes is too large (< 4 GB per pass)", total); return MLG_ERR_ARG; }
     const unsigned long long padded = (total + 128 + 15) & ~15ull;
     std::vector<unsigned char> h_text(padded, (unsigned char)'N');
     for (uint32_t i = 0; i < ng; ++i) memcpy(h_text.data() + d_off[i], text + off[idx[i]], off[idx[i] + 1] - off[idx[i]]);
@@ -317,12 +320,24 @@ MLG_API int mlg_sketch_genomes(mlg_ctx* ctx, const char* text, const uint64_t* g
     if (n < 1 || G < 1 || G >= (1u << 20)) { mlg_set_error("need n >= 1 and 1 <= G < 2^20 genomes per call"); return MLG_ERR_ARG; }
     if (prime == 0) prime = 9999999999971ull;
     if (prime < 2 || prime >= (1ull << HBITS)) { mlg_set_error("prime must be below 2^44"); return MLG_ERR_ARG; }
+    // a genome is never split: each one has to fit in one pass (its separator and the padding included)
+    const unsigned long long max_len = PASS_LIMIT - 66;
+    for (uint32_t g = 0; g < G; ++g) {
+        if (genome_off[g + 1] < genome_off[g]) { mlg_set_error("genome_off decreases at genome %u", g); return MLG_ERR_ARG; }
+        if (genome_off[g + 1] - genome_off[g] > max_len) { mlg_set_error("genome %u is too large (< 4 GB per genome)", g); return MLG_ERR_ARG; }
+    }
+    // bytes of text per pass; MLG_SKETCH_PASS_BYTES (experiment and test knob, read on every call): any value >= 1
+    unsigned long long pass_bytes = 1ull << 30;
+    if (const char* e = getenv("MLG_SKETCH_PASS_BYTES")) {
+        const unsigned long long v = strtoull(e, nullptr, 10);
+        if (v >= 1) pass_bytes = std::min(v, max_len);
+    }
     CUDA_TRY(cudaSetDevice(ctx->device));
     if (st) memset(st, 0, sizeof(*st));
     std::vector<double> tmul(G, 1.0);
     std::vector<uint32_t> todo(G), redo;
     for (uint32_t g = 0; g < G; ++g) todo[g] = g;
-    // passes of at most ~1 GB of text
+    // passes of at most pass_bytes of text (a genome larger than that gets a pass of its own)
     while (!todo.empty()) {
         redo.clear();
         size_t i = 0;
@@ -331,7 +346,7 @@ MLG_API int mlg_sketch_genomes(mlg_ctx* ctx, const char* text, const uint64_t* g
             unsigned long long bytes = 0;
             while (i < todo.size()) {
                 const unsigned long long len = genome_off[todo[i] + 1] - genome_off[todo[i]];
-                if (!batch.empty() && bytes + len > (1ull << 30)) break;
+                if (!batch.empty() && bytes + len > pass_bytes) break;
                 batch.push_back(todo[i]); bytes += len + 1; ++i;
             }
             MLG_TRY(sketch_pass(ctx, text, genome_off, batch, tmul, n, K, prime, mins, counts, kmers, st, redo));

@@ -24,6 +24,7 @@ from . import _lib
 from ._lib import check
 
 PRIME = 9999999999971      # CMash MinHash.CountEstimator's default max_prime (itself prime)
+GENOMES_PER_CALL = (1 << 20) - 1   # mlg_sketch_genomes takes G < 2^20 genomes per call
 
 
 def read_fasta(path: str) -> bytes:
@@ -62,7 +63,8 @@ def sketch_genomes(ctx, genomes: Sequence[bytes], n: int = 1000, K: int = 60, pr
 
 def build_database(ctx, paths: Iterable[str], out_path: str, n: int = 1000, K: int = 60, ks: Sequence[int] = (30, 40, 50, 60),
                    batch_bytes: int = 1 << 30, log=None):
-    """Sketch every genome file and write the .mlgdb database (metalign_b200/dbformat.py).  Returns the stats."""
+    """Sketch every genome file and write the .mlgdb database (metalign_b200/dbformat.py).  Returns the stats.
+    Genomes go to the GPU in calls of about batch_bytes of text and at most GENOMES_PER_CALL genomes."""
     from . import codec, dbformat
     paths = sorted(paths, key=os.path.basename)
     names = [os.path.basename(p) for p in paths]
@@ -72,7 +74,7 @@ def build_database(ctx, paths: Iterable[str], out_path: str, n: int = 1000, K: i
     i = 0
     while i < G:
         batch, nbytes = [], 0
-        while i < G and (not batch or nbytes < batch_bytes):
+        while i < G and (not batch or nbytes < batch_bytes) and len(batch) < GENOMES_PER_CALL:
             batch.append(read_fasta(paths[i]))
             nbytes += len(batch[-1])
             i += 1
@@ -96,8 +98,18 @@ def main(argv=None):
     ap.add_argument("--k_range", default="30-60-10", help="prefix lengths the database will be queried at")
     ap.add_argument("--device", type=int, default=0)
     a = ap.parse_args(argv)
-    lo, hi, step = (int(x) for x in a.k_range.split("-"))
+    # what the database loader accepts (1 <= K <= 63, 1..8 ascending ks within 1..K), checked before any genome is read
+    if not 1 <= a.k_size <= 63:
+        ap.error("-k %d: a database needs 1 <= K <= 63" % a.k_size)
+    try:
+        lo, hi, step = (int(x) for x in a.k_range.split("-"))
+    except ValueError:
+        ap.error("--k_range %s: expected lo-hi-step" % a.k_range)
+    if lo < 1 or step < 1:
+        ap.error("--k_range %s: need lo >= 1 and step >= 1" % a.k_range)
     ks = [k for k in range(lo, hi + 1, step) if k <= a.k_size]
+    if not 1 <= len(ks) <= 8:
+        ap.error("--k_range %s with -k %d gives %d prefix lengths %s; a database needs 1 to 8" % (a.k_range, a.k_size, len(ks), ks))
     with open(a.in_file) as f:
         paths = [ln.strip() for ln in f if ln.strip()]
     from .api import Context
