@@ -12,23 +12,30 @@ namespace {
 // per-warp TMA pipelines as the super-k-mer kernel above, but the minimizer is a 32-mer whose (order << 6 | position)
 // value is two multiply-adds, level 1 is a bit array over minimizer IDENTITIES, and there is no per-window compare:
 //   phase A  sliding minimum over the 29 32-mers under each window (van Herk / Gil-Werman on blocks of 16 positions)
-//            and the runs of equal minimizer; values of new runs go to a per-lane list in shared memory;
-//   lookup   for up to MZ_MAXRUN runs per block of 16 windows the lane fetches the two halves of the minimizer from its
-//            copy of the segment in shared memory (the position is in the value), mixes their identity and loads the
-//            bit-array word (predicated LDG);
-//   deferred the words are looked at one block LATER (after the next block's phase A, which hides the DRAM latency):
-//            a run whose bit is set becomes an ITEM (source lane, first window of the block, identity, 16-bit mask of
-//            its valid windows) in a per-warp ring in shared memory.
+//            and the runs of equal minimizer, block by block; every run start goes to the lane's run list in shared
+//            memory (one byte: the minimizer's position relative to the run's first block) and to a 96-bit mask of the
+//            segment's run starts in registers;
+//   lookup   after the segment's blocks, the warp walks the lists slot by slot up to its longest one: the lane fetches the
+//            two halves of its run's minimizer from its copy of the segment in shared memory, mixes their identity and
+//            loads the bit-array word (predicated LDG), MZ_LGROUP slots' loads in flight before the first is looked at;
+//            a run whose two bits are set becomes ITEMS (stream position of a block's first window, 16-bit mask of the
+//            run's valid windows in that block, minimizer position) in a per-warp list in shared memory, one item for
+//            each block of 16 windows the run touches (a run covers at most 29 windows: at most 3 items).
 // Items are rare (bit density <= 1/32, plus the true hits); the ring is drained 32 at a time, one item per lane: the
 // lane rebuilds the canonical key of each window of the item from the staged bases and compares it with the database
 // k-mers filed under that identity (bucket index on the identity's high word, plus the alias table).
 #ifndef MZ_MINCTAS
 #define MZ_MINCTAS 2
 #endif
-constexpr unsigned MZ_MAXRUN = 4;             // runs per block whose bit-array word is fetched ahead (the carried one + 3 new)
+// slots looked up together: their loads are all issued before the first word is looked at.  8 was slower on a B200
+// (K1 1.98 against 1.90 ms: ~13 slots per read round up to 16, and twice the unrolled code)
+constexpr unsigned MZ_LGROUP = 4;
 constexpr unsigned MZ_QDRAIN = 32;            // per-warp item list: drained whenever this many are waiting ...
-constexpr unsigned MZ_QCAP = MZ_QDRAIN + 128; // ... and one block of 16 windows adds at most 4 x 32
-constexpr unsigned MZ_LIST = 16;              // run list rows: a block of 16 windows starts at most 15 new runs (row 0 unused)
+constexpr unsigned MZ_QCAP = MZ_QDRAIN + 128; // ... and one run adds at most 3 x 32
+constexpr unsigned MZ_LIST = 64;              // run list slots per lane (bytes)
+constexpr unsigned MZ_CAP = MZ_LIST - 16;     // runs of a segment that are looked up: a block's 16 stores start at slot <= MZ_CAP
+                                              // and stay inside the list; later runs go to the drain untested (~7 per segment
+                                              // of random sequence, 96 at most)
 constexpr uint32_t MZ_M64 = MLG_MZ_ORD_MULT << 6;   // the multiplier carries the << 6 of (order << 6 | position)
 // reads per hand-out: one tile counter increment, one TMA issue and one mbarrier wait serve MZ_TILE_READS / 32 warp
 // passes.  64 halves the share of the per-tile code (~300 instructions on one lane) but doubles the staging buffers:
@@ -46,7 +53,8 @@ struct MzStage {
 };
 struct MzShared {
     MzStage stg;
-    uint32_t wm[MZ_LIST][RT];                 // [r][thread]: value of the r-th run START of the current block (r >= 1)
+    unsigned char rl[MZ_LIST][RT];            // [r][thread]: low byte of the r-th run's minimum of the current segment
+                                              //       (its minimizer's position relative to the run's first block)
     uint32_t seq[SEGW + 1][RT];               // [word][thread]: the lane's current segment (160 bases, top-aligned words)
     uint32_t qa[WARPS][MZ_QCAP];              // item: stream position (in bases) of the block's first window, low / high word
     uint32_t qc[WARPS][MZ_QCAP];
@@ -55,7 +63,7 @@ struct MzShared {
     uint32_t qoff[WARPS][32];                 // drain: windows before each item of the batch
     uint32_t qn[WARPS];                       // items waiting
 };
-constexpr uint32_t MZ_ROW = RT * 4;           // byte stride between rows of wm[] / seq[]
+constexpr uint32_t MZ_ROW = RT * 4;           // byte stride between rows of seq[]
 
 // The L2::64B qualifier matters: without a prefetch-size qualifier a miss on this part moves 128 bytes from HBM for
 // every random 4-byte access (3.8 sectors per request, whatever the load's width or cache policy); with it, 64
@@ -85,6 +93,12 @@ __device__ __forceinline__ uint32_t ldg_bitmap_if(bool p, const uint32_t* ptr) {
 __device__ __forceinline__ uint32_t ldg_u32(const uint32_t* ptr) {
     uint32_t r;
     asm volatile("ld.global.nc" MZ_L2Q ".b32 %0, [%1];" : "=r"(r) : "l"(ptr));
+    return r;
+}
+__device__ __forceinline__ void sts8(uint32_t addr, uint32_t v) { asm volatile("st.shared.u8 [%0], %1;" ::"r"(addr), "r"(v) : "memory"); }
+__device__ __forceinline__ uint32_t lds8(uint32_t addr) {
+    uint32_t r;
+    asm volatile("ld.shared.u8 %0, [%1];" : "=r"(r) : "r"(addr));
     return r;
 }
 __device__ __forceinline__ key128 ldg_key(const key128* ptr) {
@@ -207,7 +221,7 @@ __device__ __noinline__ void mz_drain(uint32_t* qn, const uint32_t* qa, const ui
     for (uint32_t base = 0; base < n; base += 32u) {
         const uint32_t i = base + lane;
         uint32_t kb0 = i < n ? qb[i] : 0u;
-        // Items of runs beyond the fourth of their block arrive untested (bit 31).  Their level-1 bits are looked at here,
+        // Items of runs beyond the run list's capacity arrive untested (bit 31).  Their level-1 bits are looked at here,
         // once per ITEM and 32 items at a time, before the items are spread over the lanes window by window: 99.6 % of
         // them fail, and used to cost every one of their ~11 windows a lookup of its own.
         if (__any_sync(FULL, (kb0 >> 31) != 0u)) {
@@ -283,7 +297,7 @@ __global__ void __launch_bounds__(RT, MZ_MINCTAS) k1_minimizer_probe(const __gri
     unsigned long long pol_stream;
     asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol_stream));
 #endif
-    const uint32_t wm_base = smem_u32(&sm.wm[0][tid]), seq_base = smem_u32(&sm.seq[0][tid]);
+    const uint32_t rl_base = smem_u32(&sm.rl[0][tid]), seq_base = smem_u32(&sm.seq[0][tid]);
     const uint32_t* const MB = db.F;
     const uint32_t lt_mask = (1u << lane) - 1u;
     // bit index = identity & (2^fbits - 1): mask of its low word, and of its high word (0 up to 2^32 bits)
@@ -409,142 +423,147 @@ __global__ void __launch_bounds__(RT, MZ_MINCTAS) k1_minimizer_probe(const __gri
             uint32_t P = 0xFFFFFFFFu;
 #pragma unroll
             for (int i = 0; i < 12; ++i) P = min(P, mz_val(loc, rcl, 1, i));
-            // the value of the run the lane is in, re-based to the coming block (positions are block-relative), and
-            // whether its bit is set
-            uint32_t held_wm = 0;
-            bool have = false, held_pass = false;
-
-            // Block b's runs are found by phase A in pass b; their bit-array words are loaded at the START of pass b + 1 and
-            // looked at after that pass's phase A, which hides the DRAM latency.  Loads and their use sit in the same loop
-            // body (nothing is in flight across the back edge), and no vote or other convergence point lies between them.
-            bool pend = false, pneed0 = false, more = true;          // more: the segment has valid windows (checked above)
-            uint32_t pW = 0, pchg = 0, pvm = 0, pnr = 0, pblk = 0;   // pW: positions of the minimizers of runs 0..3 (8 bits each)
-            uint32_t pX0 = 0, pX1 = 0, pX2 = 0, pX3 = 0, pbits = 0, pbit2 = 0;  // word index and the two bits (8 bits each) of their lookups
+            // blocks the warp walks: up to the last one in which some lane has a valid window
+            const int lastv = v2 ? 96 - __ffs(v2) : v1 ? 64 - __ffs(v1) : v0 ? 32 - __ffs(v0) : -1;
+            const unsigned nblk = __reduce_max_sync(FULL, (unsigned)(lastv + 16) >> 4);
+            // Phase A, block by block.  Every run start goes to the run list (the low byte of the window minimum: the
+            // minimizer's position relative to the block) and to c0..c2 (bit w = window w, shifted in from the top).  No
+            // window is dropped for validity here: a window that is not valid costs at most a wasted lookup; it is masked
+            // out of the items.
+            uint32_t pw = 0xFFFFFFFFu;                // minimum of the previous window (none before window 0: no value is ~0)
+            uint32_t lst = rl_base;                   // where the next run's byte goes
+            uint32_t c0 = 0, c1 = 0, c2 = 0;
 #pragma unroll 1
-            for (int blk = 0;; ++blk) {
-                const uint32_t blk16 = (uint32_t)blk * 16u;
-                // ---- load the bit-array words of the previous block's runs 0..3
-                uint32_t F0 = 0, F1 = 0, F2 = 0, F3 = 0;
-                if (pend) {
-                    F0 = ldg_bitmap_if(pneed0, MB + pX0);
-                    F1 = ldg_bitmap_if(pnr > 1u, MB + pX1);
-                    F2 = ldg_bitmap_if(pnr > 2u, MB + pX2);
-                    F3 = ldg_bitmap_if(pnr > 3u, MB + pX3);
-                    my_fetch += (pneed0 ? 1u : 0u) + pnr - 1u;
-                }
-                // ---- phase A of this block: window minima and runs of equal minimizer (validity is ignored here: a window
-                //      that is not valid costs at most a wasted lookup; it is masked out of the items)
-                uint32_t chgraw = 0, wm_first = 0, vb = 0;
-                if (more) {
-                    vb = v0 & 0xFFFF0000u;
-                    v0 = fsl(v0, v1, 16); v1 = fsl(v1, v2, 16); v2 <<= 16;
-                    uint32_t Suf[16];
-                    {
-                        uint32_t smn = 0xFFFFFFFFu;
+            for (unsigned blk = 0; blk < nblk; ++blk) {
+                lst = min(lst, rl_base + MZ_CAP * RT);   // a full list: the block's bytes overwrite slots >= MZ_CAP (never read)
+                uint32_t Suf[16];
+                {
+                    uint32_t smn = 0xFFFFFFFFu;
 #pragma unroll
-                        for (int i = 15; i >= 0; --i) { smn = min(smn, mz_val(loc, rcl, 0, i)); Suf[i] = smn; }
-                    }
-                    uint32_t A1 = 0, pw = 0;
-                    uint32_t lst = wm_base + MZ_ROW;              // where the next run's value goes
+                    for (int i = 15; i >= 0; --i) { smn = min(smn, mz_val(loc, rcl, 0, i)); Suf[i] = smn; }
+                }
+                uint32_t A1 = 0, chg = 0;
 #pragma unroll
-                    for (int tt = 0; tt < 16; ++tt) {
-                        uint32_t wm;
-                        if (tt < 4) {                              // window tt: positions tt..15, then block 1 up to index tt + 12
-                            P = min(P, mz_val(loc, rcl, 1, 12 + tt));
-                            wm = min(Suf[tt], P);
-                            if (tt == 3) { A1 = P; P = 0xFFFFFFFFu; }
-                        } else {                                   // positions tt..15, all of block 1, block 2 up to index tt - 4
-                            P = min(P, mz_val(loc, rcl, 2, tt - 4));
-                            wm = min(min(Suf[tt], A1), P);
-                        }
-                        if (tt == 0) wm_first = wm;
-                        else if (wm != pw) {                       // a new run starts at window tt
-                            sts32(lst, wm);
-                            lst += MZ_ROW;
-                            chgraw |= 1u << tt;
-                        }
-                        pw = wm;
+                for (int tt = 0; tt < 16; ++tt) {
+                    uint32_t wm;
+                    if (tt < 4) {                              // window tt: positions tt..15, then block 1 up to index tt + 12
+                        P = min(P, mz_val(loc, rcl, 1, 12 + tt));
+                        wm = min(Suf[tt], P);
+                        if (tt == 3) { A1 = P; P = 0xFFFFFFFFu; }
+                    } else {                                   // positions tt..15, all of block 1, block 2 up to index tt - 4
+                        P = min(P, mz_val(loc, rcl, 2, tt - 4));
+                        wm = min(min(Suf[tt], A1), P);
                     }
-                    P -= 16u;                                      // block 2 of this block is block 1 of the next one
-                }
-                // ---- this block's runs: 0..3 are looked up (addresses now, loads at the start of the next pass, use after
-                //      the next phase A); windows of later runs (rare) become items unfiltered
-                bool nneed0 = false;
-                uint32_t nW = 0, nchg = 0, nvm = 0, nnr = 1, nX0 = 0, nX1 = 0, nX2 = 0, nX3 = 0, nbits = 0, nbit2 = 0;
-                if (more) {
-                    uint32_t t3 = chgraw;
-                    t3 &= t3 - 1u; t3 &= t3 - 1u; t3 &= t3 - 1u;      // changes beyond the third
-                    nchg = chgraw ^ t3;
-                    const uint32_t ovfm = t3 ? (~((t3 & (0u - t3)) - 1u) & 0xFFFFu) : 0u;   // every window from the fourth change on
-                    const uint32_t vwin = __brev(vb) & 0xFFFFu;      // bit tt = validity of window tt
-                    nnr = 1u + __popc(nchg);
-                    nvm = vwin & ~ovfm;
-                    if (__any_sync(FULL, t3 != 0u)) {
-                        const unsigned long long ia = s_bw0[warp][stage] * 32ull + brel0 + (unsigned long long)seg * WMAX + blk16;
-                        uint32_t rest = t3;
-                        unsigned rr = MZ_MAXRUN;
-                        while (__any_sync(FULL, rest != 0u)) {
-                            const uint32_t low = rest & (0u - rest), nxt = rest ^ low;
-                            const uint32_t upto = nxt ? (nxt & (0u - nxt)) : 0x10000u;
-                            const uint32_t mk = rest ? ((upto - low) & vwin) : 0u;
-                            const uint32_t w = rest ? lds32(wm_base + rr * MZ_ROW) : 0u;
-                            push(mk != 0u, ia, mk, (w & 63u) | 0x8000u);     // bit 31 of the item: level 1 not looked at yet
-                            drain_if_full();
-                            rest = nxt; ++rr;
-                        }
+                    if (wm != pw) {                            // a new run starts at window tt
+                        sts8(lst, wm);
+                        lst += RT;
+                        chg |= 1u << tt;
                     }
-                    const uint32_t W1 = lds32(wm_base + 1u * MZ_ROW), W2 = lds32(wm_base + 2u * MZ_ROW), W3 = lds32(wm_base + 3u * MZ_ROW);
-                    nneed0 = !have || wm_first != held_wm;
-                    have = true;
-                    held_wm = (nnr == 1u ? wm_first : nnr == 2u ? W1 : nnr == 3u ? W2 : W3) - 16u;
-                    nW = (wm_first & 63u) | ((W1 & 63u) << 8) | ((W2 & 63u) << 16) | ((W3 & 63u) << 24);
-                    auto locate = [&](uint32_t w, unsigned sl) -> uint32_t {
-                        uint32_t ha, hb;
-                        halves_at(blk16 + (w & 63u), ha, hb);
-                        const uint32_t zlo = mz_ident_lo(ha, hb) & fmask_lo, zhi = mz_ident_hi(ha, hb);
-                        nbits |= (zlo & 31u) << (8u * sl);
-                        nbit2 |= mz_bit2(zhi) << (8u * sl);
-                        return (zlo >> 5) | ((zhi & fmask_hi) << 27);
-                    };
-                    nX0 = locate(wm_first, 0); nX1 = locate(W1, 1); nX2 = locate(W2, 2); nX3 = locate(W3, 3);
+                    pw = wm;
                 }
-                // ---- the previous block's words have had a phase A and the address work above to arrive
-                if (pend) {
-                    auto both = [&](uint32_t f, unsigned sh) -> bool {       // both bits of the identity set in its word
-                        return ((f >> ((pbits >> sh) & 31u)) & (f >> ((pbit2 >> sh) & 31u)) & 1u) != 0u;
-                    };
-                    const bool b0 = pneed0 ? both(F0, 0) : held_pass;
-                    const bool b1 = (pnr > 1u) & both(F1, 8);
-                    const bool b2 = (pnr > 2u) & both(F2, 16);
-                    const bool b3 = (pnr > 3u) & both(F3, 24);
-                    held_pass = pnr == 1u ? b0 : pnr == 2u ? b1 : pnr == 3u ? b2 : b3;
-                    // Few runs pass (0.4 % by chance, plus the true hits): in three blocks of four no lane has one, and the window
-                    // masks below are not needed at all.
-                    if (__any_sync(FULL, b0 | b1 | b2 | b3)) {
-                        // windows of run 0..3: [0, c1) [c1, c2) [c2, c3) [c3, 16); sentinels above bit 15 stand in for missing changes
-                        uint32_t cc = pchg | 0x70000u;
-                        const uint32_t c1 = cc & (0u - cc); cc ^= c1;
-                        const uint32_t c2 = cc & (0u - cc); cc ^= c2;
-                        const uint32_t c3 = cc & (0u - cc);
-                        const uint32_t m0 = (c1 - 1u) & pvm, m1 = (c2 - c1) & pvm, m2 = (c3 - c2) & pvm, m3 = (0x10000u - c3) & pvm;
-                        const bool q0 = b0 & (m0 != 0u), q1 = b1 & (m1 != 0u), q2 = b2 & (m2 != 0u), q3 = b3 & (m3 != 0u);
-                        const unsigned long long ia = s_bw0[warp][stage] * 32ull + brel0 + (unsigned long long)seg * WMAX + pblk;
-                        push(q0, ia, m0, pW & 63u);
-                        push(q1, ia, m1, (pW >> 8) & 63u);
-                        push(q2, ia, m2, (pW >> 16) & 63u);
-                        push(q3, ia, m3, pW >> 24);
-                        drain_if_full();
-                    }
-                }
-                if (!more) break;
-                pneed0 = nneed0; pW = nW; pnr = nnr; pchg = nchg; pvm = nvm; pblk = blk16; pend = true;
-                pX0 = nX0; pX1 = nX1; pX2 = nX2; pX3 = nX3; pbits = nbits; pbit2 = nbit2;
-                more = blk + 1 < (int)(WMAX / 16) && !__all_sync(FULL, (v0 | v1 | v2) == 0u);   // anything valid after this block?
+                P -= 16u;                                      // block 2 of this block is block 1 of the next one
+                pw -= 16u;                                     // (a run going on keeps its value; a position of -1 becomes 63,
+                                                               //  which no window minimum has)
+                c0 = __funnelshift_r(c0, c1, 16); c1 = __funnelshift_r(c1, c2, 16); c2 = __funnelshift_r(c2, chg, 16);
                 // slide the register windows by one word
 #pragma unroll
                 for (int k = 0; k < (int)SEGW - 1; ++k) loc[k] = loc[k + 1];
 #pragma unroll
                 for (int k = (int)SEGW - 1; k > 0; --k) rcl[k] = rcl[k - 1];
+            }
+            for (unsigned blk = nblk; blk < WMAX / 16u; ++blk) { c0 = __funnelshift_r(c0, c1, 16); c1 = __funnelshift_r(c1, c2, 16); c2 >>= 16; }
+
+            // Runs that start after the lane's last valid window have no window to look up.  Window 0 always starts a run.
+            {
+                const uint32_t lim = (uint32_t)(lastv + 1);
+                c0 &= lim >= 32u ? 0xFFFFFFFFu : (1u << lim) - 1u;
+                c1 &= lim >= 64u ? 0xFFFFFFFFu : lim > 32u ? (1u << (lim - 32u)) - 1u : 0u;
+                c2 &= lim >= 96u ? 0xFFFFFFFFu : lim > 64u ? (1u << (lim - 64u)) - 1u : 0u;
+            }
+            const uint32_t nr = (uint32_t)(__popc(c0) + __popc(c1) + __popc(c2));
+            // fw walks the run starts; c0..c2 hold the starts after it, from window fw + 1 on.  A run covers at most 29
+            // windows, so the next start is always in c0.
+            uint32_t fw = 0;
+            c0 = __funnelshift_r(c0, c1, 1); c1 = __funnelshift_r(c1, c2, 1); c2 >>= 1;
+            auto next_start = [&]() -> uint32_t {        // start of the run after the one at fw (96: none)
+                const uint32_t d = __ffs(c0);
+                c0 = __funnelshift_r(c0, c1, d); c1 = __funnelshift_r(c1, c2, d); c2 >>= d;
+                return d ? fw + d : WMAX;
+            };
+            const uint32_t V0 = __brev(v0), V1 = __brev(v1), V2 = __brev(v2);      // validity, bit w = window w
+            // lanes with `on` turn run pk (first window | end << 8 | minimizer position << 16) into items, one for every block
+            // of 16 windows the run has valid windows in; `unt`: 0x8000 for runs whose level-1 bits the drain looks at
+            auto emit = [&](bool on, uint32_t pk, uint32_t unt) {
+                const uint32_t f = pk & 127u, e = (pk >> 8) & 127u, pz = pk >> 16;
+                const unsigned long long ia = s_bw0[warp][stage] * 32ull + brel0 + (unsigned long long)seg * WMAX;
+#pragma unroll
+                for (uint32_t k = 0; k < 3u; ++k) {
+                    const uint32_t b0 = (f & ~15u) + 16u * k;                          // the block's first window
+                    const uint32_t vb = ((b0 < 32u ? V0 : b0 < 64u ? V1 : V2) >> (b0 & 16u)) & 0xFFFFu;
+                    const uint32_t lo = k == 0 ? f - b0 : 0u, hi = e < b0 + 16u ? e - b0 : 16u;
+                    const uint32_t mk = e > b0 ? (0xFFFFu << lo) & (0xFFFFu >> (16u - hi)) & vb : 0u;
+                    push(on && mk != 0u, ia + b0, mk, (pz - b0) | unt);
+                }
+            };
+
+            // Lookups: slot i of every lane's list, MZ_LGROUP slots at a time, up to the warp's longest list.
+            const uint32_t nrc = min(nr, MZ_CAP);
+            const uint32_t nmax = __reduce_max_sync(FULL, nrc);
+#pragma unroll 1
+            for (uint32_t i0 = 0; i0 < nmax; i0 += MZ_LGROUP) {
+                uint32_t Fw[MZ_LGROUP], Bt[MZ_LGROUP], Pk[MZ_LGROUP];      // the word, its two bit positions, the run
+#pragma unroll
+                for (uint32_t g = 0; g < MZ_LGROUP; ++g) {
+                    Fw[g] = 0; Bt[g] = 0; Pk[g] = 0;
+                    if (i0 + g < nmax) {
+                        const bool on = i0 + g < nrc;
+                        const uint32_t nx = next_start();
+                        const uint32_t pz = on ? (fw & ~15u) + (lds8(rl_base + (i0 + g) * RT) & 63u) : 0u;
+                        uint32_t ha, hb;
+                        halves_at(pz, ha, hb);
+                        const uint32_t zlo = mz_ident_lo(ha, hb) & fmask_lo, zhi = mz_ident_hi(ha, hb);
+                        Bt[g] = (zlo & 31u) | (mz_bit2(zhi) << 8);
+                        Fw[g] = ldg_bitmap_if(on, MB + ((zlo >> 5) | ((zhi & fmask_hi) << 27)));
+                        Pk[g] = fw | (nx << 8) | (pz << 16);
+                        my_fetch += on ? 1u : 0u;
+                        fw = nx;
+                    }
+                }
+                uint32_t pm = 0;                         // slots whose run passed (both bits set; 0.4 % by chance, plus the true hits)
+#pragma unroll
+                for (uint32_t g = 0; g < MZ_LGROUP; ++g) pm |= ((Fw[g] >> (Bt[g] & 31u)) & (Fw[g] >> (Bt[g] >> 8)) & 1u) << g;
+                while (__any_sync(FULL, pm != 0u)) {
+                    const uint32_t g = __ffs(pm) - 1u;
+                    uint32_t pk = Pk[0];
+#pragma unroll
+                    for (uint32_t h = 1; h < MZ_LGROUP; ++h) if (g == h) pk = Pk[h];
+                    emit(pm != 0u, pk, 0u);
+                    pm &= pm - 1u;
+                    drain_if_full();
+                }
+            }
+            // Runs beyond the list's capacity (only in sequence whose minimizer changes at more than every second window)
+            // go to the drain untested.  Their bytes were not kept: the minimizer of the run's first window is found again.
+            if (__any_sync(FULL, nr > MZ_CAP)) {
+#pragma unroll 1
+                for (uint32_t i = MZ_CAP; __any_sync(FULL, i < nr); ++i) {
+                    const bool on = i < nr;
+                    const uint32_t nx = next_start();
+                    uint32_t pk = 0;
+                    if (on) {
+                        uint32_t best = 0xFFFFFFFFu;
+#pragma unroll 1
+                        for (uint32_t q = 0; q + MLG_MZ_M <= K; ++q) {
+                            uint32_t ha, hb;
+                            halves_at(fw + q, ha, hb);
+                            best = min(best, (ha + hb) * MZ_M64 + q);
+                        }
+                        pk = fw | (nx << 8) | ((fw + (best & 63u)) << 16);
+                    }
+                    emit(on, pk, 0x8000u);
+                    drain_if_full();
+                    fw = nx;
+                }
             }
         }
         }
