@@ -333,6 +333,29 @@ typedef struct mlg_sketch_stats {
 int mlg_sketch_genomes(mlg_ctx* ctx, const char* text, const uint64_t* genome_off /* G+1 */, uint32_t G, uint32_t n, uint32_t K,
                        uint64_t prime, uint64_t* mins, uint32_t* counts, char* kmers, mlg_sketch_stats* stats_or_null);
 
+/* Genome files sketched straight into a builder (mlg_db_builder_create with the database's G, n, K and ks): the next
+ * nfiles genomes are the FASTA files bytes[file_off[i] .. file_off[i+1]) (host memory, pinned for a fast upload), raw as
+ * the files hold them (mlgi_files_next of include/metalign_b200_ingest.h delivers them so).  On the device each file is cut
+ * with the rules of metalign_b200/sketch.py:read_fasta -- lines split on '\n'; a line starting with '>' ends the current
+ * record; every other line, stripped of leading and trailing ASCII whitespace, is appended to it; records joined by one
+ * 'N' -- and sketched as mlg_sketch_genomes does (same passes and MLG_SKETCH_PASS_BYTES, K and n from the builder); the
+ * sketch k-mers become keys and are appended to the builder without leaving the device.  The call returns when the batch
+ * has been appended (bytes may be reused).  Refused with MLG_ERR_ARG before anything is written: null pointers, nfiles = 0,
+ * files past the builder's G genomes, prime = 1 or prime >= 2^44, a file_off that decreases anywhere, a file of about
+ * 4 GB or more, a batch of 2 GiB or more.  stats (may be null) are added to, not overwritten. */
+typedef struct mlg_fasta_stats {
+    uint64_t files, file_bytes;  /* files and raw bytes taken */
+    uint64_t text_bytes;         /* sketch text the FASTA cut made of them */
+    uint64_t n_windows, n_candidates;
+    uint32_t passes, reserved;
+    double ms_h2d;               /* CUDA-event time of the uploads */
+    double ms_cut;               /* ... of the FASTA cut (its one host round trip included) */
+    double ms_sketch;            /* ... of the sketch kernels */
+    double ms_keys;              /* host time of the key encoding and the builder's appends */
+} mlg_fasta_stats;
+int mlg_db_builder_add_fasta(mlg_db_builder* b, const void* bytes, const uint64_t* file_off /* nfiles+1 */, uint32_t nfiles,
+                             uint64_t prime, mlg_fasta_stats* stats_or_null);
+
 #ifdef __cplusplus
 }
 #endif

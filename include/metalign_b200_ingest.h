@@ -47,6 +47,19 @@ int mlgi_spilled_runs(mlgi_reader* r, uint32_t* nruns, uint64_t cap_runs);
 int mlgi_stats(mlgi_reader* r, uint64_t* reads, uint64_t* bases, uint64_t* text_bytes);
 void mlgi_close(mlgi_reader* r);
 
+/* Whole files, for the sketch builder (mlg_db_builder_add_fasta): each file of paths[] inflated whole and raw (headers and
+ * newlines kept), in the order given.  `threads` workers (<= 0: all hardware threads) inflate one file each -- BGZF members,
+ * other gzip streams with every member's CRC-32 and length checked, plain files with read(2) -- and run a few files ahead
+ * of the consumer.  A batch does not depend on the number of workers. */
+typedef struct mlgi_files mlgi_files;
+int mlgi_files_open(const char* const* paths, uint32_t nfiles, int threads, mlgi_files** out);
+/* Next batch: the next consecutive files, at most max_files of them, as many as fit in buf[0, cap); file i of the batch is
+ * buf[file_off[i], file_off[i + 1]), file_off has max_files + 1 entries.  Returns 1 with *n_files > 0, 0 at the end, -3
+ * when a file cannot be read or inflated (the message names it), 2 when the next file alone is larger than cap: nothing was
+ * taken, *need (if not null) is its size, and a call with a buffer of that size delivers it. */
+int mlgi_files_next(mlgi_files* r, uint8_t* buf, uint64_t cap, uint64_t* file_off, uint32_t max_files, uint32_t* n_files, uint64_t* need);
+void mlgi_files_close(mlgi_files* r);
+
 /* KMC k-mer databases (<prefix>.kmc_pre / .kmc_suf, both layouts) -- the artefacts scripts/select_db.py:44,50-56 of the
  * reference hands between kmc, kmc_tools and kmc_dump.  keys: total x (hi, lo) 2k-bit integers, first base most significant
  * (the key form of include/metalign_b200.h), in file order; k <= 63.  UNPINNED against files made by a real kmc. */

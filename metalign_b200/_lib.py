@@ -127,12 +127,19 @@ SIGNATURES = {
     "mlg_kmc_concat": (C.c_int, [C.c_char_p, C.POINTER(C.c_char_p), C.c_uint32]),
     "mlg_query_free": (C.c_int, [_vp]),
     "mlg_sketch_genomes": (C.c_int, [_vp, _vp, _u64p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint64, _u64p, _u32p, _vp, _vp]),
+    "mlg_db_builder_add_fasta": (C.c_int, [_vp, _vp, _u64p, C.c_uint32, C.c_uint64, _vp]),
 }
 
 
 class SketchStats(C.Structure):
     _fields_ = [("n_windows", C.c_uint64), ("n_candidates", C.c_uint64), ("ms_kernels", C.c_double), ("passes", C.c_uint32),
                 ("reserved", C.c_uint32)]
+
+
+class FastaStats(C.Structure):
+    _fields_ = [("files", C.c_uint64), ("file_bytes", C.c_uint64), ("text_bytes", C.c_uint64), ("n_windows", C.c_uint64),
+                ("n_candidates", C.c_uint64), ("passes", C.c_uint32), ("reserved", C.c_uint32), ("ms_h2d", C.c_double),
+                ("ms_cut", C.c_double), ("ms_sketch", C.c_double), ("ms_keys", C.c_double)]
 
 
 def lib():

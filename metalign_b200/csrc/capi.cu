@@ -330,6 +330,10 @@ MLG_API int mlg_db_builder_create(mlg_ctx* ctx, uint32_t G, uint32_t n, uint32_t
 MLG_API int mlg_db_builder_add_device(mlg_db_builder* b, const uint64_t* d_keys, uint32_t first_genome, uint32_t n_genomes) {
     return mlg_db_builder_add_impl(b, reinterpret_cast<const key128*>(d_keys), first_genome, n_genomes);
 }
+MLG_API int mlg_db_builder_add_fasta(mlg_db_builder* b, const void* bytes, const uint64_t* file_off, uint32_t nfiles, uint64_t prime,
+                                     mlg_fasta_stats* stats_or_null) {
+    return mlg_db_builder_add_fasta_impl(b, bytes, file_off, nfiles, prime, stats_or_null);
+}
 MLG_API int mlg_db_builder_finish(mlg_db_builder* b, mlg_db** out) { return mlg_db_builder_finish_impl(b, out); }
 MLG_API int mlg_db_builder_destroy(mlg_db_builder* b) { mlg_db_builder_destroy_impl(b); return MLG_OK; }
 

@@ -429,6 +429,10 @@ int mlg_db_builder_add_impl(mlg_db_builder* b, const key128* d_keys, uint32_t g0
     return MLG_OK;
 }
 
+void mlg_db_builder_shape(const mlg_db_builder* b, mlg_ctx** ctx, uint32_t* G, uint32_t* n, uint32_t* K, uint32_t* next_g) {
+    *ctx = b->ctx; *G = b->G; *n = b->n; *K = b->K; *next_g = b->next_g;
+}
+
 void mlg_db_builder_destroy_impl(mlg_db_builder* b) {
     if (!b) return;
     cudaSetDevice(b->ctx->device);

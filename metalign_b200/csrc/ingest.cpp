@@ -266,6 +266,34 @@ struct mlgi_reader {
         }
         return false;
     }
+    // inflates the members in base[in0, in1) (found by bgzf_member) into dst, which has room for the sum of their sizes;
+    // false on a member that does not inflate to its stated size and CRC-32
+    static bool bgzf_inflate(const unsigned char* base, size_t n, size_t in0, size_t in1, char* dst, size_t* out_n) {
+        size_t o = 0;
+        for (size_t q = in0; q < in1;) {
+            size_t cs = 0, hd = 0;
+            bgzf_member(base + q, n - q, &cs, &hd);
+            const unsigned char* t = base + q + cs - 4;
+            const size_t isz = (size_t)t[0] | ((size_t)t[1] << 8) | ((size_t)t[2] << 16) | ((size_t)t[3] << 24);
+            z_stream zs;
+            memset(&zs, 0, sizeof(zs));
+            if (inflateInit2(&zs, -15) != Z_OK) return false;
+            zs.next_in = const_cast<unsigned char*>(base + q + hd); zs.avail_in = (uInt)(cs - hd - 8);
+            zs.next_out = (unsigned char*)dst + o; zs.avail_out = (uInt)isz;
+            const int rc = inflate(&zs, Z_FINISH);
+            bool good = rc == Z_STREAM_END && zs.total_out == isz;
+            inflateEnd(&zs);
+            if (good) {
+                const unsigned char* c = t - 4;
+                const unsigned long want = (unsigned long)c[0] | ((unsigned long)c[1] << 8) | ((unsigned long)c[2] << 16) | ((unsigned long)c[3] << 24);
+                good = crc32(crc32(0L, Z_NULL, 0), (const Bytef*)dst + o, (uInt)isz) == want;
+            }
+            if (!good) return false;
+            o += isz; q += cs;
+        }
+        *out_n = o;
+        return true;
+    }
     void read_loop_bgzf() {
         const unsigned char* base = (const unsigned char*)gzmap->p;
         const size_t n = gzmap->n;
@@ -290,30 +318,7 @@ struct mlgi_reader {
             auto inflate_job = [&](Job& j) {
                 j.buf = std::make_shared<TextBuf>();
                 j.buf->mem.reset(new char[HEAD + j.out + 1]);
-                char* dst = j.buf->mem.get() + HEAD;
-                size_t o = 0;
-                for (size_t q = j.in0; q < j.in1;) {
-                    size_t cs = 0, hd = 0;
-                    bgzf_member(base + q, n - q, &cs, &hd);
-                    const unsigned char* t = base + q + cs - 4;
-                    const size_t isz = (size_t)t[0] | ((size_t)t[1] << 8) | ((size_t)t[2] << 16) | ((size_t)t[3] << 24);
-                    z_stream zs;
-                    memset(&zs, 0, sizeof(zs));
-                    if (inflateInit2(&zs, -15) != Z_OK) { j.ok = false; return; }
-                    zs.next_in = const_cast<unsigned char*>(base + q + hd); zs.avail_in = (uInt)(cs - hd - 8);
-                    zs.next_out = (unsigned char*)dst + o; zs.avail_out = (uInt)isz;
-                    const int rc = inflate(&zs, Z_FINISH);
-                    bool good = rc == Z_STREAM_END && zs.total_out == isz;
-                    inflateEnd(&zs);
-                    if (good) {
-                        const unsigned char* c = t - 4;
-                        const unsigned long want = (unsigned long)c[0] | ((unsigned long)c[1] << 8) | ((unsigned long)c[2] << 16) | ((unsigned long)c[3] << 24);
-                        good = crc32(crc32(0L, Z_NULL, 0), (const Bytef*)dst + o, (uInt)isz) == want;
-                    }
-                    if (!good) { j.ok = false; return; }
-                    o += isz; q += cs;
-                }
-                j.buf->n = o;
+                j.ok = bgzf_inflate(base, n, j.in0, j.in1, j.buf->mem.get() + HEAD, &j.buf->n);
             };
             std::vector<std::thread> th;
             for (size_t i = 1; i < jobs.size(); ++i) th.emplace_back([&, i] { inflate_job(jobs[i]); });
@@ -644,11 +649,172 @@ void pack_range(PackJob& j) {
     }
 }
 
+// ---- whole files (mlgi_files_*): genome files for the sketch builder ----------------------------------------------------
+// One file, inflated whole into a fresh buffer: BGZF members through bgzf_inflate, any other gzip through fast_inflate.h
+// (every member's CRC-32 and length checked), a plain file through read(2).  Returns "" or what went wrong.
+std::string inflate_whole_file(const char* path, std::unique_ptr<char[]>& out, size_t* out_n) {
+    const int fd = open(path, O_RDONLY);
+    if (fd < 0) return std::string("cannot open: ") + strerror(errno);
+    struct Closer { int fd; ~Closer() { close(fd); } } closer{fd};
+    struct stat sb;
+    if (fstat(fd, &sb) != 0) return std::string("fstat failed: ") + strerror(errno);
+    const size_t size = (size_t)sb.st_size;
+    unsigned char magic[2] = {0, 0};
+    if (size < 2 || pread(fd, magic, 2, 0) != 2 || magic[0] != 0x1f || magic[1] != 0x8b) {
+        out.reset(new char[size + 1]);
+        size_t got = 0;
+        while (got < size) {
+            const ssize_t k = read(fd, out.get() + got, size - got);
+            if (k < 0) return std::string("read failed: ") + strerror(errno);
+            if (k == 0) return "file shrank while it was read";
+            got += (size_t)k;
+        }
+        *out_n = size;
+        return "";
+    }
+    Mapping m;
+    m.p = mmap(nullptr, size, PROT_READ, MAP_PRIVATE, fd, 0);
+    if (m.p == MAP_FAILED) { m.p = nullptr; return std::string("mmap failed: ") + strerror(errno); }
+    m.n = size;
+    const unsigned char* base = (const unsigned char*)m.p;
+    size_t cs = 0, hd = 0;
+    if (mlgi_reader::bgzf_member(base, size, &cs, &hd)) {
+        size_t total = 0;
+        for (size_t q = 0; q < size; q += cs) {
+            if (!mlgi_reader::bgzf_member(base + q, size - q, &cs, &hd)) return "truncated or corrupt BGZF file";
+            const unsigned char* t = base + q + cs - 4;
+            total += (size_t)t[0] | ((size_t)t[1] << 8) | ((size_t)t[2] << 16) | ((size_t)t[3] << 24);
+        }
+        out.reset(new char[total + 1]);
+        if (!mlgi_reader::bgzf_inflate(base, size, 0, size, out.get(), out_n)) return "corrupt BGZF member (CRC or length mismatch)";
+        return "";
+    }
+    // the output buffer grows as needed; the trailer's ISIZE (the last member's length mod 2^32) is the first guess
+    const uint32_t isize_hint = size < 4 ? 0u : (uint32_t)base[size - 4] | ((uint32_t)base[size - 3] << 8) | ((uint32_t)base[size - 2] << 16) |
+                                                ((uint32_t)base[size - 1] << 24);
+    size_t cap = std::max<size_t>({(size_t)isize_hint + 64, size * 4, (size_t)1 << 16});
+    std::unique_ptr<uint8_t[]> buf(new uint8_t[cap + fastinf::SLACK]);
+    std::unique_ptr<fastinf::Inflater> z(new fastinf::Inflater());
+    z->in = base; z->in_end = base + size;
+    size_t produced = 0, member = 0;
+    for (;;) {
+        uint8_t* o = buf.get() + produced;
+        const int rc = z->run(o, buf.get() + cap, buf.get());
+        produced = (size_t)(o - buf.get());
+        if (rc < 0) return std::string("corrupt or truncated gzip stream: ") + (z->error ? z->error : "?");
+        if (rc == 2) break;
+        if (rc == 1) {
+            if ((uint32_t)(produced - member) != z->isize_expected) return "gzip length mismatch";
+            if ((uint32_t)crc32(crc32(0L, Z_NULL, 0), buf.get() + member, (uInt)(produced - member)) != z->crc_expected) return "gzip CRC mismatch";
+            member = produced;
+            continue;
+        }
+        cap *= 2;                                        // rc == 0: the buffer is full
+        std::unique_ptr<uint8_t[]> bigger(new uint8_t[cap + fastinf::SLACK]);
+        memcpy(bigger.get(), buf.get(), produced);
+        buf.swap(bigger);
+    }
+    out.reset(reinterpret_cast<char*>(buf.release()));
+    *out_n = produced;
+    return "";
+}
+
 }  // namespace
+
+// Workers take the files in order, one file each, and run at most `ahead` files past the one the consumer waits for;
+// mlgi_files_next hands them over strictly in order, so a batch does not depend on the number of workers or their timing.
+struct mlgi_files {
+    struct Slot { std::unique_ptr<char[]> buf; size_t n = 0; std::string err; bool ready = false; };
+    std::vector<std::string> paths;
+    std::vector<Slot> slots;
+    std::mutex mu;
+    std::condition_variable cv_ready, cv_room;
+    size_t next_job = 0, consumed = 0, ahead = 4;
+    bool stop = false;
+    std::vector<std::thread> workers;
+
+    void work() {
+        for (;;) {
+            size_t i;
+            {
+                std::unique_lock<std::mutex> g(mu);
+                cv_room.wait(g, [&] { return stop || next_job >= paths.size() || next_job < consumed + ahead; });
+                if (stop || next_job >= paths.size()) return;
+                i = next_job++;
+            }
+            Slot s;
+            s.err = inflate_whole_file(paths[i].c_str(), s.buf, &s.n);
+            if (!s.err.empty()) s.buf.reset();
+            s.ready = true;
+            std::lock_guard<std::mutex> g(mu);
+            slots[i] = std::move(s);
+            cv_ready.notify_all();
+        }
+    }
+};
 
 extern "C" {
 
 MLGI_API const char* mlgi_last_error(void) { return g_err; }
+
+MLGI_API int mlgi_files_open(const char* const* paths, uint32_t nfiles, int threads, mlgi_files** out) {
+    if ((!paths && nfiles) || !out) { set_error("null argument"); return -2; }
+    for (uint32_t i = 0; i < nfiles; ++i) if (!paths[i]) { set_error("null path %u", i); return -2; }
+    std::unique_ptr<mlgi_files> r(new mlgi_files());
+    r->paths.assign(paths, paths + nfiles);
+    r->slots.resize(nfiles);
+    int hw = (int)std::thread::hardware_concurrency();
+    if (hw < 1) hw = 1;
+    const int T = std::max(1, std::min<int>(threads > 0 ? threads : hw, (int)std::max<uint32_t>(nfiles, 1u)));
+    r->ahead = (size_t)std::max(4, 4 * T);
+    for (int t = 0; t < T; ++t) r->workers.emplace_back([p = r.get()] { p->work(); });
+    *out = r.release();
+    return 0;
+}
+
+MLGI_API int mlgi_files_next(mlgi_files* r, uint8_t* buf, uint64_t cap, uint64_t* file_off, uint32_t max_files, uint32_t* n_files,
+                             uint64_t* need) {
+    if (!r || !buf || !file_off || !n_files || max_files == 0) { set_error("null argument or max_files = 0"); return -2; }
+    *n_files = 0;
+    if (need) *need = 0;
+    file_off[0] = 0;
+    uint64_t pos = 0;
+    uint32_t k = 0;
+    while (k < max_files) {
+        std::unique_lock<std::mutex> g(r->mu);
+        if (r->consumed >= r->paths.size()) break;
+        mlgi_files::Slot& s = r->slots[r->consumed];
+        r->cv_ready.wait(g, [&] { return s.ready; });
+        if (!s.err.empty()) { set_error("%s: %s", r->paths[r->consumed].c_str(), s.err.c_str()); return -3; }
+        if (pos + s.n > cap) {
+            if (k) break;
+            if (need) *need = s.n;           // a file larger than the buffer comes alone, in a buffer of its size
+            set_error("%s: %llu bytes do not fit a buffer of %llu", r->paths[r->consumed].c_str(), (unsigned long long)s.n, (unsigned long long)cap);
+            return 2;
+        }
+        std::unique_ptr<char[]> mem = std::move(s.buf);
+        const size_t m = s.n;
+        ++r->consumed;
+        r->cv_room.notify_all();
+        g.unlock();
+        if (m) memcpy(buf + pos, mem.get(), m);
+        pos += m;
+        file_off[++k] = pos;
+    }
+    *n_files = k;
+    return k ? 1 : 0;
+}
+
+MLGI_API void mlgi_files_close(mlgi_files* r) {
+    if (!r) return;
+    {
+        std::lock_guard<std::mutex> g(r->mu);
+        r->stop = true;
+    }
+    r->cv_room.notify_all();
+    for (auto& t : r->workers) t.join();
+    delete r;
+}
 
 MLGI_API int mlgi_open(const char* path, int input_type, int threads, mlgi_reader** out) {
     if (!path || !out) { set_error("null argument"); return -2; }

@@ -131,6 +131,10 @@ int mlg_db_builder_create_impl(mlg_ctx* ctx, uint32_t G, uint32_t n, uint32_t K,
 int mlg_db_builder_add_impl(mlg_db_builder* b, const key128* d_keys, uint32_t g0, uint32_t count);
 int mlg_db_builder_finish_impl(mlg_db_builder* b, mlg_db** out);      // frees the builder on success
 void mlg_db_builder_destroy_impl(mlg_db_builder* b);
+void mlg_db_builder_shape(const mlg_db_builder* b, mlg_ctx** ctx, uint32_t* G, uint32_t* n, uint32_t* K, uint32_t* next_g);
+// genome files sketched on the device and appended to the builder (sketch.cu)
+int mlg_db_builder_add_fasta_impl(mlg_db_builder* b, const void* bytes, const uint64_t* file_off, uint32_t nfiles, uint64_t prime,
+                                  mlg_fasta_stats* st);
 // .mlgdb files (dbfile.cu): version 1 = source keys (built on load), version 2 = the built structures
 int mlg_db_load_file(mlg_ctx* ctx, const char* path, mlg_db** out);
 int mlg_db_save_file(const mlg_db* db, const char* path, const char* names, uint64_t names_bytes);

@@ -51,8 +51,68 @@ def ingest_lib():
         L.mlgi_stats.argtypes = [C.c_void_p] + [C.POINTER(C.c_uint64)] * 3
         L.mlgi_close.argtypes = [C.c_void_p]
         L.mlgi_close.restype = None
+        L.mlgi_files_open.argtypes = [C.POINTER(C.c_char_p), C.c_uint32, C.c_int, C.POINTER(C.c_void_p)]
+        L.mlgi_files_next.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32),
+                                      C.POINTER(C.c_uint64)]
+        L.mlgi_files_close.argtypes = [C.c_void_p]
+        L.mlgi_files_close.restype = None
         _INGEST = L
     return _INGEST
+
+
+class FileBatches:
+    """Whole files (gzip, BGZF or plain), inflated by `threads` workers of the native reader (mlgi_files_*) and handed
+    over in the order given, as batches of consecutive files.  next_batch() fills one of two alternating buffers of
+    batch_bytes (`alloc(nbytes) -> uint8 ndarray`: pinned memory from api.pinned_array for the GPU), so one batch can be
+    read while the other is in use; a file larger than batch_bytes comes alone, in a buffer of its own size."""
+
+    def __init__(self, paths, batch_bytes: int = 1 << 30, threads: int = 0, max_files: int = 1 << 16, alloc=None):
+        self.L = ingest_lib()
+        self.h = C.c_void_p()
+        self._paths = (C.c_char_p * max(1, len(paths)))(*[os.fsencode(p) for p in paths])
+        if self.L.mlgi_files_open(self._paths, len(paths), int(threads), C.byref(self.h)) != 0:
+            raise IOError(self.L.mlgi_last_error().decode())
+        self.alloc = alloc or (lambda nbytes: np.empty(nbytes, dtype=np.uint8))
+        self.max_files = int(max_files)
+        self.bufs = [self.alloc(int(batch_bytes)), self.alloc(int(batch_bytes))]
+        self.offs = [np.zeros(self.max_files + 1, dtype=np.uint64) for _ in range(2)]
+        self.cur = 0
+
+    def next_batch(self):
+        """-> (buf uint8 ndarray, file_off uint64[n+1]) of the next batch, or None at the end"""
+        k = self.cur
+        self.cur ^= 1
+        n, need = C.c_uint32(), C.c_uint64()
+        while True:
+            b, o = self.bufs[k], self.offs[k]
+            rc = self.L.mlgi_files_next(self.h, b.ctypes.data, b.size, o.ctypes.data, self.max_files, C.byref(n), C.byref(need))
+            if rc != 2:
+                break
+            self.bufs[k] = None
+            self.bufs[k] = self.alloc(int(need.value))
+        if rc < 0:
+            raise IOError(self.L.mlgi_last_error().decode())
+        if rc == 0:
+            return None
+        return b, o[:n.value + 1]
+
+    def __iter__(self):
+        while True:
+            r = self.next_batch()
+            if r is None:
+                return
+            yield r
+
+    def close(self):
+        if self.h:
+            self.L.mlgi_files_close(self.h)
+            self.h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:  # noqa: BLE001
+            pass
 
 
 class PackedBatches:

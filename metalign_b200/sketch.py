@@ -1,12 +1,13 @@
 """Sketch builder: the GPU replacement of CMash's `MakeStreamingDNADatabase.py <list> <out.h5> -n 1000 -k 60`
 (local_tests/retrain_and_test_metalign.sh:49 of the reference) for this repo's database format.
 
-    python scripts/make_sketch_db.py genomes.txt out.mlgdb [-n 1000] [-k 60] [--k_range 30-60-10]
+    python scripts/make_sketch_db.py genomes.txt out.mlgdb [-n 1000] [-k 60] [--k_range 30-60-10] [--built [--threads T]]
 
 `genomes.txt` lists one FASTA path per line (plain or .gz), as the reference's training list does.  Each genome's
 bottom-n MinHash sketch (forward strand, MurmurHash3 mod prime: include/metalign_b200.h, mlg_sketch_genomes) is computed
 on the GPU; genomes are stored in sorted-basename order, the order in which CMash's import_multiple_from_single_hdf5
 hands them to dump_kmers.py:7-14 and StreamingQueryDNADatabase.py, so genome indices mean the same thing.
+--built writes the built form (what scripts/build_db.py makes of the source form) in one go: build_database_from_files.
 No CPU fallback: without the CUDA library and a GPU every call raises.
 """
 from __future__ import annotations
@@ -89,6 +90,73 @@ def build_database(ctx, paths: Iterable[str], out_path: str, n: int = 1000, K: i
     return tot
 
 
+def build_database_from_files(ctx, paths: Iterable[str], out_path: str, n: int = 1000, K: int = 60, ks: Sequence[int] = (30, 40, 50, 60),
+                              threads: int = 0, batch_bytes: int = 64 << 20, prime: int = 0, log=None):
+    """Sketch every genome file into the BUILT .mlgdb (the form Database.load reads without a rebuild), the genomes in
+    sorted-basename order as build_database stores them; the same file build_database -> Database.load -> save writes.
+    The host only inflates: the native reader (ingest.FileBatches, `threads` workers) fills pinned batches of about
+    batch_bytes of raw file bytes, the next batch while the GPU cuts and sketches the current one
+    (mlg_db_builder_add_fasta), and the keys go to the builder on the device.  (The two pinned buffers cost about
+    0.7 ms per MiB to page-lock, which is why batches are 64 MiB: the GPU's share of one is a few milliseconds.)  Nothing is left at out_path when any
+    step fails, e.g. a database whose hit records do not fit beside its other structures (no built form exists for it).
+    Returns the stats: the library's stage times plus seconds spent waiting for the reader, in finish and in save."""
+    import concurrent.futures
+    import time
+    from .api import Database, pinned_array
+    from .ingest import FileBatches
+    paths = sorted(paths, key=os.path.basename)
+    names = [os.path.basename(p) for p in paths]
+    G = len(paths)
+    ksa = np.asarray(ks, dtype=np.uint32)
+    L = _lib.lib()
+    st = _lib.FastaStats()
+    b = C.c_void_p()
+    check(L.mlg_db_builder_create(ctx._h, G, n, K, ksa.ctypes.data, ksa.size, C.byref(b)))
+    h = C.c_void_p()
+    s_read = 0.0
+    reader = None
+    try:
+        reader = FileBatches(paths, batch_bytes=batch_bytes, threads=threads, alloc=pinned_array)
+        with concurrent.futures.ThreadPoolExecutor(1) as ex:
+            nxt = ex.submit(reader.next_batch)
+            done = 0
+            while True:
+                t0 = time.perf_counter()
+                batch = nxt.result()
+                s_read += time.perf_counter() - t0
+                if batch is None:
+                    break
+                buf, off = batch
+                nxt = ex.submit(reader.next_batch)       # the other buffer: read while this batch is on the GPU
+                check(L.mlg_db_builder_add_fasta(b, buf.ctypes.data, off.ctypes.data, off.size - 1, prime, C.byref(st)))
+                done += off.size - 1
+                if log:
+                    log("sketched %d / %d genomes" % (done, G))
+        t0 = time.perf_counter()
+        check(L.mlg_db_builder_finish(b, C.byref(h)))
+        s_finish = time.perf_counter() - t0
+    except BaseException:
+        L.mlg_db_builder_destroy(b)
+        raise
+    finally:
+        if reader is not None:
+            reader.close()
+    db = Database(ctx, h, names)
+    try:
+        t0 = time.perf_counter()
+        db.save(out_path)
+        s_save = time.perf_counter() - t0
+    except BaseException:
+        if os.path.exists(out_path):
+            os.remove(out_path)
+        raise
+    finally:
+        db.close()
+    out = {f: getattr(st, f) for f, _ in st._fields_ if f != "reserved"}
+    out.update(s_read_wait=s_read, s_finish=s_finish, s_save=s_save)
+    return out
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description="GPU sketch builder (CMash MakeStreamingDNADatabase.py equivalent) -> .mlgdb")
     ap.add_argument("in_file", help="text file with one genome FASTA path (plain or .gz) per line")
@@ -97,6 +165,9 @@ def main(argv=None):
     ap.add_argument("-k", "--k_size", type=int, default=60)
     ap.add_argument("--k_range", default="30-60-10", help="prefix lengths the database will be queried at")
     ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--built", action="store_true",
+                    help="write the built form (what scripts/build_db.py makes of the source form) straight from the files")
+    ap.add_argument("--threads", type=int, default=0, help="--built: reader threads inflating the files (0 = all cores)")
     a = ap.parse_args(argv)
     # what the database loader accepts (1 <= K <= 63, 1..8 ascending ks within 1..K), checked before any genome is read
     if not 1 <= a.k_size <= 63:
@@ -113,8 +184,14 @@ def main(argv=None):
     with open(a.in_file) as f:
         paths = [ln.strip() for ln in f if ln.strip()]
     from .api import Context
+    log = lambda m: print(m, file=sys.stderr)  # noqa: E731
     with Context(a.device) as ctx:
-        st = build_database(ctx, paths, a.out_file, a.num_hashes, a.k_size, ks, log=lambda m: print(m, file=sys.stderr))
+        if a.built:
+            st = build_database_from_files(ctx, paths, a.out_file, a.num_hashes, a.k_size, ks, threads=a.threads, log=log)
+            print("wrote %s (built form): %d genomes x %d slots, K=%d, ks=%s; %.2f GB of files, %d windows hashed in %.1f ms of kernels"
+                  % (a.out_file, len(paths), a.num_hashes, a.k_size, ks, st["file_bytes"] / 1e9, st["n_windows"], st["ms_sketch"]))
+            return
+        st = build_database(ctx, paths, a.out_file, a.num_hashes, a.k_size, ks, log=log)
     print("wrote %s: %d genomes x %d slots, K=%d, ks=%s; %d windows hashed in %.1f ms of kernels"
           % (a.out_file, len(paths), a.num_hashes, a.k_size, ks, st["n_windows"], st["ms_kernels"]))
 
