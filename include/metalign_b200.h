@@ -167,8 +167,14 @@ int mlg_query_counts_merge_sparse(mlg_query* q, const uint64_t* d_entries, uint6
  * If some rank had more than cap_entries non-zero counters, nothing is merged on any rank and mlg_query_finish()
  * returns MLG_ERR_RETRY: repeat the exchange with a larger mlg_exchange and call finish again.  Every rank judges all
  * world counts, its own included, so every rank gets the same answer, and the error message names the largest count.
- * Every form leaves the same counters on every rank: the sum over ranks of min(count, ci_min).  The pack calls
- * (mlg_query_counts_export*, mlg_query_exchange_pack / _p2p / _dense) clamp the rank's own counters to ci_min in place. */
+ * Every form leaves the same counters on every rank: the sum over ranks of min(count, clamp), clamp = ci_min unless
+ * mlg_query_set_exchange_clamp() set another level.  The pack calls (mlg_query_counts_export*, mlg_query_exchange_pack /
+ * _p2p / _dense) clamp the rank's own counters to it in place. */
+/* The clamp level of the rank's own counters before any of these exchanges: ci_min (the default) .. 255, set before the
+ * first exchange call (MLG_ERR_STATE after it).  Presence (a summed counter >= ci_min) does not depend on it, but the counts
+ * that mlg_query_dump_intersection / mlg_query_write_intersection_kmc write are min(sum, multiplicity, counter_max): with a
+ * clamp >= counter_max they equal the counts of one query over all the reads.  clamp * world must fit the 8-bit counters. */
+int mlg_query_set_exchange_clamp(mlg_query* q, int clamp);
 int mlg_exchange_create(mlg_ctx* ctx, uint32_t world, uint32_t rank, uint64_t cap_entries, mlg_exchange** out);
 int mlg_exchange_destroy(mlg_exchange* ex);
 int mlg_exchange_buffers(mlg_exchange* ex, uint64_t** d_send, uint64_t** d_recv, uint64_t* block_words);

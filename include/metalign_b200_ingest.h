@@ -43,6 +43,22 @@ int mlgi_open(const char* path, int input_type, int threads, mlgi_reader** out);
 int mlgi_next(mlgi_reader* r, uint8_t* bases, uint64_t cap_bases_bytes, uint32_t* nruns, uint64_t cap_runs, uint64_t* off,
               uint64_t max_reads, uint64_t max_bases, uint64_t* n_reads, uint64_t* n_runs);
 int mlgi_spilled_runs(mlgi_reader* r, uint32_t* nruns, uint64_t cap_runs);
+/* A share of a reads file for one of several readers (one per GPU): like mlgi_open, but only the records of the byte range
+ * [begin, end) of the file on disk.  A line belongs to the share that holds its first byte and is read to its end.
+ *   plain file   the range is a range of the file's bytes
+ *   BGZF         the share takes the members whose compressed start is in the range, and the lines that start in their
+ *                text (inflating the following members as far as its last line runs)
+ *   other gzip   one DEFLATE stream cannot be split: the share with begin = 0 reads the whole file (and says so on stderr
+ *                when end is before the end of the file), every other share is empty
+ * FASTA shares start at the first line start in the range.  A FASTQ share also needs the line number mod 4 of its first
+ * line: it takes the first line that starts with '@' and whose line two after starts with '+' (exact for 4-line FASTQ).
+ * Shares of consecutive ranges that cover the file deliver, joined in order, the reads of mlgi_open -- if every share's
+ * phase equals the sum of the earlier shares' newline counts mod 4 (mlgi_share_info); otherwise the file is not 4-line
+ * FASTQ and must be read whole. */
+int mlgi_open_share(const char* path, int input_type, int threads, uint64_t begin, uint64_t end, mlgi_reader** out);
+/* after mlgi_next returned 0: text offset of the share's first line, its number of '\n', and the phase it took (-1: the
+ * share is empty, -2: no record start near it) */
+int mlgi_share_info(mlgi_reader* r, uint64_t* first, uint64_t* newlines, int* phase);
 /* totals so far: reads and bases delivered, compressed/raw bytes consumed from the file */
 int mlgi_stats(mlgi_reader* r, uint64_t* reads, uint64_t* bases, uint64_t* text_bytes);
 void mlgi_close(mlgi_reader* r);

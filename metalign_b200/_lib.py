@@ -109,6 +109,7 @@ SIGNATURES = {
     "mlg_query_exchange_merge": (C.c_int, [_vp, _vp]),
     "mlg_query_exchange_p2p": (C.c_int, [_vp, _vp]),
     "mlg_query_exchange_dense": (C.c_int, [_vp, _pp, C.POINTER(C.c_uint64)]),
+    "mlg_query_set_exchange_clamp": (C.c_int, [_vp, C.c_int]),
     "mlg_query_finish": (C.c_int, [_vp, _i64p, _i64p, _f64p, C.POINTER(C.c_uint64)]),
     "mlg_query_finish_sparse": (C.c_int, [_vp, _u32p, _i64p, _i64p, _f64p, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "mlg_query_hit_flags": (C.c_int, [_vp, _u32p, C.c_uint32, _u8p]),

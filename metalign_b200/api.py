@@ -185,6 +185,7 @@ class Query:
     def __init__(self, db: Database, ci_min: int = 2, gate: str = "exact", count_empty_in_den: bool = True):
         self.db = db
         self.ci_min = int(ci_min)
+        self.exchange_clamp = self.ci_min
         self._h = C.c_void_p()
         check(_lib.lib().mlg_query_begin(db.ctx._h, db._h, int(ci_min), GATE[gate], int(count_empty_in_den),
                                          C.byref(self._h)))
@@ -261,6 +262,12 @@ class Query:
         check(_lib.lib().mlg_query_counts_import(self._h))
 
     # -- multi-GPU exchange without a host round trip (see metalign_b200.dist) -------------------------------
+    def set_exchange_clamp(self, clamp: int):
+        """clamp this rank's counters to `clamp` (ci_min .. 255; default ci_min) before the exchange, so that the summed
+        counters give the single-query intersection counts up to `clamp` (the drop-in sets counter_max); before any exchange"""
+        check(_lib.lib().mlg_query_set_exchange_clamp(self._h, int(clamp)))
+        self.exchange_clamp = int(clamp)
+
     def exchange_pack(self, ex: "Exchange"):
         check(_lib.lib().mlg_query_exchange_pack(self._h, ex._h))
 

@@ -130,6 +130,7 @@ struct mlg_query {
     mlg_ctx* ctx = nullptr;
     mlg_db* db = nullptr;
     int ci_min = 2, gate = MLG_GATE_EXACT, count_empty = 1;
+    int ex_clamp = 2;                              // a rank's counters are clamped to this before an exchange (>= ci_min)
     DevBuf<unsigned char> cnt8;
     DevBuf<unsigned long long> d_nkmers, d_scalar;
     Staging stg[2];
@@ -419,7 +420,7 @@ MLG_API int mlg_query_begin(mlg_ctx* ctx, mlg_db* db, int ci_min, int gate_mode,
     MLG_TRY(ensure_device(ctx));
     mlg_query* q = new mlg_query();
     struct Guard { mlg_query* q; ~Guard() { if (q) mlg_query_free(q); } } guard{q};
-    q->ctx = ctx; q->db = db; q->ci_min = ci_min; q->gate = gate_mode; q->count_empty = count_empty_in_den ? 1 : 0;
+    q->ctx = ctx; q->db = db; q->ci_min = ci_min; q->ex_clamp = ci_min; q->gate = gate_mode; q->count_empty = count_empty_in_den ? 1 : 0;
     size_t cbytes = round_up((size_t)db->v.nd + 4, 16);
     if (db->clean_cnt8.p && db->clean_cnt8.n >= cbytes) {        // left all-zero by the query before (mlg_query_free)
         std::swap(q->cnt8.p, db->clean_cnt8.p); std::swap(q->cnt8.n, db->clean_cnt8.n);
@@ -593,7 +594,7 @@ MLG_API int mlg_query_counts_export(mlg_query* q, uint8_t** d_counts, uint64_t* 
     MLG_TRY(ensure_device(q->ctx));
     q->exchanged = true;
     if (q->touched.p) {     // nothing pushed: every counter is still zero
-        MLG_TRY(launch_clamp_counts(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ci_min, q->ctx->s_comp));
+        MLG_TRY(launch_clamp_counts(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ex_clamp, q->ctx->s_comp));
         q->st.gpu_launches += 1;
     }
     MLG_TRY(mlg_query_sync(q));
@@ -614,7 +615,7 @@ MLG_API int mlg_query_counts_export_sparse(mlg_query* q, uint64_t** d_entries, u
     CUDA_TRY(cudaMemcpyAsync(&nt, q->d_scalar.p + 1, 8, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));                   // joins the probe kernels
     MLG_TRY(q->sparse.ensure(nt));
-    MLG_TRY(launch_pack_touched(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ci_min, q->sparse.p, st));
+    MLG_TRY(launch_pack_touched(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ex_clamp, q->sparse.p, st));
     q->st.gpu_launches += 1;
     CUDA_TRY(cudaStreamSynchronize(st));
     *d_entries = reinterpret_cast<uint64_t*>(q->sparse.p); *n_entries = nt;
@@ -637,6 +638,14 @@ MLG_API int mlg_query_counts_merge_sparse(mlg_query* q, const uint64_t* d_entrie
 MLG_API int mlg_query_counts_import(mlg_query* q) {
     if (!q) { mlg_set_error("null query"); return MLG_ERR_ARG; }
     q->reduced = true; q->exchanged = true;
+    return MLG_OK;
+}
+
+MLG_API int mlg_query_set_exchange_clamp(mlg_query* q, int clamp) {
+    if (!q) { mlg_set_error("null query"); return MLG_ERR_ARG; }
+    if (q->exchanged || q->finished) { mlg_set_error("the exchange clamp must be set before any exchange"); return MLG_ERR_STATE; }
+    if (clamp < q->ci_min || clamp > 255) { mlg_set_error("exchange clamp %d out of range ci_min (%d)..255", clamp, q->ci_min); return MLG_ERR_ARG; }
+    q->ex_clamp = clamp;
     return MLG_OK;
 }
 
@@ -708,7 +717,7 @@ static int check_exchange(mlg_query* q, mlg_exchange* ex) {
     if (q->finished) { mlg_set_error("query already finished"); return MLG_ERR_STATE; }
     if (q->reduced) { mlg_set_error("counters were already reduced densely"); return MLG_ERR_STATE; }
     if (ex->ctx != q->ctx) { mlg_set_error("exchange belongs to another context"); return MLG_ERR_ARG; }
-    if ((unsigned long long)q->ci_min * ex->world > 255ull) { mlg_set_error("ci_min * world must fit the 8-bit counters"); return MLG_ERR_ARG; }
+    if ((unsigned long long)q->ex_clamp * ex->world > 255ull) { mlg_set_error("exchange clamp (%d) * world must fit the 8-bit counters", q->ex_clamp); return MLG_ERR_ARG; }
     MLG_TRY(ensure_device(q->ctx));
     if (!q->present.p) { MLG_TRY(q->present.alloc((size_t)q->db->v.nd + 1)); MLG_TRY(q->touched.alloc((size_t)q->db->v.nd + 1)); }
     q->exchanged = true;
@@ -721,7 +730,7 @@ MLG_API int mlg_query_exchange_pack(mlg_query* q, mlg_exchange* ex) {
     MLG_TRY(check_exchange(q, ex));
     cudaStream_t st = q->ctx->s_comp;
     CUDA_TRY(cudaMemsetAsync(ex->status.p, 0, 16, st));
-    MLG_TRY(launch_pack_exchange(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ci_min, ex->send.p, ex->cap, ex->status.p + 3,
+    MLG_TRY(launch_pack_exchange(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ex_clamp, ex->send.p, ex->cap, ex->status.p + 3,
                                  st));
     q->st.gpu_launches += 1;
     return MLG_OK;
@@ -746,7 +755,7 @@ MLG_API int mlg_query_exchange_p2p(mlg_query* q, mlg_exchange* ex) {
     for (uint32_t w = 0; w < ex->world; ++w)
         if (w != ex->rank) boxes[np++] = ex->peer_mailbox[w] + ((unsigned long long)ex->rank * 2ull + parity) * ex->block_words;
     CUDA_TRY(cudaMemsetAsync(ex->status.p, 0, 16, st));
-    MLG_TRY(launch_push_peers(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ci_min, boxes, np, ex->cap, epoch,
+    MLG_TRY(launch_push_peers(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ex_clamp, boxes, np, ex->cap, epoch,
                               reinterpret_cast<unsigned int*>(ex->status.p + 2), ex->status.p + 3, st));
     MLG_TRY(launch_merge_exchange(q->cnt8.p, ex->mailbox + parity * ex->block_words, 2ull * ex->block_words, ex->world, ex->rank, ex->cap,
                                   q->db->v.nd, (uint32_t)q->ci_min, q->present.p, q->touched.p, q->d_scalar.p, ex->status.p, epoch,
@@ -763,7 +772,7 @@ MLG_API int mlg_query_exchange_dense(mlg_query* q, uint8_t** d_counts, uint64_t*
     if (q->merged) { mlg_set_error("counters were already merged sparsely"); return MLG_ERR_STATE; }
     MLG_TRY(ensure_device(q->ctx));
     if (q->touched.p) {
-        MLG_TRY(launch_clamp_counts(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ci_min, q->ctx->s_comp));
+        MLG_TRY(launch_clamp_counts(q->cnt8.p, q->touched.p, q->d_scalar.p + 1, (uint32_t)q->ex_clamp, q->ctx->s_comp));
         q->st.gpu_launches += 1;
     }
     *d_counts = q->cnt8.p; *n_counts = q->db->v.nd;

@@ -40,6 +40,7 @@
 #include <thread>
 #include <vector>
 #include <chrono>
+#include <stdexcept>
 #include "../../include/metalign_b200_ingest.h"
 #include "fast_inflate.h"
 #include "kmcdb.h"
@@ -199,6 +200,13 @@ struct mlgi_reader {
     size_t cur_i = 0;
     bool eof = false;
     uint64_t tot_reads = 0, tot_bases = 0, tot_text = 0;
+    // a share of the file (mlgi_open_share): the text [share_lo, share_hi) of a mapped plain file, or the members
+    // [bgzf_in0, bgzf_in1) of a BGZF file less bgzf_skip bytes in front and cut after bgzf_take bytes; its first line has
+    // number line_no0 (FASTQ phase) and share_first is its offset in the file's text
+    size_t share_lo = 0, share_hi = ~(size_t)0, bgzf_in0 = 0, bgzf_in1 = ~(size_t)0, bgzf_skip = 0, bgzf_take = ~(size_t)0;
+    uint64_t line_no0 = 0, share_first = 0;
+    int share_phase = 0;
+    bool tail_open = false;             // the text's last line has no '\n' (scanner thread)
     double t_wait_lines = 0, t_gather = 0, t_pack = 0, t_scan_wait = 0;   // MLGI_PROFILE=1
 
     // plain gzip (one long deflate stream): fast_inflate.h on the mapped file, one thread -- the stream is sequential.
@@ -296,10 +304,11 @@ struct mlgi_reader {
     }
     void read_loop_bgzf() {
         const unsigned char* base = (const unsigned char*)gzmap->p;
-        const size_t n = gzmap->n;
+        const size_t n = std::min(gzmap->n, bgzf_in1);
         struct Job { size_t in0, in1, out; std::shared_ptr<TextBuf> buf; bool ok = true; };
         const size_t P = (size_t)std::max(1, std::min(threads, 32));
-        size_t pos = 0;
+        size_t pos = bgzf_in0;
+        uint64_t upos = 0;                                           // text offset of the next job (share trimming)
         auto fail = [&](const char* m) { std::lock_guard<std::mutex> g(err_mu); io_error = m; q_raw.finish(); };
         while (pos < n) {
             std::vector<Job> jobs;
@@ -326,6 +335,12 @@ struct mlgi_reader {
             for (auto& x : th) x.join();
             for (auto& j : jobs) {
                 if (!j.ok) { fail("corrupt BGZF member"); return; }
+                const size_t jn = j.buf->n;                          // keep [bgzf_skip, bgzf_skip + bgzf_take) of the text
+                const size_t lo = (size_t)std::min<uint64_t>(jn, bgzf_skip > upos ? bgzf_skip - upos : 0);
+                const uint64_t stop = bgzf_take > ~(size_t)0 - bgzf_skip ? ~(uint64_t)0 : (uint64_t)(bgzf_skip + bgzf_take);
+                const size_t hi = (size_t)std::max<uint64_t>(lo, std::min<uint64_t>(jn, stop > upos ? stop - upos : 0));
+                upos += jn;
+                j.buf->off = HEAD + lo; j.buf->n = hi - lo;
                 RawBlock b; b.buf = j.buf;
                 if (j.buf->n && !q_raw.push(std::move(b))) return;
             }
@@ -391,7 +406,7 @@ struct mlgi_reader {
             line_ends_at(e);
             p = e + 1; q = e + 1;
         }
-        if (p < n && final_block) { line_ends_at(n); p = n; }   // the file's last line has no '\n'
+        if (p < n && final_block) { line_ends_at(n); p = n; tail_open = true; }   // the file's last line has no '\n'
         return p;                                         // bytes consumed; an incomplete line is carried into the next block
     }
 
@@ -442,8 +457,8 @@ struct mlgi_reader {
     // plain file: walk the mapping in views of `threads` blocks, scanned by that many threads (pass 1 counts the '\n' of
     // every part, pass 2 cuts the lines); a view's unterminated last line simply starts the next view
     void scan_loop_mapped() {
-        const char* base = (const char*)map->p;
-        const size_t n = map->n;
+        const char* base = (const char*)map->p + share_lo;
+        const size_t n = std::min(map->n, share_hi) - share_lo;
         const size_t P = (size_t)std::max(1, std::min(threads, 16));
         size_t pos = 0, span = block_bytes * P;
         while (pos < n) {
@@ -474,7 +489,8 @@ struct mlgi_reader {
             for (size_t i = 0; i < parts; ++i) if (open[i] != (size_t)-1) { used = open[i]; break; }
             if (used == 0 && end < n) { span += block_bytes * P; continue; }      // one line longer than the view: widen it
             // lines completed in this view: its '\n' up to `used`, plus the file's unterminated last line
-            line_no += (parts > 1 ? before[parts] - line_no : (uint64_t)count_newlines(vb, vn)) + ((end == n && vn && vb[vn - 1] != '\n') ? 1u : 0u);
+            if (end == n && vn && vb[vn - 1] != '\n') tail_open = true;
+            line_no += (parts > 1 ? before[parts] - line_no : (uint64_t)count_newlines(vb, vn)) + (tail_open ? 1u : 0u);
             pos += used; span = block_bytes * P;
             for (size_t i = 0; i < parts; ++i)
                 if (!outs[i].start.empty() && !q_lines.push(std::move(outs[i]))) return;
@@ -505,10 +521,10 @@ struct mlgi_reader {
                 if (bad) { std::lock_guard<std::mutex> g(err_mu); io_error = "gzip CRC mismatch"; break; }
             }
             std::shared_ptr<TextBuf> text;
-            if (more && carry.size() <= HEAD) {                // the usual case: the carried tail fits in front of the block
+            if (more && carry.size() <= b.buf->off) {          // the usual case: the carried tail fits in front of the block
                 text = b.buf;
-                memcpy(text->mem.get() + HEAD - carry.size(), carry.data(), carry.size());
-                text->off = HEAD - carry.size(); text->n += carry.size();
+                memcpy(text->mem.get() + text->off - carry.size(), carry.data(), carry.size());
+                text->off -= carry.size(); text->n += carry.size();
             } else {
                 text = std::make_shared<TextBuf>();
                 const size_t bn = more ? b.buf->n : 0;
@@ -882,6 +898,216 @@ MLGI_API int mlgi_open(const char* path, int input_type, int threads, mlgi_reade
         r->t_scan = std::thread([r] { r->scan_loop(); });
     }
     *out = r;
+    return 0;
+}
+
+}  // extern "C"
+
+namespace {
+
+// Random access to the text of a file, for the share geometry: a mapped plain file, or the members of a BGZF file
+// inflated on demand (a share looks at a few lines around its two ends only).
+struct TextAccess {
+    size_t total = 0;
+    virtual ~TextAccess() {}
+    virtual int at(size_t u) = 0;                       // the byte at u < total
+    virtual size_t find_nl(size_t u) = 0;               // the first '\n' at or after u, or total
+    size_t line_from(size_t u) {                        // the first line start at or after u
+        if (u == 0) return 0;
+        if (u >= total) return total;
+        if (at(u - 1) == '\n') return u;
+        const size_t e = find_nl(u);
+        return e >= total ? total : e + 1;
+    }
+    size_t next_line(size_t p) { const size_t e = find_nl(p); return e >= total ? total : e + 1; }
+    size_t prev_line(size_t p) {                        // the start of the line before the one starting at p > 0
+        size_t u = p - 1;
+        while (u > 0 && at(u - 1) != '\n') --u;
+        return u;
+    }
+    // a FASTQ header: the line starts with '@' and the line two after it with '+'
+    bool header_at(size_t p) {
+        if (p >= total || at(p) != '@') return false;
+        const size_t q = next_line(p);
+        if (q >= total) return false;
+        const size_t q2 = next_line(q);
+        return q2 < total && at(q2) == '+';
+    }
+    // FASTQ line number mod 4 of the line starting at s: from the first header among it and the next three lines, or,
+    // near the end of the file, among the four lines before it; -2 when there is none
+    int phase(size_t s) {
+        size_t p = s;
+        for (int k = 0; k < 4 && p < total; ++k, p = next_line(p))
+            if (header_at(p)) return (4 - k) & 3;
+        p = s;
+        for (int k = 1; k <= 4 && p > 0; ++k) {
+            p = prev_line(p);
+            if (header_at(p)) return k & 3;
+        }
+        return -2;
+    }
+};
+struct MappedText : TextAccess {
+    const char* b;
+    MappedText(const char* base, size_t n) : b(base) { total = n; }
+    int at(size_t u) override { return (unsigned char)b[u]; }
+    size_t find_nl(size_t u) override {
+        if (u >= total) return total;
+        const char* q = (const char*)memchr(b + u, '\n', total - u);
+        return q ? (size_t)(q - b) : total;
+    }
+};
+struct BgzfText : TextAccess {
+    const unsigned char* base; size_t n;
+    std::vector<size_t> cstart, ustart;                 // per member, plus one entry past the last
+    std::vector<std::string> cache;
+    BgzfText(const unsigned char* b, size_t nn) : base(b), n(nn) {}
+    std::string index() {
+        size_t u = 0;
+        for (size_t q = 0; q < n;) {
+            size_t cs = 0, hd = 0;
+            if (!mlgi_reader::bgzf_member(base + q, n - q, &cs, &hd)) return "not a BGZF member at byte " + std::to_string(q);
+            cstart.push_back(q); ustart.push_back(u);
+            const unsigned char* t = base + q + cs - 4;
+            u += (size_t)t[0] | ((size_t)t[1] << 8) | ((size_t)t[2] << 16) | ((size_t)t[3] << 24);
+            q += cs;
+        }
+        cstart.push_back(n); ustart.push_back(u);
+        total = u;
+        cache.resize(cstart.size());
+        return "";
+    }
+    size_t member_of(size_t u) const { return (size_t)(std::upper_bound(ustart.begin(), ustart.end() - 1, u) - ustart.begin()) - 1; }
+    const std::string& text(size_t m) {
+        std::string& c = cache[m];
+        const size_t want = ustart[m + 1] - ustart[m];
+        if (c.size() != want) {
+            c.assign(want + 1, '\0');
+            size_t got = 0;
+            if (!mlgi_reader::bgzf_inflate(base, n, cstart[m], cstart[m + 1], &c[0], &got) || got != want) throw std::runtime_error("corrupt BGZF member");
+            c.resize(want);
+        }
+        return c;
+    }
+    int at(size_t u) override { const size_t m = member_of(u); return (unsigned char)text(m)[u - ustart[m]]; }
+    size_t find_nl(size_t u) override {
+        for (size_t m = u < total ? member_of(u) : cstart.size() - 1; u < total; ++m) {
+            const std::string& t = text(m);
+            const size_t o = u - ustart[m];
+            const char* q = (const char*)memchr(t.data() + o, '\n', t.size() - o);
+            if (q) return ustart[m] + (size_t)(q - t.data());
+            u = ustart[m + 1];
+        }
+        return total;
+    }
+};
+
+}  // namespace
+
+extern "C" {
+
+// A share [begin, end) of a reads file: the lines whose first byte is in it (plain file), or in the text of the BGZF members
+// whose compressed start is in it.  A plain gzip stream cannot be split: the share that starts at byte 0 reads it all.
+MLGI_API int mlgi_open_share(const char* path, int input_type, int threads, uint64_t begin, uint64_t end, mlgi_reader** out) {
+    if (!path || !out) { set_error("null argument"); return -2; }
+    if (input_type != MLGI_FASTQ && input_type != MLGI_FASTA) { set_error("input_type must be MLGI_FASTQ or MLGI_FASTA"); return -2; }
+    if (begin > end) { set_error("share begins at %llu, after its end %llu", (unsigned long long)begin, (unsigned long long)end); return -2; }
+    const int fd = open(path, O_RDONLY);
+    if (fd < 0) { set_error("cannot open %s", path); return -3; }
+    struct Closer { int fd; ~Closer() { close(fd); } } closer{fd};
+    struct stat sb;
+    if (fstat(fd, &sb) != 0 || !S_ISREG(sb.st_mode)) { set_error("%s: a share needs a regular file", path); return -3; }
+    const size_t size = (size_t)sb.st_size;
+    if (end > size) end = size;
+    if (begin > end) begin = end;
+    std::shared_ptr<Mapping> map;
+    if (size) {
+        void* p = mmap(nullptr, size, PROT_READ, MAP_PRIVATE, fd, 0);
+        if (p == MAP_FAILED) { set_error("%s: mmap failed: %s", path, strerror(errno)); return -3; }
+        map = std::make_shared<Mapping>(); map->p = p; map->n = size;
+    }
+    const unsigned char* base = map ? (const unsigned char*)map->p : nullptr;
+    const bool gz = size >= 2 && base[0] == 0x1f && base[1] == 0x8b;
+    size_t cs = 0, hd = 0;
+    const bool bgzf = gz && mlgi_reader::bgzf_member(base, size, &cs, &hd);
+    std::unique_ptr<mlgi_reader> r;
+    if (gz && !bgzf) {                                   // one DEFLATE stream: all of it or nothing
+        if (begin == 0) {
+            if (end < size)
+                fprintf(stderr, "mlgi: %s is one gzip stream and cannot be split: one share reads all of it, the others none "
+                                "(recompress it with bgzip to read it in parallel)\n", path);
+            mlgi_reader* whole = nullptr;
+            const int rc = mlgi_open(path, input_type, threads, &whole);
+            if (rc) return rc;
+            *out = whole;
+            return 0;
+        }
+        r.reset(new mlgi_reader());
+        r->share_phase = -1;
+        r->q_lines.finish();
+        *out = r.release();
+        return 0;
+    }
+    r.reset(new mlgi_reader());
+    r->type = input_type;
+    int hw = (int)std::thread::hardware_concurrency();
+    if (hw < 1) hw = 1;
+    r->threads = threads > 0 ? threads : hw;
+    if (const char* s = getenv("MLGI_BLOCK_BYTES")) { long v = atol(s); if (v >= 16) r->block_bytes = (size_t)v; }
+    size_t S = 0, E = 0;
+    try {
+        std::unique_ptr<TextAccess> t;
+        size_t u0 = 0, u1 = 0;
+        BgzfText* bt = nullptr;
+        if (bgzf) {
+            bt = new BgzfText(base, size);
+            t.reset(bt);
+            const std::string e = bt->index();
+            if (!e.empty()) { set_error("%s: %s", path, e.c_str()); return -3; }
+            const size_t m0 = (size_t)(std::lower_bound(bt->cstart.begin(), bt->cstart.end(), (size_t)begin) - bt->cstart.begin());
+            const size_t m1 = (size_t)(std::lower_bound(bt->cstart.begin(), bt->cstart.end(), (size_t)end) - bt->cstart.begin());
+            u0 = bt->ustart[m0]; u1 = bt->ustart[m1];
+        } else {
+            t.reset(new MappedText((const char*)base, size));
+            u0 = begin; u1 = end;
+        }
+        S = t->line_from(u0);
+        E = std::max(S, t->line_from(u1));
+        r->share_first = S;
+        r->share_phase = S < E ? (input_type == MLGI_FASTQ ? t->phase(S) : 0) : -1;
+        if (bt && S < E) {                               // the members that hold [S, E)
+            const size_t a = bt->member_of(S), b = bt->member_of(E - 1) + 1;
+            r->bgzf_in0 = bt->cstart[a]; r->bgzf_in1 = bt->cstart[b];
+            r->bgzf_skip = S - bt->ustart[a]; r->bgzf_take = E - S;
+        }
+    } catch (const std::exception& e) {
+        set_error("%s: %s", path, e.what());
+        return -3;
+    }
+    r->line_no = r->line_no0 = r->share_phase > 0 ? (uint64_t)r->share_phase : 0;
+    if (S >= E) r->q_lines.finish();
+    else if (bgzf) {
+        r->gzmap = map;
+        r->t_read = std::thread([p = r.get()] { p->read_loop_bgzf(); });
+        r->t_scan = std::thread([p = r.get()] { p->scan_loop(); });
+    } else {
+        r->map = map;
+        r->share_lo = S; r->share_hi = E;
+        r->t_scan = std::thread([p = r.get()] { p->scan_loop_mapped(); });
+    }
+    *out = r.release();
+    return 0;
+}
+
+// What the phase check of a split FASTQ file needs from a share, once mlgi_next has returned 0: the text offset of its
+// first line, its number of '\n', and the FASTQ line number mod 4 it took for its first line (-1: the share is empty, -2:
+// no record start was found near it).
+MLGI_API int mlgi_share_info(mlgi_reader* r, uint64_t* first, uint64_t* newlines, int* phase) {
+    if (!r) { set_error("null reader"); return -2; }
+    if (!r->eof) { set_error("the share has not been read to its end"); return -4; }
+    if (first) *first = r->share_first;
+    if (newlines) *newlines = r->line_no - r->line_no0 - (r->tail_open ? 1u : 0u);
+    if (phase) *phase = r->share_phase;
     return 0;
 }
 

@@ -344,30 +344,31 @@ __global__ void k_clear_touched(unsigned char* cnt8, const uint32_t* __restrict_
     for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x)
         cnt8[touched[i]] = 0;
 }
-// clamp the counters that are non-zero (listed in touched[]) to ci_min: what a rank contributes to the cross-rank sum
+// clamp the counters that are non-zero (listed in touched[]) to `clamp` (ci_min unless the query set another level):
+// what a rank contributes to the cross-rank sum
 __global__ void k_clamp_counts(unsigned char* cnt8, const uint32_t* __restrict__ touched, const unsigned long long* __restrict__ d_n,
-                               uint32_t ci_min) {
+                               uint32_t clamp) {
     const unsigned long long n = *d_n;
     for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
         const uint32_t e = touched[i];
-        if (cnt8[e] > ci_min) cnt8[e] = (unsigned char)ci_min;
+        if (cnt8[e] > clamp) cnt8[e] = (unsigned char)clamp;
     }
 }
-// a rank's own counter clamped to ci_min in place, as its contribution to the cross-rank sum: after a merge the table
-// holds sum over ranks of min(count, ci_min) on every rank, the same as the dense form (k_clamp_counts) leaves it
-__device__ __forceinline__ uint32_t clamp_own(unsigned char* cnt8, uint32_t e, uint32_t ci_min) {
+// a rank's own counter clamped to `clamp` in place, as its contribution to the cross-rank sum: after a merge the table
+// holds sum over ranks of min(count, clamp) on every rank, the same as the dense form (k_clamp_counts) leaves it
+__device__ __forceinline__ uint32_t clamp_own(unsigned char* cnt8, uint32_t e, uint32_t clamp) {
     const uint32_t c = cnt8[e];
-    if (c <= ci_min) return c;
-    cnt8[e] = (unsigned char)ci_min;
-    return ci_min;
+    if (c <= clamp) return c;
+    cnt8[e] = (unsigned char)clamp;
+    return clamp;
 }
-// sparse form of a rank's contribution: one 64-bit entry per non-zero counter = index | min(count, ci_min) << 32
+// sparse form of a rank's contribution: one 64-bit entry per non-zero counter = index | min(count, clamp) << 32
 __global__ void k_pack_touched(unsigned char* cnt8, const uint32_t* __restrict__ touched,
-                               const unsigned long long* __restrict__ d_n, uint32_t ci_min, unsigned long long* out) {
+                               const unsigned long long* __restrict__ d_n, uint32_t clamp, unsigned long long* out) {
     const unsigned long long n = *d_n;
     for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
         const uint32_t e = touched[i];
-        out[i] = (unsigned long long)e | ((unsigned long long)clamp_own(cnt8, e, ci_min) << 32);
+        out[i] = (unsigned long long)e | ((unsigned long long)clamp_own(cnt8, e, clamp) << 32);
     }
 }
 // add another rank's sparse entries into this rank's counters (saturating); a counter that crosses ci_min joins present[]
@@ -396,18 +397,18 @@ __global__ void k_merge_sparse(unsigned char* cnt8, const unsigned long long* __
 }
 // ---- the multi-GPU exchange without a host round trip (mlg_exchange, capi.cu) --------------------------------------
 // A rank's contribution travels as one BLOCK of block_words 64-bit words: word 0 = number of non-zero counters n
-// (| epoch << 40 on the direct path), word 1 unused, then min(n, cap) entries index | min(count, ci_min) << 32.
+// (| epoch << 40 on the direct path), word 1 unused, then min(n, cap) entries index | min(count, clamp) << 32.
 // Both pack kernels clamp ALL n own counters (not only the first cap) and leave n in *own_count, the count the merge
 // judges this rank's block by: the merge itself appends to touched[] and so cannot read n there.
 constexpr unsigned long long XCNT_MASK = (1ull << 40) - 1ull;
 // fill this rank's block in local memory (the caller all-gathers the blocks, e.g. with NCCL)
 __global__ void k_pack_exchange(unsigned char* cnt8, const uint32_t* __restrict__ touched, const unsigned long long* __restrict__ d_n,
-                                uint32_t ci_min, unsigned long long* out, unsigned long long cap, unsigned long long* own_count) {
+                                uint32_t clamp, unsigned long long* out, unsigned long long cap, unsigned long long* own_count) {
     const unsigned long long n = *d_n;
     if (blockIdx.x == 0 && threadIdx.x == 0) { out[0] = n; out[1] = 0; *own_count = n; }
     for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
         const uint32_t e = touched[i];
-        const uint32_t c = clamp_own(cnt8, e, ci_min);
+        const uint32_t c = clamp_own(cnt8, e, clamp);
         if (i < cap) out[2 + i] = (unsigned long long)e | ((unsigned long long)c << 32);
     }
 }
@@ -415,12 +416,12 @@ __global__ void k_pack_exchange(unsigned char* cnt8, const uint32_t* __restrict_
 // CTA's stores are fenced -- publish count | epoch << 40 in word 0 of each copy with a system-scope release
 struct PeerBoxes { unsigned long long* box[MLG_MAX_RANKS]; uint32_t n; };
 __global__ void k_push_peers(unsigned char* cnt8, const uint32_t* __restrict__ touched, const unsigned long long* __restrict__ d_n,
-                             uint32_t ci_min, PeerBoxes pb, unsigned long long cap, unsigned long long epoch, unsigned int* done_ctas,
+                             uint32_t clamp, PeerBoxes pb, unsigned long long cap, unsigned long long epoch, unsigned int* done_ctas,
                              unsigned long long* own_count) {
     const unsigned long long n = *d_n;
     for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
         const uint32_t e = touched[i];
-        const uint32_t c = clamp_own(cnt8, e, ci_min);
+        const uint32_t c = clamp_own(cnt8, e, clamp);
         if (i >= cap) continue;
         const unsigned long long en = (unsigned long long)e | ((unsigned long long)c << 32);
         for (uint32_t p = 0; p < pb.n; ++p) pb.box[p][2 + i] = en;
@@ -581,14 +582,14 @@ __global__ void k_gather_hit_flags(const uint32_t* hitbits, unsigned long long w
 
 }  // namespace
 
-int launch_clamp_counts(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min, cudaStream_t st) {
-    k_clamp_counts<<<148u * 4u, 256, 0, st>>>(cnt8, touched, d_n_touched, ci_min);
+int launch_clamp_counts(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t clamp, cudaStream_t st) {
+    k_clamp_counts<<<148u * 4u, 256, 0, st>>>(cnt8, touched, d_n_touched, clamp);
     CUDA_TRY(cudaGetLastError());
     return MLG_OK;
 }
-int launch_pack_touched(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
+int launch_pack_touched(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t clamp,
                         unsigned long long* out, cudaStream_t st) {
-    k_pack_touched<<<148u * 4u, 256, 0, st>>>(cnt8, touched, d_n_touched, ci_min, out);
+    k_pack_touched<<<148u * 4u, 256, 0, st>>>(cnt8, touched, d_n_touched, clamp, out);
     CUDA_TRY(cudaGetLastError());
     return MLG_OK;
 }
@@ -600,19 +601,19 @@ int launch_merge_sparse(unsigned char* cnt8, const unsigned long long* entries, 
     CUDA_TRY(cudaGetLastError());
     return MLG_OK;
 }
-int launch_pack_exchange(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
+int launch_pack_exchange(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t clamp,
                          unsigned long long* out, unsigned long long cap, unsigned long long* own_count, cudaStream_t st) {
-    k_pack_exchange<<<148u * 2u, 256, 0, st>>>(cnt8, touched, d_n_touched, ci_min, out, cap, own_count);
+    k_pack_exchange<<<148u * 2u, 256, 0, st>>>(cnt8, touched, d_n_touched, clamp, out, cap, own_count);
     CUDA_TRY(cudaGetLastError());
     return MLG_OK;
 }
-int launch_push_peers(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t ci_min,
+int launch_push_peers(unsigned char* cnt8, const uint32_t* touched, const unsigned long long* d_n_touched, uint32_t clamp,
                       unsigned long long* const* boxes, uint32_t n_peers, unsigned long long cap, unsigned long long epoch,
                       unsigned int* done_ctas, unsigned long long* own_count, cudaStream_t st) {
     PeerBoxes pb{};
     pb.n = n_peers;
     for (uint32_t p = 0; p < n_peers && p < MLG_MAX_RANKS; ++p) pb.box[p] = boxes[p];
-    k_push_peers<<<148u, 256, 0, st>>>(cnt8, touched, d_n_touched, ci_min, pb, cap, epoch, done_ctas, own_count);
+    k_push_peers<<<148u, 256, 0, st>>>(cnt8, touched, d_n_touched, clamp, pb, cap, epoch, done_ctas, own_count);
     CUDA_TRY(cudaGetLastError());
     return MLG_OK;
 }

@@ -1,8 +1,8 @@
 """Read-sharded multi-GPU run (SURVEY.md 8e): one process per GPU, database replicated, each rank probes
 its own contiguous share of the reads, then ONE exchange step -- the sum over ranks of the per-database-k-mer
-occurrence counters, each rank's counters clamped to ci_min first -- and the per-genome table is derived from
-the summed counters.  Per-genome tables of shards are never summed: the >= ci_min threshold is global and
-hits have set semantics.
+occurrence counters, each rank's counters clamped first (to ci_min, or higher: reduce_query's clamp) -- and the
+per-genome table is derived from the summed counters.  Per-genome tables of shards are never summed: the >= ci_min
+threshold is global and hits have set semantics.
 
 The sum comes in two equivalent forms (NCCL over NVLink on GPUs, gloo on CPU):
   "sparse" (default)  the counter table is >99.9 % zeros, so every rank all-gathers its non-zero counters
@@ -45,13 +45,14 @@ def shard_range(n_items: int, rank: int, world: int) -> Tuple[int, int]:
     return begin, begin + base + (1 if rank < rem else 0)
 
 
-def max_summed_count(ci_min: int, world: int) -> int:
-    return ci_min * world
+def max_summed_count(clamp: int, world: int) -> int:
+    return clamp * world
 
 
-def check_reducible(ci_min: int, world: int) -> None:
-    if max_summed_count(ci_min, world) > 255:
-        raise ValueError("ci_min * world_size must fit in uint8 for the counter all-reduce")
+def check_reducible(clamp: int, world: int) -> None:
+    """clamp: the level each rank's counters are clamped to before the sum (the query's ci_min unless set higher)"""
+    if max_summed_count(clamp, world) > 255:
+        raise ValueError("exchange clamp * world_size must fit in uint8 for the counter all-reduce")
 
 
 def allreduce_counts(counts, group=None):
@@ -179,18 +180,21 @@ def _get_exchange(ctx, device: int, group, p2p: bool, cap: int = 0):
     return cur
 
 
-def reduce_query(query, device: int = 0, group=None, mode: str = None) -> None:
+def reduce_query(query, device: int = 0, group=None, mode: str = None, clamp: int = None) -> None:
     """The exchange step for a live GPU Query (see the module docstring).  Nothing here synchronises the host: every
     kernel and the collective are queued on the library's compute stream, and `query.finish()` is the join.  If some
     rank had more non-zero counters than the persistent blocks hold, finish() comes back asking for a repeat, and the
     closure left in `query._exchange_retry` redoes the exchange with larger blocks (collectively: every rank sees the
-    same gathered counts)."""
+    same gathered counts).  clamp (ci_min .. 255, default ci_min): the level every rank's counters are clamped to before
+    the sum; with counter_max (3) the intersection files of every rank have the counts of one query over all the reads."""
     import torch
     import torch.distributed as dist
     if not (dist.is_initialized() and dist.get_world_size(group) > 1):
         return
     world = dist.get_world_size(group)
-    check_reducible(query_ci_min(query), world)
+    check_reducible(query_ci_min(query) if clamp is None else int(clamp), world)
+    if clamp is not None:
+        query.set_exchange_clamp(clamp)
     mode = mode or exchange_mode()
     ctx = query.db.ctx
     if mode == "dense":

@@ -39,6 +39,8 @@ def ingest_lib():
         L = C.CDLL(path)
         L.mlgi_last_error.restype = C.c_char_p
         L.mlgi_open.argtypes = [C.c_char_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]
+        L.mlgi_open_share.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_uint64, C.c_uint64, C.POINTER(C.c_void_p)]
+        L.mlgi_share_info.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_int)]
         L.mlgi_next.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_uint64,
                                 C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
         L.mlgi_spilled_runs.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64]
@@ -119,14 +121,19 @@ class PackedBatches:
     """Iterate a reads file as packed batches: yields (bases uint8[], nruns uint32[m,2], off uint64[n+1], n_reads).
     The arrays are views of two alternating buffer sets (so one batch can still be in flight to the GPU while the
     next is being filled); `alloc(nbytes) -> uint8 ndarray` supplies them (pinned memory from api.pinned_array on a
-    GPU box, numpy otherwise)."""
+    GPU box, numpy otherwise).  share = (begin, end): only the records of that byte range of the file
+    (mlgi_open_share; see share_ranges and check_share_phases)."""
 
     def __init__(self, path: str, input_type: str, reads_per_batch: int = 4_000_000, bases_per_batch: int = 0,
-                 threads: int = 0, alloc=None, max_runs: int = 0):
+                 threads: int = 0, alloc=None, max_runs: int = 0, share=None):
         self.L = ingest_lib()
         self.h = C.c_void_p()
         t = {"fastq": FASTQ, "fasta": FASTA}[input_type]
-        if self.L.mlgi_open(path.encode(), t, int(threads), C.byref(self.h)) != 0:
+        if share is not None:
+            rc = self.L.mlgi_open_share(path.encode(), t, int(threads), int(share[0]), int(share[1]), C.byref(self.h))
+        else:
+            rc = self.L.mlgi_open(path.encode(), t, int(threads), C.byref(self.h))
+        if rc != 0:
             raise IOError(self.L.mlgi_last_error().decode())
         self.max_reads = int(reads_per_batch)
         self.max_bases = int(bases_per_batch) or min(self.max_reads * 160, 0xFFFFFF00)
@@ -167,6 +174,14 @@ class PackedBatches:
         self.L.mlgi_stats(self.h, C.byref(a), C.byref(b), C.byref(c))
         return dict(reads=a.value, bases=b.value, text_bytes=c.value)
 
+    def share_info(self) -> dict:
+        """after the last batch: the text offset of the share's first line, its newline count and its FASTQ phase
+        (-1: empty share, -2: no record start found near it)"""
+        first, nl, ph = C.c_uint64(), C.c_uint64(), C.c_int()
+        if self.L.mlgi_share_info(self.h, C.byref(first), C.byref(nl), C.byref(ph)) != 0:
+            raise IOError(self.L.mlgi_last_error().decode())
+        return dict(first=first.value, newlines=nl.value, phase=ph.value)
+
     def close(self):
         if self.h:
             self.L.mlgi_close(self.h)
@@ -177,6 +192,26 @@ class PackedBatches:
             self.close()
         except Exception:  # noqa: BLE001
             pass
+
+
+def share_ranges(path: str, world: int):
+    """balanced [begin, end) byte ranges of the file on disk, one per rank"""
+    size = os.path.getsize(path)
+    return [(size * r // world, size * (r + 1) // world) for r in range(world)]
+
+
+def check_share_phases(infos, input_type: str = "fastq") -> None:
+    """infos: share_info() of every share, in file order.  A FASTQ share parses its lines from the phase it found at its
+    first record start; that is the single-reader parse only if the phase equals the number of lines before the share mod
+    4 (the earlier shares' newline counts).  Raises ValueError naming the offset where they differ."""
+    if input_type != "fastq":
+        return
+    before = 0
+    for i, info in enumerate(infos):
+        if info["phase"] != -1 and info["phase"] != before % 4:
+            raise ValueError("reads file is not 4-line FASTQ: share %d, starting at text byte %d, took line phase %d but %d "
+                             "lines come before it; read this file on one GPU" % (i, info["first"], info["phase"], before))
+        before += info["newlines"]
 
 
 def _read_all(path: str) -> np.ndarray:

@@ -2,13 +2,13 @@
 """Drop-in for scripts/metalign.py of nlapier2/Metalign: same flags; database selection runs on the GPU
 (metalign_b200.select_db), then the reference's own alignment/profiling stage (scripts/map_and_profile.py,
 minimap2 -- out of scope here, used unchanged if it is importable) runs on the files selection wrote.
-With --select_only, or when map_and_profile is not importable, it stops after selection and keeps temp_dir."""
+With --select_only, or when map_and_profile is not importable, it stops after selection and keeps temp_dir.
+Under torchrun every rank takes part in the selection (metalign_b200.select_db) and rank 0 alone maps and profiles."""
 from __future__ import annotations
 
 import argparse
 import shutil
 import sys
-import tempfile
 
 from . import select_db as select
 
@@ -47,10 +47,11 @@ def metalign_parseargs(argv=None):
 
 def main(argv=None):
     args = metalign_parseargs(argv)
+    select.init_ranks(args)
     if not args.data.endswith("/"):
         args.data += "/"
     if args.temp_dir == "AUTO/":
-        args.temp_dir = tempfile.mkdtemp(prefix=args.data)
+        args.temp_dir = select.shared_mkdtemp(args.data)
     if not args.temp_dir.endswith("/"):
         args.temp_dir += "/"
     if args.sensitive and args.precise:
@@ -68,6 +69,8 @@ def main(argv=None):
 
     select.select_main(args)
     mapper = None
+    if select.ranks()[0] != 0:
+        return
     if not args.select_only:
         try:
             import map_and_profile as mapper      # the reference's scripts/ directory on PYTHONPATH

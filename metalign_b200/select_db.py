@@ -10,6 +10,11 @@ cmash_db_n1000_k60.h5 / _30-60-10.bf / _dump.kmc_* (select_db.py:44,69,70).
 
 Extra, optional flags (not in the reference): --db_file, --gate, --device, --k_range, --read_kmer_budget,
 --read_kmer_passes.
+
+Under torchrun (WORLD_SIZE > 1) every rank drives the GPU of its LOCAL_RANK: it reads its own byte range of the reads
+file (ingest.share_ranges), the ranks sum their counters in one exchange (dist.reduce_query, each rank's counters clamped
+to counter_max so that the intersection counts are those of one GPU), and rank 0 alone writes the files -- the same bytes
+as a single-process run.  --threads is then per rank.
 """
 from __future__ import annotations
 
@@ -28,6 +33,11 @@ HEADER_LINES = ("Accesion\tLength\tTaxID\tLineage\tTaxID_Lineage\n",          # 
 _T0 = None
 
 
+def _now():
+    import time
+    return time.perf_counter()
+
+
 def _tick(label):
     """MLG_TIMING=1: stage times on stderr (seconds since the module was imported)"""
     if os.environ.get("MLG_TIMING"):
@@ -37,6 +47,63 @@ def _tick(label):
         if _T0 is None:
             _T0 = now
         sys.stderr.write("[mlg %7.3f s] %s\n" % (now - _T0, label))
+
+
+def ranks():
+    """(rank, world) of a torchrun launch with the process group up, else (0, 1)"""
+    if "torch" not in sys.modules:          # a single process need not pay for importing torch
+        return 0, 1
+    import torch.distributed as tdist
+    if tdist.is_available() and tdist.is_initialized():
+        return tdist.get_rank(), tdist.get_world_size()
+    return 0, 1
+
+
+def init_ranks(args):
+    """under torchrun (WORLD_SIZE > 1): the NCCL process group, --device = LOCAL_RANK, this process bound to the cores of
+    its GPU's NUMA node (before any reader thread starts).  Nothing for a single process."""
+    if int(os.environ.get("WORLD_SIZE", "1")) <= 1:
+        return
+    from . import dist as mdist
+    _rank, _world, local = mdist.init_from_env("nccl")
+    args.device = local
+    mdist.bind_to_gpu_numa(local)
+
+
+def shared_mkdtemp(prefix):
+    """tempfile.mkdtemp on rank 0, the same path on every rank"""
+    rank, world = ranks()
+    if world == 1:
+        return tempfile.mkdtemp(prefix=prefix)
+    import torch.distributed as tdist
+    box = [tempfile.mkdtemp(prefix=prefix) if rank == 0 else None]
+    tdist.broadcast_object_list(box, src=0)
+    return box[0]
+
+
+def _on_rank0(fn):
+    """fn() on rank 0 alone; its result, or its failure, reaches every rank"""
+    rank, world = ranks()
+    if world == 1:
+        return fn()
+    import torch.distributed as tdist
+    box = [None, None]
+    if rank == 0:
+        try:
+            box[0] = fn()
+        except Exception as e:  # noqa: BLE001  (the other ranks wait in the broadcast)
+            box[1] = e
+    tdist.broadcast_object_list(box, src=0)
+    if box[1] is not None:
+        raise box[1] if rank == 0 else RuntimeError("select_db: rank 0 failed: %s" % box[1])
+    return box[0]
+
+
+def _all_ok(err, args):
+    """collective: raise on every rank if any rank has an error (its own error where it has one)"""
+    from . import dist as mdist
+    if not mdist._flag_min(err is None, args.device, None):
+        raise err if err is not None else RuntimeError("select_db: another rank failed")
 
 
 def select_parseargs(argv=None):
@@ -56,7 +123,7 @@ def select_parseargs(argv=None):
                         "-ci2 -cs3) and of the intersection (60mers_intersection), and the intersection dump")
     p.add_argument("--strain_level", action="store_true", help="keep every strain above the cutoff (default: one per species)")
     p.add_argument("--temp_dir", default="AUTO/", help="directory for intermediate files")
-    p.add_argument("--threads", type=int, default=4, help="accepted for compatibility (KMC threads in the reference)")
+    p.add_argument("--threads", type=int, default=4, help="reader threads (per rank under torchrun; KMC threads in the reference)")
     # additions
     p.add_argument("--db_file", default="AUTO", help="native database file (default data/%s)" % DB_BASENAME)
     p.add_argument("--gate", default="exact", choices=["exact", "none"], help="smallest-k prefilter model (see DESIGN.md)")
@@ -98,7 +165,11 @@ def run_kmc_steps(args):
     reads that belong to the database sketch; the live query is parked on args for run_cmash_and_cutoff."""
     from . import ingest
     from .api import Context, Database, pinned_array
+    rank, world = ranks()
+    times = args._mlg_times = {}
+    t0 = _now()
     ctx = db = query = reader = None
+    err = None
     try:
         # pandas (the CSV tail) takes a good part of a second to import: do it while the GPU works
         import threading
@@ -116,8 +187,9 @@ def run_kmc_steps(args):
             try:
                 # 2 M reads per batch: two buffer sets of ~110 MB of page-locked memory (0.7 ms per MiB to pin: with 4 M reads
                 # per batch the reader's set-up outlasted the database load it is meant to hide behind)
+                share = ingest.share_ranges(args.reads, world)[rank] if world > 1 else None
                 box["reader"] = ingest.PackedBatches(args.reads, args.input_type, reads_per_batch=2_000_000, alloc=pinned_array,
-                                                     threads=max(1, int(getattr(args, "threads", 4) or 4)))
+                                                     threads=max(1, int(getattr(args, "threads", 4) or 4)), share=share)
             except BaseException as e:  # noqa: BLE001
                 box["error"] = e
         th = threading.Thread(target=open_reader)
@@ -131,22 +203,51 @@ def run_kmc_steps(args):
             raise box["error"]
         _tick("database loaded, reader started")
         # -ci2 (select_db.py:50); the read k-mer table only for the reads_60mers database --keep_temp_files leaves behind
+        # (across ranks the read k-mers are only counted in passes: share_read_kmers hands the reads around)
         query = db.query(ci_min=2, gate=args.gate, count_empty_in_den=True, read_kmers=bool(args.keep_temp_files),
-                         read_kmer_budget=args.read_kmer_budget, read_kmer_passes=args.read_kmer_passes)
+                         read_kmer_budget=args.read_kmer_budget, read_kmer_passes=args.read_kmer_passes or world > 1)
+        times["open_s"] = _now() - t0
+        t0 = _now()
         for bases, nruns, off, n_reads in reader:
             query.push_packed_nruns(bases, nruns if len(nruns) else None, off, n_reads)
         query.sync()
+        times["push_s"] = _now() - t0
         _tick("reads pushed and probed")
-    except BaseException:
+        if world > 1:
+            info = reader.share_info()
+    except BaseException as e:  # noqa: BLE001
+        err = e
+    if world > 1:
+        # every rank learns whether every other rank got this far, and every rank checks the FASTQ phases of all shares
+        import torch.distributed as tdist
+        try:
+            _all_ok(err, args)
+            infos = [None] * world
+            tdist.all_gather_object(infos, info)
+            ingest.check_share_phases(infos, args.input_type)
+            t0 = _now()
+            from . import dist as mdist
+            if args.keep_temp_files:
+                mdist.share_read_kmers(query, args.device)
+            mdist.reduce_query(query, args.device, clamp=3)          # -cs3: the intersection counts of one GPU
+            query.sync()
+            times["exchange_s"] = _now() - t0
+            _tick("exchange done")
+        except BaseException as e:  # noqa: BLE001
+            err = err or e
+    if err is not None:
         # a corrupt reads file, a failed push: give the device and pinned memory back before the error travels on
         # (a caller looping over samples would otherwise accumulate them)
+        if world > 1:
+            from . import dist as mdist
+            mdist.close_exchanges()
         for obj in (reader, query, db, ctx):
             if obj is not None:
                 try:
                     obj.close()
                 except Exception:  # noqa: BLE001
                     pass
-        raise
+        raise err
     reader.close()
     _tick("reader closed")
     args._mlg = (ctx, db, query)
@@ -160,7 +261,12 @@ def run_cmash_and_cutoff(args, taxid2info):
         from ._lib import MLG_ERR_NOMEM, MlgError
         ctx, db, query = args._mlg
         cmash_out = args.temp_dir + "cmash_query_results.csv"
+        rank, world = ranks()
+        if world > 1:
+            return _gpu_files_ranks(args, taxid2info, cmash_out)
+        t0 = _now()
         res = query.finish_sparse()                       # rows for the genomes with a hit: all the CSV can hold
+        args._mlg_times["finish_s"] = _now() - t0
         _tick("containment table")
         cmash_tail.write_results_csv_sparse(cmash_out, db.names, db.ks, res["genomes"], res["ci"], 0.0)      # '-c 0'
         _tick("csv written")
@@ -182,7 +288,62 @@ def run_cmash_and_cutoff(args, taxid2info):
         _tick("GPU objects closed")
     else:
         cmash_out = args.cmash_results
+    return _select(args, taxid2info, cmash_out)
 
+
+def _gpu_files_ranks(args, taxid2info, cmash_out):
+    """run_cmash_and_cutoff of a torchrun launch, after the exchange: every rank finishes its query (identical on every
+    rank), rank 0 writes the CSV and the intersection files, the ranks join reads_60mers (dist.write_reads_kmc), and rank 0
+    selects and hands the selection to every rank.  A failure anywhere raises on every rank, and rank 0 removes the files
+    of this stage."""
+    import torch.distributed as tdist
+    from . import cmash_tail
+    from . import dist as mdist
+    rank, _world = ranks()
+    ctx, db, query = args._mlg
+    del args._mlg
+    times = args._mlg_times
+    written = [cmash_out, args.temp_dir + "60mers_intersection_dump", args.temp_dir + "60mers_intersection_dump.fa", args.db,
+               args.dbinfo_out] + [args.temp_dir + p + e for p in ("60mers_intersection", "reads_60mers") for e in (".kmc_pre", ".kmc_suf")]
+    err = None
+    try:
+        try:
+            t0 = _now()
+            res = query.finish_sparse()
+            times["finish_s"] = _now() - t0
+            if rank == 0:
+                cmash_tail.write_results_csv_sparse(cmash_out, db.names, db.ks, res["genomes"], res["ci"], 0.0)
+                if args.keep_temp_files:
+                    query.dump_intersection(written[1], written[2])
+                    query.write_intersection_kmc(args.temp_dir + "60mers_intersection", counter_max=3)
+        except Exception as e:  # noqa: BLE001  (every rank has to take part in the collectives below)
+            err = e
+        _all_ok(err, args)
+        if args.keep_temp_files:
+            mdist.write_reads_kmc(query, args.temp_dir + "reads_60mers", 2, 3, args.device)
+        chosen = _on_rank0(lambda: _select_and_write(args, taxid2info, cmash_out))
+    except BaseException:
+        if rank == 0:
+            for path in written:
+                if os.path.exists(path):
+                    os.remove(path)
+        raise
+    finally:
+        query.close(); db.close()
+        mdist.close_exchanges()
+        ctx.close()
+    args._mlg_subset_written = True
+    return chosen
+
+
+def _select_and_write(args, taxid2info, cmash_out):
+    chosen = _select(args, taxid2info, cmash_out)
+    make_db_and_dbinfo(args, chosen, taxid2info)
+    return chosen
+
+
+def _select(args, taxid2info, cmash_out):
+    """the cutoff and the one-strain-per-species rule of select_db.py:80-96 on the CSV"""
     chosen, seen_species = [], set()
     with open(cmash_out, "r") as fh:
         next(fh, None)                                    # ',k=30,k=40,k=50,k=60'
@@ -244,7 +405,7 @@ def _normalise(args):
     if not args.db_dir.endswith("/"):
         args.db_dir += "/"
     if args.temp_dir == "AUTO/":
-        args.temp_dir = tempfile.mkdtemp(prefix=args.data)
+        args.temp_dir = shared_mkdtemp(args.data)
     if not args.temp_dir.endswith("/"):
         args.temp_dir += "/"
     os.makedirs(args.temp_dir, exist_ok=True)
@@ -267,6 +428,7 @@ def select_main(args=None):
     elif args.cutoff < 0.0 or args.cutoff > 1.0:
         print("Error: args.cutoff must be between 0 and 1, inclusive.")
         sys.exit()
+    init_ranks(args)
     _normalise(args)
     _tick("start")
     if args.cmash_results == "NONE":
@@ -293,7 +455,8 @@ def select_main(args=None):
     _tick("db_info read")
     organisms_to_include = run_cmash_and_cutoff(args, taxid2info)
     _tick("selection done")
-    make_db_and_dbinfo(args, organisms_to_include, taxid2info)
+    if not getattr(args, "_mlg_subset_written", False):
+        _on_rank0(lambda: make_db_and_dbinfo(args, organisms_to_include, taxid2info))
     _tick("subset files written")
     return organisms_to_include
 
