@@ -94,6 +94,11 @@ int mlg_ctx_streams(mlg_ctx* ctx, void** compute_stream, void** copy_stream);
 /* pinned host memory for callers that have no other way to get it */
 int mlg_host_alloc(void** out, uint64_t bytes);
 int mlg_host_free(void* p);
+/* the library's device memory on `device` (its caching pool): bytes held by live objects -- databases, queries, their
+ * buffers -- and bytes of freed blocks the pool keeps for reuse (given back to the device when an allocation fails, on
+ * mlg_ctx_destroy and after large builds).  Either pointer may be NULL.  For callers that check that nothing stays
+ * allocated from one query to the next; free device memory as the driver reports it also moves with the cache. */
+int mlg_device_memory(int device, uint64_t* live_bytes, uint64_t* cached_bytes);
 
 /* database: G genomes x n sketch slots of K-mers, queried at nk prefix lengths ks[] (ascending, ks[nk-1] <= K) */
 int mlg_db_from_keys(mlg_ctx* ctx, const uint64_t* keys /* host, G*n (hi,lo) pairs */, uint32_t G, uint32_t n,

@@ -78,6 +78,7 @@ SIGNATURES = {
     "mlg_ctx_streams": (C.c_int, [_vp, _pp, _pp]),
     "mlg_host_alloc": (C.c_int, [_pp, C.c_uint64]),
     "mlg_host_free": (C.c_int, [_vp]),
+    "mlg_device_memory": (C.c_int, [C.c_int, _u64p, _u64p]),
     "mlg_db_from_keys": (C.c_int, [_vp, _u64p, C.c_uint32, C.c_uint32, C.c_uint32, _u32p, C.c_uint32, _pp]),
     "mlg_db_from_keys_device": (C.c_int, [_vp, _u64p, C.c_uint32, C.c_uint32, C.c_uint32, _u32p, C.c_uint32, _pp]),
     "mlg_db_builder_create": (C.c_int, [_vp, C.c_uint32, C.c_uint32, C.c_uint32, _u32p, C.c_uint32, _pp]),

@@ -30,6 +30,14 @@ def pinned_array(nbytes: int) -> np.ndarray:
     return arr
 
 
+def device_memory(device: int = 0) -> dict:
+    """mlg_device_memory: {"live": bytes held by the library's live objects on `device`, "cached": freed blocks its pool
+    keeps for reuse}"""
+    live, cached = C.c_uint64(), C.c_uint64()
+    check(_lib.lib().mlg_device_memory(int(device), C.byref(live), C.byref(cached)))
+    return {"live": live.value, "cached": cached.value}
+
+
 class Context:
     """One GPU.  One process (host thread) per context."""
 

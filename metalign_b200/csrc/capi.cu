@@ -84,6 +84,17 @@ void mlg_pool_free(void* p) {
     }
     v.push_back({p, bytes});
 }
+MLG_API int mlg_device_memory(int device, uint64_t* live_bytes, uint64_t* cached_bytes) {
+    Pool& P = pool();
+    std::lock_guard<std::mutex> g(P.mu);
+    uint64_t live = 0, cached = 0;
+    for (const auto& kv : P.live) if (kv.second.first == device) live += kv.second.second;
+    auto it = P.free_blocks.find(device);
+    if (it != P.free_blocks.end()) for (const auto& b : it->second) cached += b.bytes;
+    if (live_bytes) *live_bytes = live;
+    if (cached_bytes) *cached_bytes = cached;
+    return MLG_OK;
+}
 void mlg_pool_trim(int device) {
     Pool& P = pool();
     std::vector<PoolBlock> blocks;

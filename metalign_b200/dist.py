@@ -331,6 +331,17 @@ def write_reads_kmc(query, prefix: str, min_count: int = 2, counter_max: int = 3
     return times
 
 
+def all_gather_rows(rows, group=None) -> list:
+    """Collective: every rank's list of rows (any picklable objects), joined in rank order, on every rank"""
+    import torch.distributed as dist
+    world, _rank = _world_rank(group)
+    if world == 1:
+        return list(rows)
+    every = [None] * world
+    dist.all_gather_object(every, list(rows), group=group)
+    return [r for part in every for r in part]
+
+
 def close_exchanges():
     for cur in _EXCHANGES.values():
         cur["ex"].close()

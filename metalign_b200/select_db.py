@@ -19,8 +19,11 @@ as a single-process run.  --threads is then per rank.
 from __future__ import annotations
 
 import argparse
+import collections
+import copy
 import gzip
 import os
+import re
 import shutil
 import sys
 import tempfile
@@ -160,11 +163,122 @@ def taxid_of(organism_name: str) -> str:
     return organism_name.split("taxid_")[1].split("_genomic.fna")[0].replace("_", ".")
 
 
+def open_reader(args, alloc=None, split=True):
+    """The native reader of args.reads (its worker count = --threads, KMC's -t in the reference): buffers allocated (pinned
+    by default), file mapped, parser threads started -- they cut the first batches at once, and later fill one buffer set
+    while the previous batch is on its way to the GPU.  Under torchrun with split (the one-file multi-rank mode, whose
+    ranks then exchange their counters) only this rank's byte range of the file; without split the whole file."""
+    from . import ingest
+    from .api import pinned_array
+    rank, world = ranks() if split else (0, 1)
+    # 2 M reads per batch: two buffer sets of ~110 MB of page-locked memory (0.7 ms per MiB to pin: with 4 M reads per batch
+    # the reader's set-up outlasted the database load it is meant to hide behind)
+    share = ingest.share_ranges(args.reads, world)[rank] if world > 1 else None
+    return ingest.PackedBatches(args.reads, args.input_type, reads_per_batch=2_000_000, alloc=alloc or pinned_array,
+                                threads=max(1, int(getattr(args, "threads", 4) or 4)), share=share)
+
+
+def _on_helper(fn):
+    """fn() started on a helper thread; the returned join() waits for it and gives (its result, its error)"""
+    import threading
+    box = {}
+
+    def run():
+        try:
+            box["value"] = fn()
+        except BaseException as e:  # noqa: BLE001
+            box["error"] = e
+    th = threading.Thread(target=run, daemon=True)
+    th.start()
+
+    def join():
+        th.join()
+        return box.get("value"), box.get("error")
+    return join
+
+
+def _close_all(*objs):
+    for obj in objs:
+        if obj is not None:
+            try:
+                obj.close()
+            except Exception:  # noqa: BLE001
+                pass
+
+
+def open_database(args, beside=None):
+    """The part of a run that does not depend on the sample: the context of args.device and the database args.db_file.
+    beside() (e.g. opening the reader) runs on a helper thread while this one reads the database file (both are C calls
+    that release the interpreter lock).  Returns (ctx, db, what beside() returned); if anything fails, what was opened is
+    closed again."""
+    from .api import Context, Database
+    ctx = db = side = None
+    try:
+        ctx = Context(args.device)
+        _tick("CUDA context")
+        join = _on_helper(beside) if beside is not None else (lambda: (None, None))
+        try:
+            db = Database.load(ctx, args.db_file)
+        finally:
+            side, side_err = join()
+        if side_err is not None:
+            raise side_err
+        return ctx, db, side
+    except BaseException:
+        _close_all(side, db, ctx)
+        raise
+
+
+def push_sample(args, db, reader, split=True):
+    """The per-sample GPU part up to the counters: a query on db, every batch of the reader pushed and probed.  -ci2
+    (select_db.py:50); the read k-mer table only for the reads_60mers database --keep_temp_files leaves behind.  Under
+    torchrun with split (a reader of this rank's byte range, open_reader) the read k-mers are counted in passes, because
+    share_read_kmers hands the reads around; without split only with --read_kmer_passes.  The query is closed again if a
+    push fails."""
+    _rank, world = ranks() if split else (0, 1)
+    query = db.query(ci_min=2, gate=args.gate, count_empty_in_den=True, read_kmers=bool(args.keep_temp_files),
+                     read_kmer_budget=args.read_kmer_budget, read_kmer_passes=args.read_kmer_passes or world > 1)
+    try:
+        for bases, nruns, off, n_reads in reader:
+            query.push_packed_nruns(bases, nruns if len(nruns) else None, off, n_reads)
+        query.sync()
+    except BaseException:
+        query.close()
+        raise
+    return query
+
+
+def write_sample_files(args, db, query, times):
+    """The per-sample GPU part after the pushes, on one GPU: the containment table as args.temp_dir/cmash_query_results.csv
+    (what the CMash subprocess writes, select_db.py:68-76) and, with --keep_temp_files, the intersection dump and the two KMC
+    databases.  A read k-mer table over --read_kmer_budget only skips reads_60mers, with a warning."""
+    from . import cmash_tail
+    from ._lib import MLG_ERR_NOMEM, MlgError
+    t0 = _now()
+    res = query.finish_sparse()                       # rows for the genomes with a hit: all the CSV can hold
+    times["finish_s"] = _now() - t0
+    _tick("containment table")
+    cmash_tail.write_results_csv_sparse(args.temp_dir + "cmash_query_results.csv", db.names, db.ks, res["genomes"], res["ci"],
+                                        0.0)          # '-c 0'
+    _tick("csv written")
+    if args.keep_temp_files:
+        # what kmc_dump and the FASTA rewrite leave in the temp dir (select_db.py:58-65): "<k-mer>\t<count>" lines
+        # and the ">seq" records CMash is given
+        query.dump_intersection(args.temp_dir + "60mers_intersection_dump", args.temp_dir + "60mers_intersection_dump.fa")
+        # the two KMC databases of select_db.py:50-56
+        query.write_intersection_kmc(args.temp_dir + "60mers_intersection", counter_max=3)
+        try:
+            query.write_reads_kmc(args.temp_dir + "reads_60mers", min_count=2, counter_max=3)
+        except MlgError as e:
+            if e.code != MLG_ERR_NOMEM:
+                raise
+            sys.stderr.write("select_db: reads_60mers.kmc_* not written: %s\n" % e)
+
+
 def run_kmc_steps(args):
     """Replaces kmc + kmc_tools intersect + kmc_dump (select_db.py:43-65): counts the canonical 60-mers of the
     reads that belong to the database sketch; the live query is parked on args for run_cmash_and_cutoff."""
     from . import ingest
-    from .api import Context, Database, pinned_array
     rank, world = ranks()
     times = args._mlg_times = {}
     t0 = _now()
@@ -175,42 +289,12 @@ def run_kmc_steps(args):
         import threading
         threading.Thread(target=lambda: __import__("pandas"), daemon=True).start()
         _tick("imports done")
-        ctx = Context(args.device)
-        _tick("CUDA context")
-        # the native reader (its worker count = --threads, KMC's -t in the reference) is set up -- pinned buffers, file
-        # mapped, parser threads started -- by a helper thread while this one reads the database file (both are C calls
-        # that release the interpreter lock); it then cuts the first batches while the database is still loading, and
-        # later fills one pinned buffer set while the previous batch is on its way to the GPU
-        box = {}
-
-        def open_reader():
-            try:
-                # 2 M reads per batch: two buffer sets of ~110 MB of page-locked memory (0.7 ms per MiB to pin: with 4 M reads
-                # per batch the reader's set-up outlasted the database load it is meant to hide behind)
-                share = ingest.share_ranges(args.reads, world)[rank] if world > 1 else None
-                box["reader"] = ingest.PackedBatches(args.reads, args.input_type, reads_per_batch=2_000_000, alloc=pinned_array,
-                                                     threads=max(1, int(getattr(args, "threads", 4) or 4)), share=share)
-            except BaseException as e:  # noqa: BLE001
-                box["error"] = e
-        th = threading.Thread(target=open_reader)
-        th.start()
-        try:
-            db = Database.load(ctx, args.db_file)
-        finally:
-            th.join()
-            reader = box.get("reader")
-        if "error" in box:
-            raise box["error"]
+        # the reader is set up while the database loads, and cuts the first batches before the load ends
+        ctx, db, reader = open_database(args, beside=lambda: open_reader(args))
         _tick("database loaded, reader started")
-        # -ci2 (select_db.py:50); the read k-mer table only for the reads_60mers database --keep_temp_files leaves behind
-        # (across ranks the read k-mers are only counted in passes: share_read_kmers hands the reads around)
-        query = db.query(ci_min=2, gate=args.gate, count_empty_in_den=True, read_kmers=bool(args.keep_temp_files),
-                         read_kmer_budget=args.read_kmer_budget, read_kmer_passes=args.read_kmer_passes or world > 1)
         times["open_s"] = _now() - t0
         t0 = _now()
-        for bases, nruns, off, n_reads in reader:
-            query.push_packed_nruns(bases, nruns if len(nruns) else None, off, n_reads)
-        query.sync()
+        query = push_sample(args, db, reader)
         times["push_s"] = _now() - t0
         _tick("reads pushed and probed")
         if world > 1:
@@ -241,12 +325,7 @@ def run_kmc_steps(args):
         if world > 1:
             from . import dist as mdist
             mdist.close_exchanges()
-        for obj in (reader, query, db, ctx):
-            if obj is not None:
-                try:
-                    obj.close()
-                except Exception:  # noqa: BLE001
-                    pass
+        _close_all(reader, query, db, ctx)
         raise err
     reader.close()
     _tick("reader closed")
@@ -257,31 +336,12 @@ def run_cmash_and_cutoff(args, taxid2info):
     """Replaces the CMash subprocess (select_db.py:68-76), then applies the cutoff and the one-strain-per-species
     rule exactly as select_db.py:80-96 does, reading the CSV back in file order."""
     if args.cmash_results == "NONE":
-        from . import cmash_tail, codec
-        from ._lib import MLG_ERR_NOMEM, MlgError
         ctx, db, query = args._mlg
         cmash_out = args.temp_dir + "cmash_query_results.csv"
         rank, world = ranks()
         if world > 1:
             return _gpu_files_ranks(args, taxid2info, cmash_out)
-        t0 = _now()
-        res = query.finish_sparse()                       # rows for the genomes with a hit: all the CSV can hold
-        args._mlg_times["finish_s"] = _now() - t0
-        _tick("containment table")
-        cmash_tail.write_results_csv_sparse(cmash_out, db.names, db.ks, res["genomes"], res["ci"], 0.0)      # '-c 0'
-        _tick("csv written")
-        if args.keep_temp_files:
-            # what kmc_dump and the FASTA rewrite leave in the temp dir (select_db.py:58-65): "<k-mer>\t<count>" lines
-            # and the ">seq" records CMash is given
-            query.dump_intersection(args.temp_dir + "60mers_intersection_dump", args.temp_dir + "60mers_intersection_dump.fa")
-            # the two KMC databases of select_db.py:50-56
-            query.write_intersection_kmc(args.temp_dir + "60mers_intersection", counter_max=3)
-            try:
-                query.write_reads_kmc(args.temp_dir + "reads_60mers", min_count=2, counter_max=3)
-            except MlgError as e:
-                if e.code != MLG_ERR_NOMEM:
-                    raise
-                sys.stderr.write("select_db: reads_60mers.kmc_* not written: %s\n" % e)
+        write_sample_files(args, db, query, args._mlg_times)
         if not getattr(args, "_mlg_leave_open", False):     # the command-line script exits right after: no point in freeing GBs first
             query.close(); db.close(); ctx.close()
         del args._mlg
@@ -459,6 +519,294 @@ def select_main(args=None):
         _on_rank0(lambda: make_db_and_dbinfo(args, organisms_to_include, taxid2info))
     _tick("subset files written")
     return organisms_to_include
+
+
+# ------------------------------------------------------------------ many samples against one database
+SUMMARY_NAME = "samples_summary.tsv"
+SUMMARY_HEADER = "sample_id\tstatus\tselected\tseconds\terror\n"
+SAMPLE_FILES = ("cmash_query_results.csv", "cmashed_db.fna", "subset_db_info.txt", "60mers_intersection_dump",
+                "60mers_intersection_dump.fa", "60mers_intersection.kmc_pre", "60mers_intersection.kmc_suf",
+                "reads_60mers.kmc_pre", "reads_60mers.kmc_suf")
+_SAFE_ID = re.compile(r"[A-Za-z0-9][A-Za-z0-9._-]{0,127}\Z")
+
+Sample = collections.namedtuple("Sample", "id reads input_type")
+# status "ok" or "failed"; organisms: the selection (None when failed); stages: seconds per stage of this sample
+SampleResult = collections.namedtuple("SampleResult", "id status organisms seconds error out_dir stages")
+
+
+class SampleSheetError(ValueError):
+    pass
+
+
+def read_sample_sheet(path):
+    """The samples of a sheet: one line per sample, `sample_id <TAB> reads_path [<TAB> fastq|fasta]` (blank lines and lines
+    starting with '#' are skipped).  Without the third column the type comes from the extension (ingest.input_type_of); a
+    relative reads path is taken from the sheet's directory.  Raises SampleSheetError naming the line for a wrong number of
+    columns, an id that is not a safe directory name, a duplicate id or an unknown type.  Whether the reads files exist is
+    not checked here: a missing one fails its own sample."""
+    from .ingest import input_type_of
+    base = os.path.dirname(os.path.abspath(path))
+    samples, first_line = [], {}
+    with open(path, "r") as fh:
+        for no, raw in enumerate(fh, 1):
+            line = raw.rstrip("\r\n")
+            if not line.strip() or line.startswith("#"):
+                continue
+            where = "%s, line %d" % (path, no)
+            cols = line.split("\t")
+            if len(cols) not in (2, 3) or not cols[1]:
+                raise SampleSheetError("%s: expected sample_id<TAB>reads_path[<TAB>fastq|fasta], got %d tab-separated "
+                                       "column(s)" % (where, len(cols)))
+            sid, reads = cols[0], cols[1]
+            if not _SAFE_ID.match(sid) or sid == SUMMARY_NAME:
+                raise SampleSheetError("%s: sample id %r is not a safe directory name (letters, digits, '.', '_', '-'; not "
+                                       "starting with '.' or '-'; at most 128 characters)" % (where, sid))
+            if sid in first_line:
+                raise SampleSheetError("%s: duplicate sample id %r (first on line %d)" % (where, sid, first_line[sid]))
+            kind = cols[2] if len(cols) == 3 else input_type_of(reads)
+            if kind not in ("fastq", "fasta"):
+                raise SampleSheetError("%s: unknown reads type %r (fastq or fasta)" % (where, cols[2]) if len(cols) == 3 else
+                                       "%s: the type of %r does not follow from its extension: add fastq or fasta as a third "
+                                       "column" % (where, reads))
+            first_line[sid] = no
+            samples.append(Sample(sid, reads if os.path.isabs(reads) else os.path.join(base, reads), kind))
+    return samples
+
+
+def rank_samples(n_samples, rank, world):
+    """the indices of the samples rank `rank` of `world` runs: i mod world == rank"""
+    return list(range(rank, n_samples, world))
+
+
+def format_summary(results):
+    """samples_summary.tsv: a header, then one line per sample -- id, ok / failed, organisms selected, seconds, error"""
+    lines = [SUMMARY_HEADER]
+    for r in results:
+        err = " ".join(str(r.error or "").split())            # one line, no tabs
+        lines.append("%s\t%s\t%d\t%.3f\t%s\n" % (r.id, r.status, len(r.organisms or ()), r.seconds, err))
+    return "".join(lines)
+
+
+def _is_device_error(e):
+    from ._lib import MlgError
+    return isinstance(e, MlgError) and e.code == -1           # MLG_ERR_CUDA: the device state is unknown
+
+
+class _NotRun(Exception):
+    pass
+
+
+def sample_reader(args, pool):
+    """the reader of one sample of a batch: the whole file whatever the torchrun world (a rank runs whole samples), in
+    buffers from `pool`"""
+    return open_reader(args, alloc=pool, split=False)
+
+
+def _remove_sample_files(sample_dir):
+    for name in SAMPLE_FILES:
+        try:
+            os.remove(os.path.join(sample_dir, name))
+        except OSError:
+            pass
+    try:
+        os.rmdir(sample_dir)
+    except OSError:
+        pass                                                  # not empty: files that are not this run's stay
+
+
+class SelectSession:
+    """One CUDA context, one loaded database, the parsed db_info and one pool of pinned reader buffers, kept for any
+    number of samples.  `run(samples, out_dir)` writes each sample's select_db.py files into out_dir/<sample_id>/.
+
+    Two threads: a GPU thread runs the per-sample GPU part (open the reader, push, finish, CSV, intersection and KMC files,
+    close the query and reader) sample after sample on the context's streams, and the calling thread applies the cutoff
+    and writes the subset FASTA and db_info (make_db_and_dbinfo).  So while sample i's subset files are written, sample
+    i + 1's reads are already read and probed; the GPU thread runs at most one sample ahead.  The next sample's reader is
+    opened while the current one finishes, in the buffers the closed reader gave back (ingest.BufferPool): pinned memory
+    stays at one reader's buffer sets.
+
+    A failing sample (an unreadable, truncated or corrupt reads file, a failed write, any library error but a device
+    error) fails alone: its query and reader are closed, its files removed, and the batch goes on.  A device error
+    (MLG_ERR_CUDA) ends the batch: the samples not yet run are reported as failed and no later run() starts any."""
+
+    def __init__(self, args):
+        """args: the flags of select_many (data and db_file resolved as _normalise resolves them)"""
+        from . import ingest
+        from .api import pinned_array
+        t0 = _now()
+        self.args = args
+        self.pool = ingest.BufferPool(pinned_array)
+        self.stopped = None          # the message of the device error that ended the batch
+        self.ctx, self.db, self.taxid2info = open_database(args, beside=lambda: read_dbinfo(args))
+        self.open_s = _now() - t0
+
+    def close(self):
+        _close_all(self.db, self.ctx)
+        self.db = self.ctx = None
+        self.pool.clear()
+
+    def _sample_args(self, s, out_dir):
+        a = copy.copy(self.args)
+        a.reads, a.input_type, a.cmash_results = s.reads, s.input_type, "NONE"
+        a.temp_dir = os.path.join(out_dir, s.id) + "/"
+        a.db, a.dbinfo_out = a.temp_dir + "cmashed_db.fna", a.temp_dir + "subset_db_info.txt"
+        return a
+
+    def _gpu_part(self, a, reader_join, open_next, stages):
+        """one sample's GPU part; open_next() is called once this sample's reader is closed"""
+        query = reader = None
+        t0 = _now()
+        try:
+            reader, err = reader_join()
+            if err is not None:
+                raise err
+            os.makedirs(a.temp_dir, exist_ok=True)
+            query = push_sample(a, self.db, reader, split=False)
+            reader.close()
+            reader = None
+            open_next()                              # its parser threads cut the first batches while this sample finishes
+            stages["push_s"] = _now() - t0
+            t0 = _now()
+            write_sample_files(a, self.db, query, {})
+            stages["gpu_files_s"] = _now() - t0
+        finally:
+            _close_all(reader, query)
+
+    def run(self, samples, out_dir):
+        """-> [SampleResult] in the order of `samples`"""
+        import queue
+        import threading
+        sargs = [self._sample_args(s, out_dir) for s in samples]
+        handoff = queue.Queue()
+        ahead = threading.Semaphore(2)               # the sample whose subset files are being written + one GPU part ahead
+
+        def reader_of(i):
+            if i >= len(samples) or self.stopped is not None:
+                return lambda: (None, None)
+            return _on_helper(lambda: sample_reader(sargs[i], self.pool))
+
+        def gpu_thread():
+            # every sample is handed over, with its error if anything failed: the calling thread waits for each one
+            join = None
+            for i, a in enumerate(sargs):
+                nxt, stages, err = [], {}, None
+                try:
+                    ahead.acquire()
+                    if join is None:
+                        join = reader_of(i)
+
+                    def open_next():
+                        nxt.append(reader_of(i + 1))
+                    if self.stopped is not None:
+                        _close_all(join()[0])
+                        err = _NotRun("not run: " + self.stopped)
+                    else:
+                        self._gpu_part(a, join, open_next, stages)
+                except BaseException as e:  # noqa: BLE001
+                    err = err or e
+                    if _is_device_error(e):
+                        self.stopped = "the batch stopped after a device error on sample %s: %s" % (samples[i].id, e)
+                join = nxt[0] if nxt else None       # None: the next sample opens its reader itself
+                handoff.put((i, stages, err))
+
+        th = threading.Thread(target=gpu_thread, daemon=True)
+        th.start()
+        results = []
+        for _ in samples:
+            i, stages, err = handoff.get()
+            a = sargs[i]
+            chosen = None
+            if err is None:
+                t0 = _now()
+                try:
+                    chosen = _select(a, self.taxid2info, a.temp_dir + "cmash_query_results.csv")
+                    make_db_and_dbinfo(a, chosen, self.taxid2info)
+                except Exception as e:  # noqa: BLE001
+                    err = e
+                stages["subset_s"] = _now() - t0
+            ahead.release()
+            seconds = sum(stages.values())
+            if err is not None:
+                _remove_sample_files(a.temp_dir)
+                msg = str(err) if isinstance(err, _NotRun) else "%s: %s" % (type(err).__name__, err)
+                results.append(SampleResult(samples[i].id, "failed", None, seconds, msg, a.temp_dir, stages))
+            else:
+                results.append(SampleResult(samples[i].id, "ok", chosen, seconds, "", a.temp_dir, stages))
+        th.join()
+        return results
+
+
+def select_many_parseargs(argv=None):
+    p = argparse.ArgumentParser(description="select_db.py for many samples against one database: one CUDA context and one "
+                                            "loaded database per GPU, each sample's files in out_dir/<sample_id>/.")
+    p.add_argument("sample_sheet", help="one line per sample: sample_id<TAB>reads_path[<TAB>fastq|fasta]")
+    p.add_argument("data", help="data/ directory (database, db_info.txt, organism_files/)")
+    p.add_argument("--out_dir", default="AUTO", help="where the sample directories and %s go (default: a new temporary "
+                                                     "directory under data/)" % SUMMARY_NAME)
+    p.add_argument("--cutoff", type=float, default=0.01, help="containment cutoff at the largest k (default 0.01)")
+    p.add_argument("--db_dir", default="AUTO", help="directory holding the organism files of the full database")
+    p.add_argument("--dbinfo_in", default="AUTO", help="db_info file of the full database (default data/db_info.txt)")
+    p.add_argument("--keep_temp_files", action="store_true", help="also write each sample's intersection dump and KMC databases")
+    p.add_argument("--strain_level", action="store_true", help="keep every strain above the cutoff (default: one per species)")
+    p.add_argument("--threads", type=int, default=4, help="reader threads (per rank under torchrun)")
+    p.add_argument("--db_file", default="AUTO", help="native database file (default data/%s)" % DB_BASENAME)
+    p.add_argument("--gate", default="exact", choices=["exact", "none"], help="smallest-k prefilter model (see DESIGN.md)")
+    p.add_argument("--device", type=int, default=0, help="CUDA device")
+    p.add_argument("--read_kmer_budget", type=int, default=0, help="as select_db.py --read_kmer_budget, per sample")
+    p.add_argument("--read_kmer_passes", action="store_true", help="as select_db.py --read_kmer_passes")
+    return p.parse_args(argv)
+
+
+def normalise_many(args):
+    """the AUTO defaults of select_many's flags, as _normalise resolves them for select_db; out_dir created"""
+    if not args.data.endswith("/"):
+        args.data += "/"
+    for name, value in (("db_dir", args.data + "organism_files/"), ("dbinfo_in", args.data + "db_info.txt"),
+                        ("db_file", args.data + DB_BASENAME)):
+        if getattr(args, name) == "AUTO":
+            setattr(args, name, value)
+    if not args.db_dir.endswith("/"):
+        args.db_dir += "/"
+    if args.out_dir == "AUTO":
+        args.out_dir = shared_mkdtemp(args.data)
+    os.makedirs(args.out_dir, exist_ok=True)
+
+
+def select_many(sample_sheet, args):
+    """select_db.py for every sample of a sample sheet (read_sample_sheet) against one database: each sample's files in
+    args.out_dir/<sample_id>/ -- byte for byte what `select_db.py <reads> <data> --temp_dir out_dir/<sample_id>/` with the
+    same flags writes -- and out_dir/samples_summary.tsv (format_summary).  Returns a SampleResult per sample in sheet
+    order; a caller can map and profile each ok sample from its out_dir.
+
+    The sheet is checked before any GPU work.  Under torchrun (WORLD_SIZE > 1) rank r runs the samples i with
+    i mod world == r on its LOCAL_RANK GPU (its own context and database, no exchange); every rank gets every result, and
+    rank 0 writes the summary."""
+    if args.cutoff < 0.0 or args.cutoff > 1.0:
+        raise ValueError("cutoff must be between 0 and 1, inclusive")
+    samples = read_sample_sheet(sample_sheet)
+    init_ranks(args)
+    rank, world = ranks()
+    normalise_many(args)
+    mine = [samples[i] for i in rank_samples(len(samples), rank, world)]
+    session = None
+    try:
+        session = SelectSession(args)
+        args._mlg_open_s = session.open_s
+        results = session.run(mine, args.out_dir)
+    except Exception as e:  # noqa: BLE001  (no context or database: none of this rank's samples runs)
+        msg = "not run: the database could not be opened on this GPU: %s: %s" % (type(e).__name__, e)
+        results = [SampleResult(s.id, "failed", None, 0.0, msg, os.path.join(args.out_dir, s.id) + "/", {}) for s in mine]
+    finally:
+        if session is not None:
+            session.close()
+    if world > 1:
+        from . import dist as mdist
+        order = {s.id: i for i, s in enumerate(samples)}
+        results = sorted(mdist.all_gather_rows(results), key=lambda r: order[r.id])
+    if rank == 0:
+        with open(os.path.join(args.out_dir, SUMMARY_NAME), "w") as f:
+            f.write(format_summary(results))
+    return results
 
 
 if __name__ == "__main__":

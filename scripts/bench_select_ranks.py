@@ -64,10 +64,22 @@ def _chunk_job(job):
 
 
 def prepare(d, nreads):
-    """reads.fq and reads.fq.gz (by host workers, before this process touches the GPU), then data/: the default-scale
-    database file, db_info.txt and one tiny organism file per genome"""
-    import gzip
+    """reads.fq and reads.fq.gz (by host workers, before this process touches the GPU), then data/ (write_data_dir)"""
     from multiprocessing import Pool
+    import bench
+    G = bench.workload_plan("weak", 1, 0)[0]
+    jobs = [(G, r0, min(CHUNK, nreads - r0)) for r0 in range(0, nreads, CHUNK)]
+    with open(os.path.join(d, "reads.fq"), "wb") as fq, open(os.path.join(d, "reads.fq.gz"), "wb") as gz, Pool(os.cpu_count()) as pool:
+        for text, members in pool.imap(_chunk_job, jobs):
+            fq.write(text)
+            gz.write(members)
+        gz.write(_bgzf_member(b""))
+    write_data_dir(d)
+
+
+def write_data_dir(d):
+    """d/data/: bench.py's default-scale database built to a file, db_info.txt and one tiny organism file per genome"""
+    import gzip
     import torch
     import bench
     import synth
@@ -78,12 +90,6 @@ def prepare(d, nreads):
     data = os.path.join(d, "data")
     os.makedirs(os.path.join(data, "organism_files"), exist_ok=True)
     names = ["taxid_%d_genomic.fna.gz" % g for g in range(G)]
-    jobs = [(G, r0, min(CHUNK, nreads - r0)) for r0 in range(0, nreads, CHUNK)]
-    with open(os.path.join(d, "reads.fq"), "wb") as fq, open(os.path.join(d, "reads.fq.gz"), "wb") as gz, Pool(os.cpu_count()) as pool:
-        for text, members in pool.imap(_chunk_job, jobs):
-            fq.write(text)
-            gz.write(members)
-        gz.write(_bgzf_member(b""))
     with Context(0) as ctx:
         d_keys = torch.empty(G * p.n * 2, dtype=torch.int64, device="cuda")
         assert synth.cuda_lib().syn_cuda_gen_sketch_keys(C.byref(p), d_keys.data_ptr(), None) == 0
