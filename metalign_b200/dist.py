@@ -224,8 +224,8 @@ def _world_rank(group):
     return 1, 0
 
 
-def _flag_min(ok: bool, device: int, group) -> bool:
-    """every rank's ok, and-ed over the ranks"""
+def all_ok(ok: bool, device: int = 0, group=None) -> bool:
+    """Collective: every rank's ok, and-ed over the ranks (ok itself without a process group)"""
     import torch
     import torch.distributed as dist
     if _world_rank(group)[0] == 1:
@@ -270,7 +270,7 @@ def share_read_kmers(query, device: int = 0, group=None) -> None:
             recv = torch.empty(max(sizes[r] for r in range(world) if r != rank), dtype=torch.uint8, device=dev)
     except Exception as e:  # noqa: BLE001
         err = e
-    if not _flag_min(err is None, device, group):
+    if not all_ok(err is None, device, group):
         raise err or RuntimeError("read k-mer exchange: a rank could not allocate its receive buffer")
     try:
         with torch.cuda.stream(comp):
@@ -282,7 +282,7 @@ def share_read_kmers(query, device: int = 0, group=None) -> None:
                         query.add_read_kmer_archive(buf.data_ptr(), sizes[src])
                     except Exception as e:  # noqa: BLE001
                         err = e
-        ok = _flag_min(err is None, device, group)
+        ok = all_ok(err is None, device, group)
     finally:
         comp.synchronize()
         del recv
@@ -309,7 +309,7 @@ def write_reads_kmc(query, prefix: str, min_count: int = 2, counter_max: int = 3
         err = e
     times = dict(part_s=time.perf_counter() - t0, concat_s=0.0)
     try:
-        written = _flag_min(err is None, device, group)
+        written = all_ok(err is None, device, group)
         if rank == 0 and written:
             t0 = time.perf_counter()
             try:
@@ -317,7 +317,7 @@ def write_reads_kmc(query, prefix: str, min_count: int = 2, counter_max: int = 3
             except Exception as e:  # noqa: BLE001
                 err = e
             times["concat_s"] = time.perf_counter() - t0
-        joined = _flag_min(err is None, device, group) and written
+        joined = all_ok(err is None, device, group) and written
     finally:
         for ext in (".kmc_pre", ".kmc_suf"):
             try:

@@ -48,10 +48,10 @@ def metalign_parseargs(argv=None):
 def main(argv=None):
     args = metalign_parseargs(argv)
     select.init_ranks(args)
-    if not args.data.endswith("/"):
-        args.data += "/"
+    rank, world = select.ranks()
+    select.resolve_data(args)
     if args.temp_dir == "AUTO/":
-        args.temp_dir = select.shared_mkdtemp(args.data)
+        args.temp_dir = select.shared_mkdtemp(args.data, rank, world)
     if not args.temp_dir.endswith("/"):
         args.temp_dir += "/"
     if args.sensitive and args.precise:
@@ -69,7 +69,7 @@ def main(argv=None):
 
     select.select_main(args)
     mapper = None
-    if select.ranks()[0] != 0:
+    if rank != 0:
         return
     if not args.select_only:
         try:

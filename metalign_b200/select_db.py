@@ -15,6 +15,10 @@ Under torchrun (WORLD_SIZE > 1) every rank drives the GPU of its LOCAL_RANK: it 
 file (ingest.share_ranges), the ranks sum their counters in one exchange (dist.reduce_query, each rank's counters clamped
 to counter_max so that the intersection counts are those of one GPU), and rank 0 alone writes the files -- the same bytes
 as a single-process run.  --threads is then per rank.
+
+A single process, the ranks of a torchrun launch and the samples of a batch (select_many) share one pipeline, whose pieces
+are told their rank and world: open_database + open_reader, push_sample, exchange (world > 1), write_gpu_files,
+run_cmash_and_cutoff.
 """
 from __future__ import annotations
 
@@ -24,13 +28,16 @@ import copy
 import gzip
 import os
 import re
-import shutil
 import sys
 import tempfile
 
 DB_BASENAME = "cmash_db_n1000_k60.mlgdb"
 HEADER_LINES = ("Accesion\tLength\tTaxID\tLineage\tTaxID_Lineage\n",          # sic: spelling of the reference, select_db.py:109
                 "Unmapped\t0\tUnmapped\t|||||||Unmapped\t|||||||Unmapped\n")
+# the files a run writes (output_paths); the CSV and the subset files always, the others with --keep_temp_files
+OUTPUT_NAMES = ("cmash_query_results.csv", "cmashed_db.fna", "subset_db_info.txt", "60mers_intersection_dump",
+                "60mers_intersection_dump.fa", "60mers_intersection.kmc_pre", "60mers_intersection.kmc_suf",
+                "reads_60mers.kmc_pre", "reads_60mers.kmc_suf")
 
 
 _T0 = None
@@ -73,9 +80,8 @@ def init_ranks(args):
     mdist.bind_to_gpu_numa(local)
 
 
-def shared_mkdtemp(prefix):
+def shared_mkdtemp(prefix, rank=0, world=1):
     """tempfile.mkdtemp on rank 0, the same path on every rank"""
-    rank, world = ranks()
     if world == 1:
         return tempfile.mkdtemp(prefix=prefix)
     import torch.distributed as tdist
@@ -84,9 +90,8 @@ def shared_mkdtemp(prefix):
     return box[0]
 
 
-def _on_rank0(fn):
+def _on_rank0(fn, rank, world):
     """fn() on rank 0 alone; its result, or its failure, reaches every rank"""
-    rank, world = ranks()
     if world == 1:
         return fn()
     import torch.distributed as tdist
@@ -102,30 +107,26 @@ def _on_rank0(fn):
     return box[0]
 
 
-def _all_ok(err, args):
-    """collective: raise on every rank if any rank has an error (its own error where it has one)"""
-    from . import dist as mdist
-    if not mdist._flag_min(err is None, args.device, None):
+def _all_ok(err, device, world):
+    """raise if this rank has an error (err) or, collectively when world > 1, any other rank has: this rank's own error
+    where it has one"""
+    ok = err is None
+    if world > 1:
+        from . import dist as mdist
+        ok = mdist.all_ok(ok, device)
+    if not ok:
         raise err if err is not None else RuntimeError("select_db: another rank failed")
 
 
-def select_parseargs(argv=None):
-    p = argparse.ArgumentParser(description="Score every database genome against the reads (containment min-hash, "
-                                            "k=30..60) and write the reduced database to align to.")
-    p.add_argument("reads", help="reads file (FASTA/FASTQ, optionally .gz)")
-    p.add_argument("data", help="data/ directory (database, db_info.txt, organism_files/)")
-    p.add_argument("--cmash_results", default="NONE", help="reuse an existing query-results CSV; skips the GPU stage")
+def _add_common_flags(p):
+    """the flags of select_db.py that are not tied to one reads file, which select_many.py takes as well"""
     p.add_argument("--cutoff", type=float, default=0.01, help="containment cutoff at the largest k (default 0.01)")
-    p.add_argument("--db", default="AUTO", help="where to write the subset FASTA (default temp_dir/cmashed_db.fna)")
     p.add_argument("--db_dir", default="AUTO", help="directory holding the organism files of the full database")
     p.add_argument("--dbinfo_in", default="AUTO", help="db_info file of the full database (default data/db_info.txt)")
-    p.add_argument("--dbinfo_out", default="AUTO", help="where to write the subset db_info (default temp_dir/subset_db_info.txt)")
-    p.add_argument("--input_type", default="AUTO", choices=["fastq", "fasta", "AUTO"], help="reads format (default: by extension)")
     p.add_argument("--keep_temp_files", action="store_true",
                    help="keep the intermediate files the reference keeps: the KMC databases of the reads (reads_60mers, "
                         "-ci2 -cs3) and of the intersection (60mers_intersection), and the intersection dump")
     p.add_argument("--strain_level", action="store_true", help="keep every strain above the cutoff (default: one per species)")
-    p.add_argument("--temp_dir", default="AUTO/", help="directory for intermediate files")
     p.add_argument("--threads", type=int, default=4, help="reader threads (per rank under torchrun; KMC threads in the reference)")
     # additions
     p.add_argument("--db_file", default="AUTO", help="native database file (default data/%s)" % DB_BASENAME)
@@ -138,6 +139,19 @@ def select_parseargs(argv=None):
                    help="with --keep_temp_files: count the k-mers behind reads_60mers in key-range passes over a GPU copy of "
                         "the reads, for read sets whose table would not fit in one GPU; --read_kmer_budget then caps that "
                         "copy plus one pass, and only reads that do not fit themselves skip the database")
+
+
+def select_parseargs(argv=None):
+    p = argparse.ArgumentParser(description="Score every database genome against the reads (containment min-hash, "
+                                            "k=30..60) and write the reduced database to align to.")
+    p.add_argument("reads", help="reads file (FASTA/FASTQ, optionally .gz)")
+    p.add_argument("data", help="data/ directory (database, db_info.txt, organism_files/)")
+    p.add_argument("--cmash_results", default="NONE", help="reuse an existing query-results CSV; skips the GPU stage")
+    p.add_argument("--db", default="AUTO", help="where to write the subset FASTA (default temp_dir/cmashed_db.fna)")
+    p.add_argument("--dbinfo_out", default="AUTO", help="where to write the subset db_info (default temp_dir/subset_db_info.txt)")
+    p.add_argument("--input_type", default="AUTO", choices=["fastq", "fasta", "AUTO"], help="reads format (default: by extension)")
+    p.add_argument("--temp_dir", default="AUTO/", help="directory for intermediate files")
+    _add_common_flags(p)
     return p.parse_args(argv)
 
 
@@ -163,14 +177,28 @@ def taxid_of(organism_name: str) -> str:
     return organism_name.split("taxid_")[1].split("_genomic.fna")[0].replace("_", ".")
 
 
-def open_reader(args, alloc=None, split=True):
+def output_paths(args):
+    """the paths of the files a run writes (OUTPUT_NAMES): in args.temp_dir, the subset files where --db and --dbinfo_out
+    put them"""
+    placed = {"cmashed_db.fna": args.db, "subset_db_info.txt": args.dbinfo_out}
+    return [placed.get(name, args.temp_dir + name) for name in OUTPUT_NAMES]
+
+
+def _remove(paths):
+    for path in paths:
+        try:
+            os.remove(path)
+        except OSError:
+            pass
+
+
+def open_reader(args, rank=0, world=1, alloc=None):
     """The native reader of args.reads (its worker count = --threads, KMC's -t in the reference): buffers allocated (pinned
     by default), file mapped, parser threads started -- they cut the first batches at once, and later fill one buffer set
-    while the previous batch is on its way to the GPU.  Under torchrun with split (the one-file multi-rank mode, whose
-    ranks then exchange their counters) only this rank's byte range of the file; without split the whole file."""
+    while the previous batch is on its way to the GPU.  With world > 1 (one reads file split over the ranks, which then
+    exchange their counters) only rank's byte range of the file; else the whole file."""
     from . import ingest
     from .api import pinned_array
-    rank, world = ranks() if split else (0, 1)
     # 2 M reads per batch: two buffer sets of ~110 MB of page-locked memory (0.7 ms per MiB to pin: with 4 M reads per batch
     # the reader's set-up outlasted the database load it is meant to hide behind)
     share = ingest.share_ranges(args.reads, world)[rank] if world > 1 else None
@@ -206,6 +234,15 @@ def _close_all(*objs):
                 pass
 
 
+def _close_gpu(world, query, db, ctx):
+    """the query and the database, the exchanges of dist (world > 1), then the context they live in"""
+    _close_all(query, db)
+    if world > 1:
+        from . import dist as mdist
+        mdist.close_exchanges()
+    _close_all(ctx)
+
+
 def open_database(args, beside=None):
     """The part of a run that does not depend on the sample: the context of args.device and the database args.db_file.
     beside() (e.g. opening the reader) runs on a helper thread while this one reads the database file (both are C calls
@@ -229,13 +266,12 @@ def open_database(args, beside=None):
         raise
 
 
-def push_sample(args, db, reader, split=True):
+def push_sample(args, db, reader, world=1):
     """The per-sample GPU part up to the counters: a query on db, every batch of the reader pushed and probed.  -ci2
-    (select_db.py:50); the read k-mer table only for the reads_60mers database --keep_temp_files leaves behind.  Under
-    torchrun with split (a reader of this rank's byte range, open_reader) the read k-mers are counted in passes, because
-    share_read_kmers hands the reads around; without split only with --read_kmer_passes.  The query is closed again if a
-    push fails."""
-    _rank, world = ranks() if split else (0, 1)
+    (select_db.py:50); the read k-mer table only for the reads_60mers database --keep_temp_files leaves behind.  With
+    world > 1 (a reader of one rank's byte range, open_reader) the read k-mers are counted in passes, because
+    share_read_kmers hands the reads around; else only with --read_kmer_passes.  The query is closed again if a push
+    fails."""
     query = db.query(ci_min=2, gate=args.gate, count_empty_in_den=True, read_kmers=bool(args.keep_temp_files),
                      read_kmer_budget=args.read_kmer_budget, read_kmer_passes=args.read_kmer_passes or world > 1)
     try:
@@ -248,157 +284,115 @@ def push_sample(args, db, reader, split=True):
     return query
 
 
-def write_sample_files(args, db, query, times):
-    """The per-sample GPU part after the pushes, on one GPU: the containment table as args.temp_dir/cmash_query_results.csv
-    (what the CMash subprocess writes, select_db.py:68-76) and, with --keep_temp_files, the intersection dump and the two KMC
-    databases.  A read k-mer table over --read_kmer_budget only skips reads_60mers, with a warning."""
-    from . import cmash_tail
-    from ._lib import MLG_ERR_NOMEM, MlgError
-    t0 = _now()
-    res = query.finish_sparse()                       # rows for the genomes with a hit: all the CSV can hold
-    times["finish_s"] = _now() - t0
-    _tick("containment table")
-    cmash_tail.write_results_csv_sparse(args.temp_dir + "cmash_query_results.csv", db.names, db.ks, res["genomes"], res["ci"],
-                                        0.0)          # '-c 0'
-    _tick("csv written")
-    if args.keep_temp_files:
-        # what kmc_dump and the FASTA rewrite leave in the temp dir (select_db.py:58-65): "<k-mer>\t<count>" lines
-        # and the ">seq" records CMash is given
-        query.dump_intersection(args.temp_dir + "60mers_intersection_dump", args.temp_dir + "60mers_intersection_dump.fa")
-        # the two KMC databases of select_db.py:50-56
-        query.write_intersection_kmc(args.temp_dir + "60mers_intersection", counter_max=3)
-        try:
-            query.write_reads_kmc(args.temp_dir + "reads_60mers", min_count=2, counter_max=3)
-        except MlgError as e:
-            if e.code != MLG_ERR_NOMEM:
-                raise
-            sys.stderr.write("select_db: reads_60mers.kmc_* not written: %s\n" % e)
-
-
-def run_kmc_steps(args):
-    """Replaces kmc + kmc_tools intersect + kmc_dump (select_db.py:43-65): counts the canonical 60-mers of the
-    reads that belong to the database sketch; the live query is parked on args for run_cmash_and_cutoff."""
+def exchange(args, query, share_info, err, world):
+    """Collective, world > 1, after every rank's pushes (err: this rank's failure so far, or None): every rank learns
+    whether every other rank got this far, and checks the FASTQ phases of all shares (share_info: this rank's reader's);
+    then the ranks hand their reads around for reads_60mers (--keep_temp_files) and sum their counters."""
+    import torch.distributed as tdist
+    from . import dist as mdist
     from . import ingest
-    rank, world = ranks()
-    times = args._mlg_times = {}
-    t0 = _now()
-    ctx = db = query = reader = None
+    _all_ok(err, args.device, world)
+    infos = [None] * world
+    tdist.all_gather_object(infos, share_info)
+    ingest.check_share_phases(infos, args.input_type)
+    if args.keep_temp_files:
+        mdist.share_read_kmers(query, args.device)
+    mdist.reduce_query(query, args.device, clamp=3)          # -cs3: the intersection counts of one GPU
+    query.sync()
+
+
+def write_gpu_files(args, db, query, rank, world, stages):
+    """The per-sample GPU part after the pushes (and the exchange): the containment table as
+    args.temp_dir/cmash_query_results.csv (what the CMash subprocess writes, select_db.py:68-76) and, with
+    --keep_temp_files, the intersection dump and the two KMC databases.  Every rank finishes its query (identical on every
+    rank after the exchange); rank 0 writes the CSV and the intersection files; with world > 1 a failure on any rank
+    raises on every rank, and the ranks join reads_60mers (dist.write_reads_kmc).  On one GPU a read k-mer table over
+    --read_kmer_budget only skips reads_60mers, with a warning."""
+    from . import cmash_tail
     err = None
+    try:
+        t0 = _now()
+        res = query.finish_sparse()                   # rows for the genomes with a hit: all the CSV can hold
+        stages["finish_s"] = _now() - t0
+        _tick("containment table")
+        if rank == 0:
+            cmash_tail.write_results_csv_sparse(args.temp_dir + "cmash_query_results.csv", db.names, db.ks, res["genomes"],
+                                                res["ci"], 0.0)          # '-c 0'
+            _tick("csv written")
+            if args.keep_temp_files:
+                # what kmc_dump and the FASTA rewrite leave in the temp dir (select_db.py:58-65): "<k-mer>\t<count>" lines
+                # and the ">seq" records CMash is given; then the intersection database of select_db.py:53-56
+                query.dump_intersection(args.temp_dir + "60mers_intersection_dump",
+                                        args.temp_dir + "60mers_intersection_dump.fa")
+                query.write_intersection_kmc(args.temp_dir + "60mers_intersection", counter_max=3)
+    except Exception as e:  # noqa: BLE001  (with world > 1 every rank has to take part in the check below)
+        err = e
+    _all_ok(err, args.device, world)
+    if not args.keep_temp_files:
+        return
+    # the reads database of select_db.py:50-52
+    prefix = args.temp_dir + "reads_60mers"
+    if world > 1:
+        from . import dist as mdist
+        mdist.write_reads_kmc(query, prefix, 2, 3, args.device)
+        return
+    from ._lib import MLG_ERR_NOMEM, MlgError
+    try:
+        query.write_reads_kmc(prefix, min_count=2, counter_max=3)
+    except MlgError as e:
+        if e.code != MLG_ERR_NOMEM:
+            raise
+        sys.stderr.write("select_db: reads_60mers.kmc_* not written: %s\n" % e)
+
+
+def run_kmc_steps(args, rank, world, stages):
+    """Replaces kmc + kmc_tools intersect + kmc_dump (select_db.py:43-65): counts the canonical 60-mers of the
+    reads that belong to the database sketch.  Returns (ctx, db, query) after the pushes and, with world > 1, the
+    exchange; if anything fails, on any rank, what was opened is closed before the error travels on."""
+    t0 = _now()
+    ctx = db = query = reader = share_info = err = None
     try:
         # pandas (the CSV tail) takes a good part of a second to import: do it while the GPU works
         import threading
         threading.Thread(target=lambda: __import__("pandas"), daemon=True).start()
         _tick("imports done")
         # the reader is set up while the database loads, and cuts the first batches before the load ends
-        ctx, db, reader = open_database(args, beside=lambda: open_reader(args))
+        ctx, db, reader = open_database(args, beside=lambda: open_reader(args, rank, world))
         _tick("database loaded, reader started")
-        times["open_s"] = _now() - t0
+        stages["open_s"] = _now() - t0
         t0 = _now()
-        query = push_sample(args, db, reader)
-        times["push_s"] = _now() - t0
+        query = push_sample(args, db, reader, world)
+        stages["push_s"] = _now() - t0
         _tick("reads pushed and probed")
         if world > 1:
-            info = reader.share_info()
-    except BaseException as e:  # noqa: BLE001
+            share_info = reader.share_info()
+    except BaseException as e:  # noqa: BLE001  (with world > 1 every rank has to reach the exchange's check)
         err = e
-    if world > 1:
-        # every rank learns whether every other rank got this far, and every rank checks the FASTQ phases of all shares
-        import torch.distributed as tdist
-        try:
-            _all_ok(err, args)
-            infos = [None] * world
-            tdist.all_gather_object(infos, info)
-            ingest.check_share_phases(infos, args.input_type)
-            t0 = _now()
-            from . import dist as mdist
-            if args.keep_temp_files:
-                mdist.share_read_kmers(query, args.device)
-            mdist.reduce_query(query, args.device, clamp=3)          # -cs3: the intersection counts of one GPU
-            query.sync()
-            times["exchange_s"] = _now() - t0
-            _tick("exchange done")
-        except BaseException as e:  # noqa: BLE001
-            err = err or e
-    if err is not None:
-        # a corrupt reads file, a failed push: give the device and pinned memory back before the error travels on
-        # (a caller looping over samples would otherwise accumulate them)
+    try:
         if world > 1:
-            from . import dist as mdist
-            mdist.close_exchanges()
-        _close_all(reader, query, db, ctx)
-        raise err
+            t0 = _now()
+            exchange(args, query, share_info, err, world)
+            stages["exchange_s"] = _now() - t0
+            _tick("exchange done")
+        elif err is not None:
+            raise err
+    except BaseException:
+        # a corrupt reads file, a failed push: give the device and pinned memory back before the error travels on
+        _close_all(reader)
+        _close_gpu(world, query, db, ctx)
+        raise
     reader.close()
     _tick("reader closed")
-    args._mlg = (ctx, db, query)
+    return ctx, db, query
 
 
-def run_cmash_and_cutoff(args, taxid2info):
-    """Replaces the CMash subprocess (select_db.py:68-76), then applies the cutoff and the one-strain-per-species
-    rule exactly as select_db.py:80-96 does, reading the CSV back in file order."""
-    if args.cmash_results == "NONE":
-        ctx, db, query = args._mlg
-        cmash_out = args.temp_dir + "cmash_query_results.csv"
-        rank, world = ranks()
-        if world > 1:
-            return _gpu_files_ranks(args, taxid2info, cmash_out)
-        write_sample_files(args, db, query, args._mlg_times)
-        if not getattr(args, "_mlg_leave_open", False):     # the command-line script exits right after: no point in freeing GBs first
-            query.close(); db.close(); ctx.close()
-        del args._mlg
-        _tick("GPU objects closed")
-    else:
-        cmash_out = args.cmash_results
-    return _select(args, taxid2info, cmash_out)
-
-
-def _gpu_files_ranks(args, taxid2info, cmash_out):
-    """run_cmash_and_cutoff of a torchrun launch, after the exchange: every rank finishes its query (identical on every
-    rank), rank 0 writes the CSV and the intersection files, the ranks join reads_60mers (dist.write_reads_kmc), and rank 0
-    selects and hands the selection to every rank.  A failure anywhere raises on every rank, and rank 0 removes the files
-    of this stage."""
-    import torch.distributed as tdist
-    from . import cmash_tail
-    from . import dist as mdist
-    rank, _world = ranks()
-    ctx, db, query = args._mlg
-    del args._mlg
-    times = args._mlg_times
-    written = [cmash_out, args.temp_dir + "60mers_intersection_dump", args.temp_dir + "60mers_intersection_dump.fa", args.db,
-               args.dbinfo_out] + [args.temp_dir + p + e for p in ("60mers_intersection", "reads_60mers") for e in (".kmc_pre", ".kmc_suf")]
-    err = None
-    try:
-        try:
-            t0 = _now()
-            res = query.finish_sparse()
-            times["finish_s"] = _now() - t0
-            if rank == 0:
-                cmash_tail.write_results_csv_sparse(cmash_out, db.names, db.ks, res["genomes"], res["ci"], 0.0)
-                if args.keep_temp_files:
-                    query.dump_intersection(written[1], written[2])
-                    query.write_intersection_kmc(args.temp_dir + "60mers_intersection", counter_max=3)
-        except Exception as e:  # noqa: BLE001  (every rank has to take part in the collectives below)
-            err = e
-        _all_ok(err, args)
-        if args.keep_temp_files:
-            mdist.write_reads_kmc(query, args.temp_dir + "reads_60mers", 2, 3, args.device)
-        chosen = _on_rank0(lambda: _select_and_write(args, taxid2info, cmash_out))
-    except BaseException:
-        if rank == 0:
-            for path in written:
-                if os.path.exists(path):
-                    os.remove(path)
-        raise
-    finally:
-        query.close(); db.close()
-        mdist.close_exchanges()
-        ctx.close()
-    args._mlg_subset_written = True
-    return chosen
-
-
-def _select_and_write(args, taxid2info, cmash_out):
+def run_cmash_and_cutoff(args, taxid2info, cmash_out):
+    """The cutoff and the one-strain-per-species rule of select_db.py:80-96 on the query-results CSV (written by
+    write_gpu_files in place of the CMash subprocess of select_db.py:68-76), then the subset files; returns the selection"""
     chosen = _select(args, taxid2info, cmash_out)
+    _tick("selection done")
     make_db_and_dbinfo(args, chosen, taxid2info)
+    _tick("subset files written")
     return chosen
 
 
@@ -452,81 +446,86 @@ def make_db_and_dbinfo(args, organisms_to_include, taxid2info):
                 out.write("\t".join((acc, length, taxid, names, taxids)) + "\n")
 
 
-def _normalise(args):
+def resolve_data(args):
+    """AUTO resolution of the full database's paths, same outcomes as select_db.py:126-153: data/ with its slash, db_dir
+    (data/organism_files/), dbinfo_in (data/db_info.txt) and the native database file"""
+    if not args.data.endswith("/"):
+        args.data += "/"
+    for name, value in (("db_dir", "organism_files/"), ("dbinfo_in", "db_info.txt"), ("db_file", DB_BASENAME)):
+        if getattr(args, name) == "AUTO":
+            setattr(args, name, args.data + value)
+    if not args.db_dir.endswith("/"):
+        args.db_dir += "/"
+
+
+def _normalise(args, rank, world):
     """AUTO / NONE resolution, same outcomes as select_db.py:126-153"""
     for name, default in (("db_file", "AUTO"), ("gate", "exact"), ("device", 0), ("read_kmer_budget", 0),
                           ("read_kmer_passes", False)):
         if not hasattr(args, name):
             setattr(args, name, default)       # Namespace handed over by the reference's metalign.py
-    if not args.data.endswith("/"):
-        args.data += "/"
-    if args.db_dir == "AUTO":
-        args.db_dir = args.data + "organism_files/"
-    if not args.db_dir.endswith("/"):
-        args.db_dir += "/"
+    resolve_data(args)
     if args.temp_dir == "AUTO/":
-        args.temp_dir = shared_mkdtemp(args.data)
+        args.temp_dir = shared_mkdtemp(args.data, rank, world)
     if not args.temp_dir.endswith("/"):
         args.temp_dir += "/"
     os.makedirs(args.temp_dir, exist_ok=True)
-    if args.dbinfo_in == "AUTO":
-        args.dbinfo_in = args.data + "db_info.txt"
     if args.dbinfo_out == "AUTO":
         args.dbinfo_out = args.temp_dir + "subset_db_info.txt"
     if args.db == "AUTO":
         args.db = args.temp_dir + "cmashed_db.fna"
-    if args.db_file == "AUTO":
-        args.db_file = args.data + DB_BASENAME
     if args.input_type == "AUTO":
         from .ingest import detect_input_type
         args.input_type = detect_input_type(args.reads)
 
 
-def select_main(args=None):
+def select_main(args=None, *, stages=None, leave_open=False):
+    """select_db.py; returns the selection.  stages: a dict the run fills with its GPU stages' seconds (open_s, push_s,
+    exchange_s, finish_s).  leave_open: a single process that succeeds does not free its context, database and query, for
+    a caller that exits right after; a failed run frees them.  Under torchrun a failure on any rank raises on every rank
+    and rank 0 removes the run's files (output_paths); a single process leaves what it wrote, as the reference does."""
     if args is None:
         args = select_parseargs()
     elif args.cutoff < 0.0 or args.cutoff > 1.0:
         print("Error: args.cutoff must be between 0 and 1, inclusive.")
         sys.exit()
     init_ranks(args)
-    _normalise(args)
+    rank, world = ranks()
+    _normalise(args, rank, world)
     _tick("start")
-    if args.cmash_results == "NONE":
-        # db_info.txt has a line per accession of the full database: parsed beside the GPU stage, needed after it
-        import threading
-        box = {}
-
-        def load_info():
-            try:
-                box["info"] = read_dbinfo(args)
-            except BaseException as e:  # noqa: BLE001
-                box["error"] = e
-        th = threading.Thread(target=load_info)
-        th.start()
-        try:
-            run_kmc_steps(args)
-        finally:
-            th.join()
-        if "error" in box:
-            raise box["error"]
-        taxid2info = box["info"]
-    else:
+    if args.cmash_results != "NONE":
         taxid2info = read_dbinfo(args)
-    _tick("db_info read")
-    organisms_to_include = run_cmash_and_cutoff(args, taxid2info)
-    _tick("selection done")
-    if not getattr(args, "_mlg_subset_written", False):
-        _on_rank0(lambda: make_db_and_dbinfo(args, organisms_to_include, taxid2info))
-    _tick("subset files written")
-    return organisms_to_include
+        _tick("db_info read")
+        return _on_rank0(lambda: run_cmash_and_cutoff(args, taxid2info, args.cmash_results), rank, world)
+    stages = {} if stages is None else stages
+    # db_info.txt has a line per accession of the full database: parsed beside the GPU stage, needed after it
+    join_info = _on_helper(lambda: read_dbinfo(args))
+    try:
+        ctx, db, query = run_kmc_steps(args, rank, world, stages)
+    finally:
+        taxid2info, info_err = join_info()
+    try:
+        _all_ok(info_err, args.device, world)
+        _tick("db_info read")
+        write_gpu_files(args, db, query, rank, world, stages)
+        if world == 1 and not leave_open:
+            _close_gpu(world, query, db, ctx)
+            _tick("GPU objects closed")
+        cmash_out = args.temp_dir + "cmash_query_results.csv"
+        chosen = _on_rank0(lambda: run_cmash_and_cutoff(args, taxid2info, cmash_out), rank, world)
+    except BaseException:
+        if world > 1 and rank == 0:
+            _remove(output_paths(args))
+        _close_gpu(world, query, db, ctx)
+        raise
+    if world > 1:
+        _close_gpu(world, query, db, ctx)
+    return chosen
 
 
 # ------------------------------------------------------------------ many samples against one database
 SUMMARY_NAME = "samples_summary.tsv"
 SUMMARY_HEADER = "sample_id\tstatus\tselected\tseconds\terror\n"
-SAMPLE_FILES = ("cmash_query_results.csv", "cmashed_db.fna", "subset_db_info.txt", "60mers_intersection_dump",
-                "60mers_intersection_dump.fa", "60mers_intersection.kmc_pre", "60mers_intersection.kmc_suf",
-                "reads_60mers.kmc_pre", "reads_60mers.kmc_suf")
 _SAFE_ID = re.compile(r"[A-Za-z0-9][A-Za-z0-9._-]{0,127}\Z")
 
 Sample = collections.namedtuple("Sample", "id reads input_type")
@@ -596,24 +595,6 @@ class _NotRun(Exception):
     pass
 
 
-def sample_reader(args, pool):
-    """the reader of one sample of a batch: the whole file whatever the torchrun world (a rank runs whole samples), in
-    buffers from `pool`"""
-    return open_reader(args, alloc=pool, split=False)
-
-
-def _remove_sample_files(sample_dir):
-    for name in SAMPLE_FILES:
-        try:
-            os.remove(os.path.join(sample_dir, name))
-        except OSError:
-            pass
-    try:
-        os.rmdir(sample_dir)
-    except OSError:
-        pass                                                  # not empty: files that are not this run's stay
-
-
 class SelectSession:
     """One CUDA context, one loaded database, the parsed db_info and one pool of pinned reader buffers, kept for any
     number of samples.  `run(samples, out_dir)` writes each sample's select_db.py files into out_dir/<sample_id>/.
@@ -623,14 +604,16 @@ class SelectSession:
     and writes the subset FASTA and db_info (make_db_and_dbinfo).  So while sample i's subset files are written, sample
     i + 1's reads are already read and probed; the GPU thread runs at most one sample ahead.  The next sample's reader is
     opened while the current one finishes, in the buffers the closed reader gave back (ingest.BufferPool): pinned memory
-    stays at one reader's buffer sets.
+    stays at one reader's buffer sets.  Every sample is read whole and queried alone (rank 0 of a world of 1), also
+    under torchrun.
 
     A failing sample (an unreadable, truncated or corrupt reads file, a failed write, any library error but a device
-    error) fails alone: its query and reader are closed, its files removed, and the batch goes on.  A device error
-    (MLG_ERR_CUDA) ends the batch: the samples not yet run are reported as failed and no later run() starts any."""
+    error) fails alone: its query and reader are closed, its files and directory removed, and the batch goes on.  A
+    device error (MLG_ERR_CUDA) ends the batch: the samples not yet run are reported as failed and no later run() starts
+    any."""
 
     def __init__(self, args):
-        """args: the flags of select_many (data and db_file resolved as _normalise resolves them)"""
+        """args: the flags of select_many (data and db_file resolved as resolve_data resolves them)"""
         from . import ingest
         from .api import pinned_array
         t0 = _now()
@@ -661,13 +644,13 @@ class SelectSession:
             if err is not None:
                 raise err
             os.makedirs(a.temp_dir, exist_ok=True)
-            query = push_sample(a, self.db, reader, split=False)
+            query = push_sample(a, self.db, reader)
             reader.close()
             reader = None
             open_next()                              # its parser threads cut the first batches while this sample finishes
             stages["push_s"] = _now() - t0
             t0 = _now()
-            write_sample_files(a, self.db, query, {})
+            write_gpu_files(a, self.db, query, 0, 1, {})
             stages["gpu_files_s"] = _now() - t0
         finally:
             _close_all(reader, query)
@@ -683,7 +666,7 @@ class SelectSession:
         def reader_of(i):
             if i >= len(samples) or self.stopped is not None:
                 return lambda: (None, None)
-            return _on_helper(lambda: sample_reader(sargs[i], self.pool))
+            return _on_helper(lambda: open_reader(sargs[i], alloc=self.pool))
 
         def gpu_thread():
             # every sample is handed over, with its error if anything failed: the calling thread waits for each one
@@ -719,15 +702,18 @@ class SelectSession:
             if err is None:
                 t0 = _now()
                 try:
-                    chosen = _select(a, self.taxid2info, a.temp_dir + "cmash_query_results.csv")
-                    make_db_and_dbinfo(a, chosen, self.taxid2info)
+                    chosen = run_cmash_and_cutoff(a, self.taxid2info, a.temp_dir + "cmash_query_results.csv")
                 except Exception as e:  # noqa: BLE001
                     err = e
                 stages["subset_s"] = _now() - t0
             ahead.release()
             seconds = sum(stages.values())
             if err is not None:
-                _remove_sample_files(a.temp_dir)
+                _remove(output_paths(a))
+                try:
+                    os.rmdir(a.temp_dir)
+                except OSError:
+                    pass                             # not empty: files that are not this run's stay
                 msg = str(err) if isinstance(err, _NotRun) else "%s: %s" % (type(err).__name__, err)
                 results.append(SampleResult(samples[i].id, "failed", None, seconds, msg, a.temp_dir, stages))
             else:
@@ -743,40 +729,24 @@ def select_many_parseargs(argv=None):
     p.add_argument("data", help="data/ directory (database, db_info.txt, organism_files/)")
     p.add_argument("--out_dir", default="AUTO", help="where the sample directories and %s go (default: a new temporary "
                                                      "directory under data/)" % SUMMARY_NAME)
-    p.add_argument("--cutoff", type=float, default=0.01, help="containment cutoff at the largest k (default 0.01)")
-    p.add_argument("--db_dir", default="AUTO", help="directory holding the organism files of the full database")
-    p.add_argument("--dbinfo_in", default="AUTO", help="db_info file of the full database (default data/db_info.txt)")
-    p.add_argument("--keep_temp_files", action="store_true", help="also write each sample's intersection dump and KMC databases")
-    p.add_argument("--strain_level", action="store_true", help="keep every strain above the cutoff (default: one per species)")
-    p.add_argument("--threads", type=int, default=4, help="reader threads (per rank under torchrun)")
-    p.add_argument("--db_file", default="AUTO", help="native database file (default data/%s)" % DB_BASENAME)
-    p.add_argument("--gate", default="exact", choices=["exact", "none"], help="smallest-k prefilter model (see DESIGN.md)")
-    p.add_argument("--device", type=int, default=0, help="CUDA device")
-    p.add_argument("--read_kmer_budget", type=int, default=0, help="as select_db.py --read_kmer_budget, per sample")
-    p.add_argument("--read_kmer_passes", action="store_true", help="as select_db.py --read_kmer_passes")
+    _add_common_flags(p)
     return p.parse_args(argv)
 
 
-def normalise_many(args):
+def normalise_many(args, rank=0, world=1):
     """the AUTO defaults of select_many's flags, as _normalise resolves them for select_db; out_dir created"""
-    if not args.data.endswith("/"):
-        args.data += "/"
-    for name, value in (("db_dir", args.data + "organism_files/"), ("dbinfo_in", args.data + "db_info.txt"),
-                        ("db_file", args.data + DB_BASENAME)):
-        if getattr(args, name) == "AUTO":
-            setattr(args, name, value)
-    if not args.db_dir.endswith("/"):
-        args.db_dir += "/"
+    resolve_data(args)
     if args.out_dir == "AUTO":
-        args.out_dir = shared_mkdtemp(args.data)
+        args.out_dir = shared_mkdtemp(args.data, rank, world)
     os.makedirs(args.out_dir, exist_ok=True)
 
 
-def select_many(sample_sheet, args):
+def select_many(sample_sheet, args, stages=None):
     """select_db.py for every sample of a sample sheet (read_sample_sheet) against one database: each sample's files in
     args.out_dir/<sample_id>/ -- byte for byte what `select_db.py <reads> <data> --temp_dir out_dir/<sample_id>/` with the
     same flags writes -- and out_dir/samples_summary.tsv (format_summary).  Returns a SampleResult per sample in sheet
-    order; a caller can map and profile each ok sample from its out_dir.
+    order; a caller can map and profile each ok sample from its out_dir.  stages: a dict this rank fills with the seconds
+    it took to open the context and the database (open_s).
 
     The sheet is checked before any GPU work.  Under torchrun (WORLD_SIZE > 1) rank r runs the samples i with
     i mod world == r on its LOCAL_RANK GPU (its own context and database, no exchange); every rank gets every result, and
@@ -786,12 +756,13 @@ def select_many(sample_sheet, args):
     samples = read_sample_sheet(sample_sheet)
     init_ranks(args)
     rank, world = ranks()
-    normalise_many(args)
+    normalise_many(args, rank, world)
     mine = [samples[i] for i in rank_samples(len(samples), rank, world)]
     session = None
     try:
         session = SelectSession(args)
-        args._mlg_open_s = session.open_s
+        if stages is not None:
+            stages["open_s"] = session.open_s
         results = session.run(mine, args.out_dir)
     except Exception as e:  # noqa: BLE001  (no context or database: none of this rank's samples runs)
         msg = "not run: the database could not be opened on this GPU: %s: %s" % (type(e).__name__, e)

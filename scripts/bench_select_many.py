@@ -62,10 +62,10 @@ def run_many(d, out, threads, stages_path):
     from metalign_b200 import select_db
     sheet = os.path.join(d, "samples.tsv")
     args = select_db.select_many_parseargs([sheet, os.path.join(d, "data"), "--out_dir", out, "--threads", str(threads)])
-    results = select_db.select_many(sheet, args)
+    st = {"open_s": 0.0}
+    results = select_db.select_many(sheet, args, stages=st)
     rank, world = select_db.ranks()
     if rank == 0:
-        st = {"open_s": getattr(args, "_mlg_open_s", 0.0)}
         for k in ("push_s", "gpu_files_s", "subset_s"):
             st[k] = sum(r.stages.get(k, 0.0) for r in results)
         st["failed"] = [r.id for r in results if r.status != "ok"]

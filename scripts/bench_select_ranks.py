@@ -127,10 +127,10 @@ def run(d, fmt, threads):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     out = os.path.join(d, "out_%s_%d" % (fmt, world))
     args = select_db.select_parseargs([reads, os.path.join(d, "data"), "--temp_dir", out, "--threads", str(threads)])
+    times = {}
     t0 = time.perf_counter()
-    select_db.select_main(args)
+    select_db.select_main(args, stages=times)
     wall = time.perf_counter() - t0
-    times = dict(args._mlg_times)
     rank, world = select_db.ranks()
     all_times = [times]
     if world > 1:

@@ -13,13 +13,11 @@ import sys
 import pytest
 
 from conftest import ROOT
+from metalign_b200.select_db import OUTPUT_NAMES
 
 pytestmark = pytest.mark.gpu
 CASE = os.path.join(ROOT, "tests", "golden", "ref_e2e_case")
 DATA = os.path.join(CASE, "data")
-FILES = ("cmash_query_results.csv", "cmashed_db.fna", "subset_db_info.txt", "60mers_intersection_dump",
-         "60mers_intersection_dump.fa", "60mers_intersection.kmc_pre", "60mers_intersection.kmc_suf", "reads_60mers.kmc_pre",
-         "reads_60mers.kmc_suf")
 
 
 def _args(reads, out):
@@ -85,10 +83,10 @@ def test_ranks_write_the_one_gpu_files(tmp_path, bgzf_reads):
         for tag, (reads, exp) in inputs.items():
             out = str(tmp_path / ("w%d_%s" % (world, tag)))
             assert not [f for f in os.listdir(str(tmp_path)) if f.startswith("raised_w%d_%s_" % (world, tag))]
-            _same(out, str(tmp_path / ("one_" + tag)), FILES)
+            _same(out, str(tmp_path / ("one_" + tag)), OUTPUT_NAMES)
             _same(out, os.path.join(CASE, exp), sorted(os.listdir(os.path.join(CASE, exp))))
         # a reads file that does not exist: every rank raises, nothing is written
         raised = [f for f in os.listdir(str(tmp_path)) if f.startswith("raised_w%d_missing_" % world)]
         assert len(raised) == world, raised
         assert os.listdir(str(tmp_path / ("w%d_missing" % world))) == []
-        _same(str(tmp_path / ("w%d_metalign" % world)), str(tmp_path / "one_fq"), FILES)
+        _same(str(tmp_path / ("w%d_metalign" % world)), str(tmp_path / "one_fq"), OUTPUT_NAMES)

@@ -147,24 +147,23 @@ def _fastq(path, n, seed=5):
     return str(path)
 
 
-def test_batch_reader_reads_whole_files_under_torchrun(tmp_path, monkeypatch):
-    """a rank of select_many runs whole samples: with the process group up (rank 1 of 2) the batch's reader still yields
-    every record of the file, while the one-file multi-rank mode of select_db reads this rank's byte range only"""
+def test_batch_reader_reads_whole_files_and_a_rank_reads_its_share(tmp_path):
+    """a rank of select_many runs whole samples: the batch's reader (world 1, in pooled buffers) yields every record of
+    the file, while the one-file multi-rank mode of select_db (here rank 1 of 2) reads this rank's byte range only"""
     import argparse
     path = _fastq(tmp_path / "r.fq", 4000)
     args = argparse.Namespace(reads=path, input_type="fastq", threads=2)
     numpy_alloc = lambda nbytes: np.zeros(nbytes, dtype=np.uint8)      # noqa: E731
-    monkeypatch.setattr(select_db, "ranks", lambda: (1, 2))
 
     def count(reader):
         n = sum(int(b[3]) for b in reader)
         reader.close()
         return n
-    assert count(select_db.sample_reader(args, ingest.BufferPool(numpy_alloc))) == 4000
-    assert 0 < count(select_db.open_reader(args, alloc=numpy_alloc)) < 4000
+    assert count(select_db.open_reader(args, alloc=ingest.BufferPool(numpy_alloc))) == 4000
+    assert 0 < count(select_db.open_reader(args, 1, 2, alloc=numpy_alloc)) < 4000
 
 
-def test_batch_query_takes_read_kmer_passes_only_when_asked(monkeypatch):
+def test_query_takes_read_kmer_passes_when_asked_or_split_over_ranks():
     """under torchrun the one-file mode counts read k-mers in passes (its ranks hand the reads around); a batch sample has
     no exchange, so its query is opened as a single run's is"""
     import argparse
@@ -178,11 +177,10 @@ def test_batch_query_takes_read_kmer_passes_only_when_asked(monkeypatch):
         def query(self, **kw):
             opened.append(kw)
             return FakeQuery()
-    monkeypatch.setattr(select_db, "ranks", lambda: (1, 2))
     for passes in (False, True):
         args = argparse.Namespace(gate="exact", keep_temp_files=True, read_kmer_budget=123, read_kmer_passes=passes)
-        select_db.push_sample(args, FakeDb(), [], split=False)
-        select_db.push_sample(args, FakeDb(), [])
+        select_db.push_sample(args, FakeDb(), [])                 # a batch sample
+        select_db.push_sample(args, FakeDb(), [], world=2)        # a rank of the one-file mode
     assert [(q["read_kmer_passes"], q["read_kmer_budget"], q["read_kmers"]) for q in opened] == \
         [(False, 123, True), (True, 123, True), (True, 123, True), (True, 123, True)]
 
